@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA, sm_100a)
     python bench.py --impl reference --gpus N ...            # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs bench_outputs         # also write the last timed step's ids there (*.npy)
 
 A "step" is one encode_batch pass over one batch of synthetic input (BASELINE.json
 configs[1]: 1 GB synthetic multi-language code corpus, 131k Unigram vocab, crlf processor,
@@ -25,6 +26,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: the benchmark leaves nothing in it
 
 VOCAB_SIZE = 131072
 MAX_TOKEN_LEN = 16
@@ -77,6 +79,28 @@ def workload(synth, n_gpus, rank, nbytes, out=None):
         kind, seed, name = synth.KIND_CODE_CJK, 3 + 1000 * rank, "encode 1GB/GPU shard of code+Chinese mix, 131k vocab (configs[2])"
     blob, off = synth.corpus(kind, seed, nbytes, out=out)
     return blob, off, name
+
+
+DUMP_BYTES = 60_000_000  # data --dump-outputs writes at most (the id offsets take at most half of it)
+
+
+def dump_outputs(path, torch, d_ids, d_id_off, S):
+    """What the last timed step handed its caller (ids u32[T], id_off u64[S+1]), as .npy files in `path`:
+      id_off.npy  float64[S+1]  every sample's first token; the last entry is T
+      rows.npy    float64[k]    a sample of the samples, drawn in an order fixed by seed 0 for as long as the three
+                                files stay within DUMP_BYTES, ascending
+      ids.npy     float32[.]    the ids of those samples, concatenated in that order (ids < 2^24: exact)"""
+    id_off = d_id_off.cpu().numpy()
+    order = np.random.default_rng(0).permutation(S)
+    cost = np.cumsum(4 * (id_off[order + 1] - id_off[order]) + 8)
+    rows = np.sort(order[:int(np.searchsorted(cost, DUMP_BYTES - 8 * id_off.size, side="right"))])
+    n = id_off[rows + 1] - id_off[rows]
+    idx = np.arange(int(n.sum()), dtype=np.int64) + np.repeat(id_off[rows] - (np.cumsum(n) - n), n)
+    ids = d_ids[torch.from_numpy(idx).to(d_ids.device)].cpu().numpy().view(np.uint32)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "id_off.npy"), id_off.astype(np.float64))
+    np.save(os.path.join(path, "rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(path, "ids.npy"), ids.astype(np.float32))
 
 
 class ClockSampler:
@@ -391,7 +415,13 @@ def main():
     ap.add_argument("--chunk-bytes", type=int, default=0, help="bytes per chunk of the pipelined host entry point")
     ap.add_argument("--g-short", type=int, default=0)
     ap.add_argument("--long-threshold", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the ids and id offsets of the last timed encode step (rank 0's) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.only_schedule):
+        ap.error("--dump-outputs writes the native encode step's outputs: not with --impl reference / --only-schedule")
 
     rank, world, local = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     if args.impl == "reference":
@@ -449,6 +479,8 @@ def main():
     h_text = N.pinned_empty(args.bytes)
     blob, off, wname = workload(synth, world, rank, args.bytes, out=h_text)
     S, NB = len(off) - 1, int(off[-1])
+    if args.dump_outputs and 16 * (S + 1) > DUMP_BYTES:
+        raise SystemExit(f"--dump-outputs: the id offsets of {S} samples take more than half of {DUMP_BYTES} bytes")
 
     d_text = torch.from_numpy(blob).cuda()
     d_off = torch.from_numpy(off.view(np.int64)).cuda()
@@ -491,6 +523,8 @@ def main():
     barrier()
     wall = time.perf_counter() - t0
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch, d_ids, d_id_off, S)
 
     # max over ranks of the device time of the K steps
     tsum = torch.tensor([sum(dev_ms), wall, float(NB), float(tokens), sum(vit_ms)], dtype=torch.float64, device="cuda")
