@@ -41,7 +41,8 @@ typedef enum tgx_status {
   TGX_ERR_CUDA = 4,        /* CUDA runtime failure (message in tgx_last_error) */
   TGX_ERR_CAPACITY = 5,    /* output buffer too small; required size reported */
   TGX_ERR_NO_PATH = 6,     /* Error::NoPath(pos,len) (src/lib.rs:219-224,243-245) */
-  TGX_ERR_BAD_Z = 7        /* E-step: normalisation constant not "normal" (src/prune.rs:90-96) */
+  TGX_ERR_BAD_Z = 7,       /* E-step: normalisation constant not "normal" (src/prune.rs:90-96) */
+  TGX_ERR_NOT_UTF8 = 8     /* a corpus sample is not valid UTF-8 (load_sources, src/cli.rs:237-314) */
 } tgx_status;
 
 /* flags */
@@ -108,6 +109,29 @@ int tgx_encode_batch_dev(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
                          uint64_t n_bytes, uint32_t flags, uint32_t* d_ids, uint64_t ids_cap,
                          uint64_t* d_id_off, int32_t* d_status, uint64_t* d_proc_len, uint64_t* total_ids,
                          int64_t* first_bad);
+
+/* A corpus file image -> token ids: load_sources (src/cli.rs:237-314; samples separated by NUL bytes, docs/DATASET.md:69,
+ * empty samples dropped, every sample strict UTF-8) followed by Model::encode of every sample (src/model.rs:59-129) —
+ * the ordinary encoding: special tokens in the text are not split out.  The sample boundaries, the UTF-8 check and the
+ * compaction run on the device (corpus_count / corpus_scatter), in chunks of ~option 7 bytes cut after a NUL byte
+ * (a sample longer than a chunk enlarges it; samples must be shorter than 4 GiB).
+ *  data[n]      the corpus image, host memory (pinned memory gives full speed)
+ *  flags        TGX_FLAG_CRLF: CrlfProcessor per sample after the split ("\r" NUL "\n" stays two samples)
+ *  sample_base  index of the buffer's first non-empty sample in the whole file: the dropout draw is keyed by
+ *               sample_base + index (tgx_model_set_dropout), so ids do not depend on how a file is cut into buffers
+ *  sep_id       -1 = none, else appended after every sample (the last one included)
+ *  id_bytes     2 or 4: width of ids; with 2 the vocabulary and sep_id must be below 65536 (else TGX_ERR_UNSUPPORTED)
+ *  ids          [ids_cap] of id_bytes each; ids_cap >= n + 1 always suffices
+ *  id_off       [off_cap], n_samples + 1 entries written: sample i (its separator included) is ids[id_off[i] ..
+ *               id_off[i+1]); off_cap >= (NUL bytes in data) + 2 always suffices
+ *  n_samples / n_ids  non-empty samples and ids written (also when TGX_ERR_CAPACITY reports what is needed)
+ * Returns TGX_OK; TGX_ERR_NOT_UTF8 (*first_bad = lowest invalid sample, relative to the buffer, *bad_pos = byte offset
+ * of its first byte in data; nothing else is defined); TGX_ERR_NO_PATH (*first_bad = lowest failing sample, *bad_pos =
+ * its length after processing; the other samples are encoded); TGX_ERR_CAPACITY.  The handle's dropout applies as for
+ * tgx_encode_batch. */
+int tgx_encode_corpus(tgx_model* m, const uint8_t* data, uint64_t n, uint32_t flags, uint64_t sample_base,
+                      int64_t sep_id, uint32_t id_bytes, void* ids, uint64_t ids_cap, uint64_t* id_off,
+                      uint64_t off_cap, uint64_t* n_samples, uint64_t* n_ids, int64_t* first_bad, uint64_t* bad_pos);
 
 /* ModelVocabularyPruner::run_e_step (src/prune.rs:64-120): forward-backward expected
  * counts (Lattice::populate_marginal, src/lattice.rs:245-312, over Model::populate_nodes
@@ -191,12 +215,13 @@ int tgx_host_free(void* p);
  * 3 = fb-backward ms, 4 = whole call device ms, 5 = backtrack ms, 6 = emit ms, 7 = match_kernel ms (forward passes over
  * the match stream; then 1 = the consumer of the stream alone: viterbi_rows_kernel / viterbi_team_kernel), 8 = the whole
  * forward pass (match + consumers + the wait for the side stream), 9 = the pair-CTA kernel of the longest samples on its
- * side stream (forward pass 3), 10 = the forward pass the call used (option 3; automatic resolves to 2 or 3).  (For the
- * chunked host entry point these describe the LAST chunk.) */
+ * side stream (forward pass 3), 10 = the forward pass the call used (option 3; automatic resolves to 2 or 3), 11 = the
+ * split kernels of tgx_encode_corpus summed over its chunks.  (For the chunked host entry points the others describe the
+ * LAST chunk.) */
 double tgx_model_last_stat(const tgx_model* m, int what);
 
 /* Options.  Two of them are for callers:
- *    7 = bytes per chunk of the pipelined host entry point tgx_encode_batch (default ~352 MiB);
+ *    7 = bytes per chunk of the pipelined host entry points tgx_encode_batch / tgx_encode_corpus (default ~352 MiB);
  *   22 = byte offset of the E-step's text in the whole corpus when the call handles one shard of it (keyed dropout
  *        draw, see tgx_model_set_dropout).
  * The rest select between tested kernel variants and their launch shapes (bench / tests / tools/probe.py; not a stable

@@ -19,6 +19,7 @@ LIB_PATH = os.path.join(_HERE, "csrc", "libtokengeex_b200.so")
 
 TGX_OK, TGX_ERR_INVALID, TGX_ERR_UNSUPPORTED, TGX_ERR_NO_DEVICE = 0, 1, 2, 3
 TGX_ERR_CUDA, TGX_ERR_CAPACITY, TGX_ERR_NO_PATH, TGX_ERR_BAD_Z = 4, 5, 6, 7
+TGX_ERR_NOT_UTF8 = 8
 TGX_FLAG_CRLF = 1
 SNIPPET_LEN = 8192 * 10  # MAX_SAMPLE_LENGTH, /root/reference/src/prune.rs:75
 
@@ -47,6 +48,8 @@ SYMBOLS = [
                                    u64p, i64p]),
     ("tgx_encode_batch_dev", C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32,
                                        C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, u64p, i64p]),
+    ("tgx_encode_corpus", C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint64, C.c_int64, C.c_uint32,
+                                    C.c_void_p, C.c_uint64, u64p, C.c_uint64, u64p, u64p, i64p, u64p]),
     ("tgx_expected_counts", C.c_int, [C.c_void_p, u8p, u64p, C.c_uint64, C.c_uint64, f64p, i64p, f64p]),
     ("tgx_expected_counts_dev", C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64,
                                           C.c_void_p, i64p, f64p]),
@@ -225,6 +228,30 @@ class Model:
                                     C.byref(bad))
         _check(rc, (TGX_OK, TGX_ERR_NO_PATH))
         return ids[:int(id_off[S])], id_off, status[:S], plen[:S], rc, int(bad.value)
+
+    def encode_corpus(self, data: np.ndarray, crlf: bool = False, sample_base: int = 0, sep_id: int = -1,
+                      dtype=np.uint32, ids_out: np.ndarray = None, off_out: np.ndarray = None):
+        """tgx_encode_corpus over a NUL-separated corpus image (u8[n]) → (ids, id_off u64[S+1], rc, first_bad,
+        bad_pos); rc is TGX_OK, TGX_ERR_NOT_UTF8 or TGX_ERR_NO_PATH (see include/tokengeex_b200.h).  ids_out / off_out:
+        buffers to write into (e.g. pinned); too small ones are replaced by ones of the size the call reports."""
+        dtype = np.dtype(dtype)
+        n = int(data.size)
+        ids = ids_out if ids_out is not None else np.empty(n + 1, dtype)
+        off = off_out if off_out is not None else np.empty(n // 64 + 2, np.uint64)
+        while True:
+            ns, ni, bad, pos = C.c_uint64(0), C.c_uint64(0), C.c_int64(-1), C.c_uint64(0)
+            rc = lib().tgx_encode_corpus(self._h, data.ctypes.data, n, TGX_FLAG_CRLF if crlf else 0, sample_base,
+                                         sep_id, dtype.itemsize, ids.ctypes.data, ids.size, _p(off, u64p), off.size,
+                                         C.byref(ns), C.byref(ni), C.byref(bad), C.byref(pos))
+            if rc != TGX_ERR_CAPACITY:
+                break
+            if int(ni.value) > ids.size:
+                ids = np.empty(int(ni.value), dtype)
+            if int(ns.value) + 1 > off.size:
+                off = np.empty(int(ns.value) + 1, np.uint64)
+        _check(rc, (TGX_OK, TGX_ERR_NOT_UTF8, TGX_ERR_NO_PATH))
+        S = int(ns.value)
+        return ids[:int(ni.value)], off[:S + 1], rc, int(bad.value), int(pos.value)
 
     def expected_counts(self, blob: np.ndarray, off: np.ndarray, snippet_len: int = SNIPPET_LEN):
         """→ (expected f64[V], rc, bad_sample, bad_z)"""

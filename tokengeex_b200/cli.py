@@ -7,6 +7,10 @@ Mirrors the reference's command line for this one sub-command (/root/reference/s
         --train code:./data/train/code.bin:0.5 --train zh:./data/train/zh.bin \\
         --dropout 0.0 --shrink-factor 0.8 --em-subiters 2
 
+`encode` pretokenizes one corpus file to token ids on disk (tokengeex_b200/corpus.py):
+
+    python -m tokengeex_b200.cli encode -i tokenizer.json --input corpus.bin -o out/prefix --separator "<eos>"
+
 A source is `name:path[:proportion]`; the file holds samples separated by NUL bytes (docs/DATASET.md:69); every
 sample must be valid UTF-8; empty samples are dropped; `floor(count * proportion)` samples are taken from the front;
 the tokenizer's processors are applied and samples that became empty are dropped.  The reference then shuffles the
@@ -139,6 +143,29 @@ def prune_cmd(input: str, output: str, vocab_size: int, train: Sequence[str], dr
     return report
 
 
+def encode_cmd(input: str, source: str, output: str, separator: Optional[str] = None, dtype: str = "auto",
+               dropout: float = 0.0, dropout_seed: Optional[int] = None, device: Optional[int] = None,
+               window_bytes: Optional[int] = None) -> dict:
+    """Pretokenizes a NUL-separated corpus file into OUTPUT.{ids,idx,json} (tokengeex_b200/corpus.py)."""
+    import time
+
+    from . import corpus
+
+    if device is None:
+        device = int(os.environ.get("TGX_DEVICE", "0"))
+    log.info("Encoding corpus input=%r source=%r output=%r separator=%r dtype=%s dropout=%s", input, source, output,
+             separator, dtype, dropout)
+    t0 = time.perf_counter()
+    meta = corpus.encode_file(input, source, output, separator=separator, dtype=None if dtype == "auto" else dtype,
+                              dropout=dropout, dropout_seed=dropout_seed, device=device,
+                              window_bytes=window_bytes or corpus.DEFAULT_WINDOW_BYTES)
+    dt = time.perf_counter() - t0
+    size = meta["source"]["bytes"]
+    log.info("Encoded %d samples into %d %s ids from %r (%.2fMB) in %.2fs (%.2f GB/s)", meta["n_samples"],
+             meta["n_ids"], meta["dtype"], source, size / 1e6, dt, size / dt / 1e9 if dt > 0 else 0.0)
+    return meta
+
+
 def main(argv: Optional[Sequence[str]] = None) -> int:
     ap = argparse.ArgumentParser(prog="tokengeex_b200", description=__doc__.split("\n\n")[0])
     sub = ap.add_subparsers(dest="cmd", required=True)
@@ -153,8 +180,22 @@ def main(argv: Optional[Sequence[str]] = None) -> int:
     pr.add_argument("--em-subiters", type=int, default=1)
     pr.add_argument("--device", type=int, default=None)
     pr.add_argument("--shuffle-seed", type=int, default=None)
+    en = sub.add_parser("encode", help="tokenize a NUL-separated corpus file into token ids on the GPU")
+    en.add_argument("-i", dest="tokenizer", required=True, help="tokenizer JSON")
+    en.add_argument("--input", dest="source", required=True, help="corpus file: samples separated by NUL bytes")
+    en.add_argument("-o", "--output", required=True, help="output prefix: PREFIX.ids, PREFIX.idx, PREFIX.json")
+    en.add_argument("--separator", default=None, metavar="TOKEN", help="token appended after every sample")
+    en.add_argument("--dtype", choices=("auto", "uint16", "uint32"), default="auto")
+    en.add_argument("--dropout", type=float, default=0.0, help="dropout in [0, 1) (default 0.0: plain encoding)")
+    en.add_argument("--dropout-seed", type=int, default=None, help="seed of the keyed dropout draw (default: fresh)")
+    en.add_argument("--device", type=int, default=None)
+    en.add_argument("--window-bytes", type=int, default=None, help="bytes read per window (default 2 GiB)")
     args = ap.parse_args(argv)
     logging.basicConfig(level=logging.INFO, format="%(asctime)s %(levelname)s %(message)s")
+    if args.cmd == "encode":
+        encode_cmd(args.tokenizer, args.source, args.output, args.separator, args.dtype, args.dropout, args.dropout_seed,
+                   args.device, args.window_bytes)
+        return 0
     if not args.train:
         ap.error("at least one --train source is required")
     prune_cmd(args.input, args.output, args.vocab_size, args.train, args.dropout, args.shrink_factor, args.em_subiters,

@@ -65,7 +65,7 @@ struct DevBuf {
 
 struct Stats {
   double launches = 0, viterbi_ms = 0, fwd_ms = 0, bwd_ms = 0, total_ms = 0, back_ms = 0, emit_ms = 0, match_ms = 0,
-         side_ms = 0, forward_ms = 0, algo = 0;
+         side_ms = 0, forward_ms = 0, algo = 0, split_ms = 0;
 };
 
 }  // namespace
@@ -194,6 +194,10 @@ struct tgx_model {
   // buffers of the host entry points (two sets for the chunk pipeline) and of the E-step / frequency pass
   DevBuf Bbeta, accfix;
   DevBuf text, off, idoff, A, expected, freq, ids, scount, hot, text_b, off_b, ids_b, idoff_b, scount_b;
+  // tgx_encode_corpus, per buffer set: raw chunk, split scratch (tile counts and their scan, control words), the ids
+  // as they leave the device (corpus_finalize); events around the split kernels (tgx_model_last_stat 11)
+  DevBuf raw[2], split[2], fin[2];
+  cudaEvent_t ev_split[2][4] = {};
 };
 
 // =========================================================================================
@@ -311,6 +315,45 @@ __device__ __forceinline__ uint64_t lower_bound_off(const uint64_t* __restrict__
   return lo;
 }
 
+// Compaction of one tile (CRLF_TILE bytes at most) through shared memory: the thread's 16 bytes `v` minus the bytes flagged
+// in `m` go to stage[o ..], then the tile's `total` kept bytes are written to out[ob ..] with aligned 16-byte stores.
+__device__ __forceinline__ void tile_compact_store(const uint4& v, uint32_t m, uint32_t nvalid, uint32_t o, uint64_t ob,
+                                                   uint32_t total, uint8_t* stage, uint8_t* __restrict__ out) {
+  const uint32_t wv[4] = {v.x, v.y, v.z, v.w};
+  if (m == 0 && nvalid == 16 && (o & 3u) == 0) {
+#pragma unroll
+    for (int j = 0; j < 4; j++) *reinterpret_cast<uint32_t*>(stage + o + 4 * j) = wv[j];
+  } else {
+    uint32_t q = o;
+#pragma unroll
+    for (int i = 0; i < 16; i++)
+      if (i < (int)nvalid && !((m >> i) & 1u)) stage[q++] = (uint8_t)(wv[i >> 2] >> (8 * (i & 3)));
+  }
+  __syncthreads();
+  // ---- [ob, ob + total) of `out`: unaligned head and tail by bytes, the rest by 16-byte vectors
+  const uint64_t oe = ob + total;
+  const uint64_t a0 = min((uint64_t)((ob + 15) & ~15ull), oe);
+  const uint32_t head = (uint32_t)(a0 - ob);
+  if (threadIdx.x < head) out[ob + threadIdx.x] = stage[threadIdx.x];
+  const uint32_t nvec = (uint32_t)((oe - a0) >> 4);
+  for (uint32_t c = threadIdx.x; c < nvec; c += CRLF_BLOCK) {
+    const uint32_t so = head + 16 * c;  // source offset in stage (any alignment)
+    const uint32_t* sw = reinterpret_cast<const uint32_t*>(stage + (so & ~3u));
+    const uint32_t sh = 8 * (so & 3u);
+    uint32_t w[5];
+#pragma unroll
+    for (int j = 0; j < 5; j++) w[j] = sw[j];
+    uint4 r;
+    r.x = __funnelshift_r(w[0], w[1], sh);
+    r.y = __funnelshift_r(w[1], w[2], sh);
+    r.z = __funnelshift_r(w[2], w[3], sh);
+    r.w = __funnelshift_r(w[3], w[4], sh);
+    *reinterpret_cast<uint4*>(out + a0 + 16ull * c) = r;
+  }
+  const uint64_t t0 = a0 + 16ull * nvec;
+  if (threadIdx.x < (uint32_t)(oe - t0)) out[t0 + threadIdx.x] = stage[(uint32_t)(t0 - ob) + threadIdx.x];
+}
+
 // K1c: compact every tile through shared memory and write it with aligned 16-byte stores; the
 // thread that sees a sample start also writes that sample's new offset (found by binary search).
 // blk_prefix = exclusive scan of blk_removed (n_tiles + 1 entries).
@@ -346,40 +389,166 @@ __global__ void __launch_bounds__(CRLF_BLOCK) crlf_scatter(const uint8_t* __rest
     const uint64_t np = N - blk_prefix[n_tiles];
     for (uint64_t s = lower_bound_off(off, S, N); s <= S; s++) new_off[s] = np;
   }
-  // ---- compaction into shared memory
-  const uint32_t wv[4] = {v.x, v.y, v.z, v.w};
-  if (m == 0 && nvalid == 16 && (o & 3u) == 0) {
-#pragma unroll
-    for (int j = 0; j < 4; j++) *reinterpret_cast<uint32_t*>(stage + o + 4 * j) = wv[j];
+  tile_compact_store(v, m, nvalid, o, ob, total, stage, out);
+}
+
+// ---- corpus split (tgx_encode_corpus): a raw chunk of NUL-separated samples -> blob + offsets of the non-empty
+// samples, every sample checked to be strict UTF-8 (Unicode Table 3-7, what str::from_utf8 and Python's strict decode
+// accept).  Same shape as the crlf kernels: per-thread 16-byte masks, counts per 4096-byte tile, one scan, scatter.
+
+// Masks of the 16 positions base .. base+15 (bit i <-> base + i): `keep` = not NUL, `start` = first byte of a
+// non-empty sample (a byte before position 0 counts as NUL), `bad` = where strict decoding fails.  Bytes at or beyond N
+// read as NUL, so a sequence cut off by a NUL or by the end of the buffer fails at its lead byte.
+__device__ __forceinline__ void corpus_mask16(const uint8_t* __restrict__ text, uint64_t N, uint64_t base, uint4& v,
+                                              uint32_t& keep, uint32_t& start, uint32_t& bad, uint32_t& nvalid) {
+  nvalid = base < N ? (uint32_t)min((uint64_t)16, N - base) : 0u;
+  if (nvalid == 16) {
+    v = *reinterpret_cast<const uint4*>(text + base);
   } else {
-    uint32_t q = o;
-#pragma unroll
-    for (int i = 0; i < 16; i++)
-      if (i < (int)nvalid && !((m >> i) & 1u)) stage[q++] = (uint8_t)(wv[i >> 2] >> (8 * (i & 3)));
+    uint32_t w[4] = {0, 0, 0, 0};
+    for (uint32_t i = 0; i < nvalid; i++) w[i >> 2] |= (uint32_t)text[base + i] << (8 * (i & 3));
+    v = make_uint4(w[0], w[1], w[2], w[3]);
   }
+  // bit e <-> position base + e - 3: the three bytes before the thread's 16 and the three after them
+  const uint32_t wv[4] = {v.x, v.y, v.z, v.w};
+  uint32_t nul = 0, cont = 0, ge2 = 0, ge3 = 0, l4 = 0, badlead = 0, e0 = 0, ed = 0, f0 = 0, f4 = 0, c8 = 0, c9 = 0,
+           ca = 0;
+#pragma unroll
+  for (int e = 0; e < 22; e++) {
+    uint32_t c;
+    if (e < 3) {
+      c = (base + e >= 3 && base + e - 3 < N) ? text[base + e - 3] : 0u;
+    } else if (e < 19) {
+      c = (wv[(e - 3) >> 2] >> (8 * ((e - 3) & 3))) & 0xFFu;
+    } else {
+      c = base + e - 3 < N ? text[base + e - 3] : 0u;
+    }
+    nul |= (uint32_t)(c == 0) << e;
+    cont |= (uint32_t)((c & 0xC0u) == 0x80u) << e;
+    ge2 |= (uint32_t)(c >= 0xC2u && c <= 0xF4u) << e;
+    ge3 |= (uint32_t)(c >= 0xE0u && c <= 0xF4u) << e;
+    l4 |= (uint32_t)(c >= 0xF0u && c <= 0xF4u) << e;
+    badlead |= (uint32_t)(c == 0xC0u || c == 0xC1u || c >= 0xF5u) << e;
+    e0 |= (uint32_t)(c == 0xE0u) << e;
+    ed |= (uint32_t)(c == 0xEDu) << e;
+    f0 |= (uint32_t)(c == 0xF0u) << e;
+    f4 |= (uint32_t)(c == 0xF4u) << e;
+    c8 |= (uint32_t)(c >= 0x80u && c <= 0x8Fu) << e;
+    c9 |= (uint32_t)(c >= 0x80u && c <= 0x9Fu) << e;
+    ca |= (uint32_t)(c >= 0xA0u && c <= 0xBFu) << e;
+  }
+  const uint32_t covered = (ge2 << 1) | (ge3 << 2) | (l4 << 3);  // continuation positions some lead byte claims
+  uint32_t b = badlead | (cont & ~covered);
+  b |= (ge2 & ~(cont >> 1)) | (ge3 & ~(cont >> 2)) | (l4 & ~(cont >> 3));
+  // second-byte ranges: E0 A0..BF (overlong), ED 80..9F (surrogates), F0 90..BF (overlong), F4 80..8F (> U+10FFFF)
+  b |= (e0 & ~(ca >> 1)) | (ed & ~(c9 >> 1)) | (f0 & ~((ca | (c9 & ~c8)) >> 1)) | (f4 & ~(c8 >> 1));
+  const uint32_t valid = nvalid == 16 ? 0xFFFFu : (1u << nvalid) - 1u;
+  keep = (~nul >> 3) & valid;
+  start = (~nul & (nul << 1)) >> 3 & valid;
+  bad = (b >> 3) & valid;
+}
+
+struct KeptStarts {  // scan element: kept bytes (x) and sample starts (y) before a tile
+  unsigned long long x, y;
+};
+struct AddKeptStarts {
+  __host__ __device__ KeptStarts operator()(const KeptStarts& a, const KeptStarts& b) const { return {a.x + b.x, a.y + b.y}; }
+};
+
+// S1: kept bytes and sample starts per tile; the lowest position where decoding fails (atomicMin into *bad_pos).
+__global__ void __launch_bounds__(CRLF_BLOCK) corpus_count(const uint8_t* __restrict__ text, uint64_t N,
+                                                           KeptStarts* __restrict__ tile_cnt,
+                                                           unsigned long long* __restrict__ bad_pos) {
+  __shared__ uint32_t ws[CRLF_BLOCK / 32];
+  const uint64_t base = (uint64_t)blockIdx.x * CRLF_TILE + (uint64_t)threadIdx.x * CRLF_PER_THREAD;
+  uint4 v;
+  uint32_t keep, start, bad, nvalid;
+  corpus_mask16(text, N, base, v, keep, start, bad, nvalid);
+  if (bad) atomicMin(bad_pos, (unsigned long long)(base + __ffs(bad) - 1));
+  uint32_t c = __popc(keep) | (__popc(start) << 16);  // a tile has at most 4096 kept bytes and 2048 starts
+#pragma unroll
+  for (int o = 16; o; o >>= 1) c += __shfl_xor_sync(0xFFFFFFFFu, c, o);
+  if ((threadIdx.x & 31) == 0) ws[threadIdx.x >> 5] = c;
   __syncthreads();
-  // ---- [ob, ob + total) of `out`: unaligned head and tail by bytes, the rest by 16-byte vectors
-  const uint64_t oe = ob + total;
-  const uint64_t a0 = min((uint64_t)((ob + 15) & ~15ull), oe);
-  const uint32_t head = (uint32_t)(a0 - ob);
-  if (threadIdx.x < head) out[ob + threadIdx.x] = stage[threadIdx.x];
-  const uint32_t nvec = (uint32_t)((oe - a0) >> 4);
-  for (uint32_t c = threadIdx.x; c < nvec; c += CRLF_BLOCK) {
-    const uint32_t so = head + 16 * c;  // source offset in stage (any alignment)
-    const uint32_t* sw = reinterpret_cast<const uint32_t*>(stage + (so & ~3u));
-    const uint32_t sh = 8 * (so & 3u);
-    uint32_t w[5];
+  if (threadIdx.x == 0) {
+    uint32_t t = 0;
 #pragma unroll
-    for (int j = 0; j < 5; j++) w[j] = sw[j];
-    uint4 r;
-    r.x = __funnelshift_r(w[0], w[1], sh);
-    r.y = __funnelshift_r(w[1], w[2], sh);
-    r.z = __funnelshift_r(w[2], w[3], sh);
-    r.w = __funnelshift_r(w[3], w[4], sh);
-    *reinterpret_cast<uint4*>(out + a0 + 16ull * c) = r;
+    for (int i = 0; i < CRLF_BLOCK / 32; i++) t += ws[i];
+    tile_cnt[blockIdx.x] = {t & 0xFFFFu, t >> 16};
   }
-  const uint64_t t0 = a0 + 16ull * nvec;
-  if (threadIdx.x < (uint32_t)(oe - t0)) out[t0 + threadIdx.x] = stage[(uint32_t)(t0 - ob) + threadIdx.x];
+}
+
+// S2 (one thread, after the scan): words[0] = samples, words[1] = kept bytes, words[2] = the sample *bad_pos lies in
+// (~0 = every sample is valid UTF-8).
+__global__ void corpus_words(const uint8_t* __restrict__ text, const KeptStarts* __restrict__ prefix, uint64_t n_tiles,
+                             const unsigned long long* __restrict__ bad_pos, unsigned long long* __restrict__ words) {
+  if (threadIdx.x || blockIdx.x) return;
+  words[0] = prefix[n_tiles].y;
+  words[1] = prefix[n_tiles].x;
+  const unsigned long long q = *bad_pos;
+  unsigned long long s = ~0ull;
+  if (q != ~0ull) {
+    const uint64_t t0 = q / CRLF_TILE * CRLF_TILE;
+    s = prefix[q / CRLF_TILE].y;
+    for (uint64_t p = t0; p <= q; p++) s += text[p] != 0 && (p == 0 || text[p - 1] == 0);
+    s -= 1;  // a failing byte is never NUL, so a sample starts at or before it
+  }
+  words[2] = s;
+}
+
+// S3: compaction of the kept bytes (tile_compact_store) and the offset of every sample (off[S] = kept bytes).
+__global__ void __launch_bounds__(CRLF_BLOCK) corpus_scatter(const uint8_t* __restrict__ text, uint64_t N,
+                                                             const KeptStarts* __restrict__ prefix, uint64_t n_tiles,
+                                                             uint8_t* __restrict__ out, uint64_t* __restrict__ off) {
+  __shared__ uint32_t ws[CRLF_BLOCK / 32];
+  __shared__ __align__(16) uint8_t stage[CRLF_TILE + 32];
+  const uint64_t base = (uint64_t)blockIdx.x * CRLF_TILE + (uint64_t)threadIdx.x * CRLF_PER_THREAD;
+  uint4 v;
+  uint32_t keep, start, bad, nvalid;
+  corpus_mask16(text, N, base, v, keep, start, bad, nvalid);
+  uint32_t total;
+  const uint32_t o = block_exclusive_scan(__popc(keep) | (__popc(start) << 16), ws, &total);
+  const KeptStarts tp = prefix[blockIdx.x];
+  uint64_t s = tp.y + (o >> 16);
+  for (uint32_t sb = start; sb; sb &= sb - 1) {
+    const int i = __ffs(sb) - 1;
+    off[s++] = tp.x + (o & 0xFFFFu) + __popc(keep & ((1u << i) - 1u));
+  }
+  if (blockIdx.x == n_tiles - 1 && threadIdx.x == 0) off[prefix[n_tiles].y] = prefix[n_tiles].x;
+  tile_compact_store(v, ~keep & 0xFFFFu, nvalid, o & 0xFFFFu, tp.x, total & 0xFFFFu, stage, out);
+}
+
+// Output of tgx_encode_corpus: the ids narrowed to T and, when sep >= 0, sep after every sample (sample i's ids move
+// to id_off[i] + i).  Blocks take 256 consecutive ids; each finds its rows by binary search inside the rows of its block.
+template <class T>
+__global__ void __launch_bounds__(256) corpus_finalize(const uint32_t* __restrict__ ids, const uint64_t* __restrict__ id_off,
+                                                       uint64_t S, long long sep, T* __restrict__ out) {
+  __shared__ uint64_t rows[2];
+  const uint64_t n = id_off[S];
+  for (uint64_t b0 = (uint64_t)blockIdx.x * 256; b0 < n; b0 += (uint64_t)gridDim.x * 256) {
+    const uint64_t t = b0 + threadIdx.x;
+    if (sep < 0) {
+      if (t < n) out[t] = (T)ids[t];
+      continue;
+    }
+    auto row_of = [&](uint64_t x, uint64_t lo, uint64_t hi) {  // last r in [lo, hi] with id_off[r] <= x
+      while (lo < hi) {
+        const uint64_t mid = (lo + hi + 1) >> 1;
+        if (id_off[mid] <= x) lo = mid; else hi = mid - 1;
+      }
+      return lo;
+    };
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      rows[0] = row_of(b0, 0, S - 1);
+      rows[1] = row_of(min(b0 + 255, n - 1), rows[0], S - 1);
+    }
+    __syncthreads();
+    if (t < n) out[t + row_of(t, rows[0], rows[1])] = (T)ids[t];
+  }
+  if (sep >= 0)
+    for (uint64_t r = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; r < S; r += (uint64_t)gridDim.x * blockDim.x)
+      out[id_off[r + 1] + r] = (T)sep;
 }
 
 // units = samples
@@ -1194,6 +1363,7 @@ int tgx_model_create(const uint8_t* token_bytes, const uint64_t* token_offsets, 
     for (int i = 0; i < 2; i++) {
       CU(cudaEventCreateWithFlags(&m->ev_h2d[i], cudaEventDisableTiming));
       CU(cudaEventCreateWithFlags(&m->ev_d2h[i], cudaEventDisableTiming));
+      for (auto& e : m->ev_split[i]) CU(cudaEventCreate(&e));
     }
     CU(cudaEventCreateWithFlags(&m->ev_fork, cudaEventDisableTiming));
     CU(cudaEventCreateWithFlags(&m->ev_join, cudaEventDisableTiming));
@@ -1309,6 +1479,11 @@ void tgx_model_destroy(tgx_model* m) {
     for (int i = 0; i < 2; i++) {
       if (m->ev_h2d[i]) cudaEventDestroy(m->ev_h2d[i]);
       if (m->ev_d2h[i]) cudaEventDestroy(m->ev_d2h[i]);
+      for (auto& e : m->ev_split[i])
+        if (e) cudaEventDestroy(e);
+      m->raw[i].release();
+      m->split[i].release();
+      m->fin[i].release();
     }
     if (m->h_off) cudaFreeHost(m->h_off);
     if (m->h_out) cudaFreeHost(m->h_out);
@@ -1410,6 +1585,7 @@ double tgx_model_last_stat(const tgx_model* m, int what) {
     case 8: return m->last_stats.forward_ms;  // match + consumers (+ the wait for the side stream)
     case 10: return m->last_stats.algo;       // forward algorithm the call used (option 3; 4 = automatic resolves to 2 or 3)
     case 9: return m->last_stats.side_ms;     // pair-CTA kernel of the longest samples on the side stream (algo 3)
+    case 11: return m->last_stats.split_ms;   // tgx_encode_corpus: split kernels of every chunk
   }
   return 0;
 }
@@ -1577,88 +1753,79 @@ int tgx_encode_batch_dev(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
   return TGX_OK;
 }
 
-int tgx_encode_batch(tgx_model* m, const uint8_t* text, const uint64_t* off, uint64_t S, uint32_t flags,
-                     uint32_t* ids, uint64_t ids_cap, uint64_t* id_off, int32_t* status, uint64_t* proc_len,
-                     int64_t* first_bad_out) {
-  int rc = check_model(m);
-  if (rc) return rc;
-  if (!off || !id_off || off[0] != 0) return fail(TGX_ERR_INVALID, "offsets must start at 0");
-  for (uint64_t i = 0; i < S; i++) {  // (the reference has no limit on a sample; the kernels index positions with 32 bits)
-    if (off[i + 1] < off[i]) return fail(TGX_ERR_INVALID, "offsets must not decrease");
-    if (off[i + 1] - off[i] >= (1ull << 32)) return fail(TGX_ERR_UNSUPPORTED, "a sample of 4 GiB or more is not supported");
-  }
-  const uint64_t N = off[S];
-  std::lock_guard<std::recursive_mutex> g(m->mu);
-  struct WiGuard {  // whatever path leaves this function, the next call starts on workspace 0
-    tgx_model* m;
-    ~WiGuard() { m->wi = 0; }
-  } wi_guard{m};
-  if (first_bad_out) *first_bad_out = -1;
-  if (S == 0) {
-    id_off[0] = 0;
-    return TGX_OK;
-  }
-  // Chunks of whole samples (~chunk_bytes each): the H2D copy of chunk k+1 and the D2H copy of
-  // chunk k-1 run on their own streams beside the kernels of chunk k (two buffer sets).
-  const uint64_t K = std::max<uint64_t>(1, std::min<uint64_t>(16, (N + m->chunk_bytes - 1) / m->chunk_bytes));
-  std::vector<uint64_t> cut(K + 1, 0);
-  cut[K] = S;
-  for (uint64_t k = 1; k < K; k++) {
-    const uint64_t target = N / K * k;
-    uint64_t i = (uint64_t)(std::lower_bound(off, off + S + 1, target) - off);
-    cut[k] = std::min<uint64_t>(std::max<uint64_t>(i, cut[k - 1]), S);
-  }
-  uint64_t max_b = 0, max_s = 0;
-  for (uint64_t k = 0; k < K; k++) {
-    max_b = std::max(max_b, off[cut[k + 1]] - off[cut[k]]);
-    max_s = std::max(max_s, cut[k + 1] - cut[k]);
-  }
-  DevBuf* d_text[2] = {&m->text, &m->text_b};
-  DevBuf* d_off[2] = {&m->off, &m->off_b};
-  DevBuf* d_ids[2] = {&m->ids, &m->ids_b};
-  DevBuf* d_idoff[2] = {&m->idoff, &m->idoff_b};
-  DevBuf* d_sc[2] = {&m->scount, &m->scount_b};
+namespace {
+
+// ---- chunk pipeline of the host entry points (tgx_encode_batch, tgx_encode_corpus)
+// Chunks of whole samples (~chunk_bytes each): the H2D copy of chunk k+1 and the D2H copy of chunk k-1 run on their own
+// streams beside the kernels of chunk k (two buffer sets).  What reaches the device and what leaves it is the caller's:
+
+// Input stage: puts chunk k's samples as blob + offsets into buffer set b (m->text / m->text_b, m->off / m->off_b).
+struct ChunkInput {
+  uint64_t K = 1;      // chunks
+  uint64_t max_b = 0;  // bytes of the largest chunk as it reaches the device
+  uint64_t max_s = 0;  // samples of the largest chunk, when known before the chunks are split
+  virtual ~ChunkInput() = default;
+  // Queues the H2D copy of chunk k on `st` (the copy-in stream when K > 1); returns without waiting.
+  virtual int h2d(tgx_model* m, uint64_t k, int b, cudaStream_t st) = 0;
+  // Queued on the compute stream of chunk k's workspace right after the copy was queued (so behind the previous
+  // chunk's kernels); returns without waiting.
+  virtual int after_h2d(tgx_model*, uint64_t, int) { return TGX_OK; }
+  // Chunk k's first sample, sample count and text bytes once its blob + offsets are (queued to be) in set b.  May wait.
+  virtual int samples(tgx_model* m, uint64_t k, int b, uint64_t* s0, uint64_t* S, uint64_t* n) = 0;
+};
+
+// Output stage: takes chunk k's ids (m->ids / m->ids_b), id offsets (chunk-relative) and per-sample status / length.
+struct ChunkOutput {
+  virtual ~ChunkOutput() = default;
+  // Queued on the compute stream behind the chunk's encode kernels.
+  virtual int after_encode(tgx_model*, uint64_t, int, uint64_t) { return TGX_OK; }
+  // Queues the D2H copies of chunk k on `st` (its kernels have finished); `tot` ids, `base` ids in earlier chunks.
+  // `bad` = the chunk's lowest sample without a path (-1 = none).
+  virtual int d2h(tgx_model* m, uint64_t k, int b, uint64_t s0, uint64_t S, uint64_t tot, uint64_t base, int64_t bad,
+                  const int32_t* d_status, const uint64_t* d_plen, cudaStream_t st) = 0;
+};
+
+DevBuf* set_text(tgx_model* m, int b) { return b ? &m->text_b : &m->text; }
+DevBuf* set_off(tgx_model* m, int b) { return b ? &m->off_b : &m->off; }
+DevBuf* set_ids(tgx_model* m, int b) { return b ? &m->ids_b : &m->ids; }
+DevBuf* set_idoff(tgx_model* m, int b) { return b ? &m->idoff_b : &m->idoff; }
+DevBuf* set_sc(tgx_model* m, int b) { return b ? &m->scount_b : &m->scount; }
+
+// Runs the pipeline; *bad_all = lowest failing sample (-1 = none), *total = ids of all chunks, *stop = the input stage
+// refused a chunk (its status; the chunks before it are encoded).  Returns with every copy finished.
+int encode_chunks(tgx_model* m, uint32_t flags, uint64_t unit_base, ChunkInput& in, ChunkOutput& out,
+                  int64_t* bad_all_out, uint64_t* total) {
+  const uint64_t K = in.K;
   const int nset = K > 1 ? 2 : 1;
   for (int i = 0; i < nset; i++) {
-    CU(d_text[i]->reserve(max_b + 16));
-    CU(d_off[i]->reserve((max_s + 1) * 8));
-    CU(d_ids[i]->reserve((max_b + 4) * 4));
-    CU(d_idoff[i]->reserve((max_s + 1) * 8));
-    CU(d_sc[i]->reserve((max_s + 1) * 12 + 32));
+    CU(set_text(m, i)->reserve(in.max_b + 16));
+    CU(set_off(m, i)->reserve((in.max_s + 1) * 8));
+    CU(set_ids(m, i)->reserve((in.max_b + 4) * 4));
+    CU(set_idoff(m, i)->reserve((in.max_s + 1) * 8));
+    CU(set_sc(m, i)->reserve((in.max_s + 1) * 12 + 32));
   }
-  // rebased offsets travel through pinned staging (one slice per chunk, alive until the end)
-  if (m->h_off_cap < S + K + 1) {
-    if (m->h_off) cudaFreeHost(m->h_off);
-    m->h_off = nullptr;
-    m->h_off_cap = 0;
-    CU(cudaHostAlloc(reinterpret_cast<void**>(&m->h_off), (S + K + 1) * 8, cudaHostAllocDefault));
-    m->h_off_cap = S + K + 1;
-  }
-  const uint64_t so_idoff = 0, so_status = (S + K + 1) * 8, so_plen = so_status + ((S * 4 + 15) & ~15ull);
-  const uint64_t out_bytes = so_plen + S * 8 + 16;
-  if (m->h_out_cap < out_bytes) {
-    if (m->h_out) cudaFreeHost(m->h_out);
-    m->h_out = nullptr;
-    m->h_out_cap = 0;
-    CU(cudaHostAlloc(reinterpret_cast<void**>(&m->h_out), out_bytes, cudaHostAllocDefault));
-    m->h_out_cap = out_bytes;
-  }
-  uint64_t* st_idoff = reinterpret_cast<uint64_t*>(m->h_out + so_idoff);  // chunk k's S_k + 1 entries at [s0 + k ..]
-  int32_t* st_status = reinterpret_cast<int32_t*>(m->h_out + so_status);
-  uint64_t* st_plen = reinterpret_cast<uint64_t*>(m->h_out + so_plen);
+  auto reserve_samples = [&](uint64_t k, int b, uint64_t Sk) -> int {  // (chunks split on the device only)
+    if ((Sk + 1) * 8 <= set_idoff(m, b)->cap && (Sk + 1) * 12 + 32 <= set_sc(m, b)->cap) return TGX_OK;
+    if (K > 1 && k >= 2) CU(cudaEventSynchronize(m->ev_d2h[b]));  // the set's previous results left the device
+    CU(set_idoff(m, b)->reserve((Sk + 1) * 8));
+    CU(set_sc(m, b)->reserve((Sk + 1) * 12 + 32));
+    return TGX_OK;
+  };
   std::vector<cudaEvent_t> tev;  // trace: [base, per chunk: h2d0,h2d1,c0,c1,d2h0,d2h1]
+  const bool overlap = K > 1 && m->overlap_chunks;
   auto h2d = [&](uint64_t k) -> int {
     const int b = (int)(k & 1);
-    const uint64_t s0 = cut[k], s1 = cut[k + 1], b0 = off[s0], nb = off[s1] - b0;
-    uint64_t* ho = m->h_off + s0 + k;
-    for (uint64_t i = 0; i <= s1 - s0; i++) ho[i] = off[s0 + i] - b0;
     cudaStream_t st = K > 1 ? m->stream_h2d : m->w().stream;
     if (!tev.empty()) cudaEventRecord(tev[1 + 6 * k + 0], st);
-    if (nb) CU(cudaMemcpyAsync(d_text[b]->p, text + b0, nb, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_off[b]->p, ho, (s1 - s0 + 1) * 8, cudaMemcpyHostToDevice, st));
+    int r = in.h2d(m, k, b, st);
+    if (r) return r;
     if (!tev.empty()) cudaEventRecord(tev[1 + 6 * k + 1], st);
     if (K > 1) CU(cudaEventRecord(m->ev_h2d[b], st));
-    return TGX_OK;
+    const int wi = m->wi;
+    m->wi = overlap ? b : 0;
+    r = in.after_h2d(m, k, b);
+    m->wi = wi;
+    return r;
   };
   const bool trace = getenv("TGX_TRACE") != nullptr;
   auto now_ms = [] {
@@ -1676,83 +1843,87 @@ int tgx_encode_batch(tgx_model* m, const uint8_t* text, const uint64_t* off, uin
   //   H2D(k+1) on the copy-in stream, kernels(k+1) QUEUED on the other workspace before the host waits for
   //   chunk k, D2H(k) on the copy-out stream.  Queuing the next chunk early lets its kernels take over the SMs
   //   that chunk k's forward kernel frees while its last long samples finish on a few SMs.
-  const bool overlap = K > 1 && m->overlap_chunks;
+  std::vector<uint64_t> s0s(K, 0), Sks(K, 0), nbs(K, 0);
   auto enqueue = [&](uint64_t k) -> int {
     const int b = (int)(k & 1);
-    const uint64_t s0 = cut[k], s1 = cut[k + 1], Sk = s1 - s0, nb = off[s1] - off[s0];
     m->wi = overlap ? b : 0;
     if (K > 1) {
       CU(cudaStreamWaitEvent(m->w().stream, m->ev_h2d[b], 0));
       if (k >= 2) CU(cudaStreamWaitEvent(m->w().stream, m->ev_d2h[b], 0));  // the set's previous results left the device
     }
-    int32_t* dst = d_sc[b]->as<int32_t>();
-    uint64_t* dpl = reinterpret_cast<uint64_t*>(d_sc[b]->as<unsigned char>() + ((Sk * 4 + 15) & ~15ull));
+    uint64_t s0 = 0, Sk = 0, nb = 0;
+    int r = in.samples(m, k, b, &s0, &Sk, &nb);
+    if (r) return r;
+    s0s[k] = s0;
+    Sks[k] = Sk;
+    nbs[k] = nb;
+    if (Sk >= (1ull << 32)) return fail(TGX_ERR_UNSUPPORTED, "too many samples in one chunk (< 2^32)");
+    r = reserve_samples(k, b, Sk);
+    if (r) return r;
+    int32_t* dst = set_sc(m, b)->as<int32_t>();
+    uint64_t* dpl = reinterpret_cast<uint64_t*>(set_sc(m, b)->as<unsigned char>() + ((Sk * 4 + 15) & ~15ull));
     if (!tev.empty()) cudaEventRecord(tev[1 + 6 * k + 2], m->w().stream);
     if (Sk == 0) return TGX_OK;
-    m->drop_unit_base = cut[k];  // the draw is keyed by the sample's index in the whole call, not in its chunk
-    int r = encode_enqueue(m, d_text[b]->as<uint8_t>(), d_off[b]->as<uint64_t>(), Sk, nb, flags,
-                           d_ids[b]->as<uint32_t>(), nb + 4, d_idoff[b]->as<uint64_t>(), dst, dpl, true);
+    m->drop_unit_base = unit_base + s0;  // the draw is keyed by the sample's index in the whole input, not in its chunk
+    r = encode_enqueue(m, set_text(m, b)->as<uint8_t>(), set_off(m, b)->as<uint64_t>(), Sk, nb, flags,
+                       set_ids(m, b)->as<uint32_t>(), nb + 4, set_idoff(m, b)->as<uint64_t>(), dst, dpl, true);
+    if (r) return r;
+    r = out.after_encode(m, k, b, Sk);
     if (r) return r;
     if (!tev.empty()) cudaEventRecord(tev[1 + 6 * k + 3], m->w().stream);
     return TGX_OK;
   };
-  rc = h2d(0);
-  if (rc) return rc;
+  // (a failure below leaves copies in flight: callers' buffers are written until the streams drain)
+  auto drain = [&](int rc) {
+    if (K > 1) {
+      cudaStreamSynchronize(m->stream_h2d);
+      cudaStreamSynchronize(m->stream_d2h);
+    }
+    for (auto& w : m->ws) cudaStreamSynchronize(w.stream);
+    for (auto& e : tev) cudaEventDestroy(e);
+    return rc;
+  };
+  int rc = h2d(0);
+  if (rc) return drain(rc);
   rc = enqueue(0);
-  if (rc) return rc;
+  if (rc) return drain(rc);
   uint64_t base = 0;  // ids emitted by earlier chunks
-  std::vector<uint64_t> bases(K, 0);
   int64_t bad_all = -1;
-  bool overflow = false;
-  std::string keep_err;
-  int final_rc = TGX_OK;
   for (uint64_t k = 0; k < K; k++) {
     const int b = (int)(k & 1);
-    const uint64_t s0 = cut[k], s1 = cut[k + 1], Sk = s1 - s0;
     if (k + 1 < K) {
       rc = h2d(k + 1);
-      if (rc) return rc;
+      if (rc) return drain(rc);
       if (overlap) {
         rc = enqueue(k + 1);
-        if (rc) return rc;
+        if (rc) return drain(rc);
       }
     }
-    int32_t* dst = d_sc[b]->as<int32_t>();
-    uint64_t* dpl = reinterpret_cast<uint64_t*>(d_sc[b]->as<unsigned char>() + ((Sk * 4 + 15) & ~15ull));
+    const uint64_t s0 = s0s[k], Sk = Sks[k];
+    int32_t* dst = set_sc(m, b)->as<int32_t>();
+    uint64_t* dpl = reinterpret_cast<uint64_t*>(set_sc(m, b)->as<unsigned char>() + ((Sk * 4 + 15) & ~15ull));
     uint64_t tot = 0;
     int64_t bad = -1;
     m->wi = overlap ? b : 0;
     if (Sk) {
       rc = encode_finish(m, &tot, &bad);
-      if (rc) return rc;
+      if (rc) return drain(rc);
     }
     if (trace)
       fprintf(stderr, "[tgx] chunk %llu/%llu: kernels done at %.2f ms (device %.2f ms)\n", (unsigned long long)k,
               (unsigned long long)K, now_ms() - t_begin, m->last_stats.total_ms);
-    if (tot > off[s1] - off[s0] + 4) return fail(TGX_ERR_CUDA, "internal: more ids than bytes");
-    if (bad >= 0 && bad_all < 0) {
-      bad_all = (int64_t)s0 + bad;
-      keep_err = "no path for sample " + std::to_string(bad_all);
-      final_rc = TGX_ERR_NO_PATH;
-    }
+    if (tot > nbs[k] + 4) return drain(fail(TGX_ERR_CUDA, "internal: more ids than bytes"));
+    if (bad >= 0 && bad_all < 0) bad_all = (int64_t)(s0 + bad);
     cudaStream_t st = K > 1 ? m->stream_d2h : m->w().stream;  // the chunk's kernels have finished
     if (!tev.empty()) cudaEventRecord(tev[1 + 6 * k + 4], st);
-    if (Sk) {
-      CU(cudaMemcpyAsync(st_idoff + s0 + k, d_idoff[b]->p, (Sk + 1) * 8, cudaMemcpyDeviceToHost, st));
-      if (status) CU(cudaMemcpyAsync(st_status + s0, dst, Sk * 4, cudaMemcpyDeviceToHost, st));
-      if (proc_len) CU(cudaMemcpyAsync(st_plen + s0, dpl, Sk * 8, cudaMemcpyDeviceToHost, st));
-    } else {
-      st_idoff[s0 + k] = 0;
-    }
-    if (base + tot > ids_cap) overflow = true;
-    if (!overflow && tot) CU(cudaMemcpyAsync(ids + base, d_ids[b]->p, tot * 4, cudaMemcpyDeviceToHost, st));
+    rc = out.d2h(m, k, b, s0, Sk, tot, base, bad, dst, dpl, st);
+    if (rc) return drain(rc);
     if (K > 1) CU(cudaEventRecord(m->ev_d2h[b], st));
     if (!tev.empty()) cudaEventRecord(tev[1 + 6 * k + 5], st);
-    bases[k] = base;
     base += tot;
     if (!overlap && k + 1 < K) {
       rc = enqueue(k + 1);
-      if (rc) return rc;
+      if (rc) return drain(rc);
     }
   }
   CU(cudaStreamSynchronize(K > 1 ? m->stream_d2h : m->w().stream));
@@ -1768,18 +1939,361 @@ int tgx_encode_batch(tgx_model* m, const uint8_t* text, const uint64_t* off, uin
     }
     for (auto& e : tev) cudaEventDestroy(e);
   }
+  *bad_all_out = bad_all;
+  *total = base;
+  return TGX_OK;
+}
+
+// Input stage of tgx_encode_batch: the H2D copy of a chunk's packed text and its rebased offsets.
+struct PackedInput : ChunkInput {
+  const uint8_t* text;
+  const uint64_t* off;
+  std::vector<uint64_t> cut;  // first sample of every chunk
+  PackedInput(tgx_model* m, const uint8_t* text_, const uint64_t* off_, uint64_t S) : text(text_), off(off_) {
+    const uint64_t N = off[S];
+    K = std::max<uint64_t>(1, std::min<uint64_t>(16, (N + m->chunk_bytes - 1) / m->chunk_bytes));
+    cut.assign(K + 1, 0);
+    cut[K] = S;
+    for (uint64_t k = 1; k < K; k++) {
+      const uint64_t target = N / K * k;
+      uint64_t i = (uint64_t)(std::lower_bound(off, off + S + 1, target) - off);
+      cut[k] = std::min<uint64_t>(std::max<uint64_t>(i, cut[k - 1]), S);
+    }
+    for (uint64_t k = 0; k < K; k++) {
+      max_b = std::max(max_b, off[cut[k + 1]] - off[cut[k]]);
+      max_s = std::max(max_s, cut[k + 1] - cut[k]);
+    }
+  }
+  int h2d(tgx_model* m, uint64_t k, int b, cudaStream_t st) override {
+    const uint64_t s0 = cut[k], s1 = cut[k + 1], b0 = off[s0], nb = off[s1] - b0;
+    uint64_t* ho = m->h_off + s0 + k;  // rebased offsets travel through pinned staging (one slice per chunk)
+    for (uint64_t i = 0; i <= s1 - s0; i++) ho[i] = off[s0 + i] - b0;
+    if (nb) CU(cudaMemcpyAsync(set_text(m, b)->p, text + b0, nb, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(set_off(m, b)->p, ho, (s1 - s0 + 1) * 8, cudaMemcpyHostToDevice, st));
+    return TGX_OK;
+  }
+  int samples(tgx_model*, uint64_t k, int, uint64_t* s0, uint64_t* S, uint64_t* n) override {
+    *s0 = cut[k];
+    *S = cut[k + 1] - cut[k];
+    *n = off[cut[k + 1]] - off[cut[k]];
+    return TGX_OK;
+  }
+};
+
+// Output stage of tgx_encode_batch: u32 ids straight into the caller's buffer, id offsets / status / processed lengths
+// through pinned staging (rebased when every chunk is done).
+struct PackedOutput : ChunkOutput {
+  uint32_t* ids = nullptr;
+  uint64_t ids_cap = 0;
+  bool want_status = false, want_plen = false;
+  uint64_t* st_idoff = nullptr;  // chunk k's S_k + 1 entries at [s0 + k ..]
+  int32_t* st_status = nullptr;
+  uint64_t* st_plen = nullptr;
+  std::vector<uint64_t> bases;
+  bool overflow = false;
+  int d2h(tgx_model* m, uint64_t k, int b, uint64_t s0, uint64_t Sk, uint64_t tot, uint64_t base, int64_t,
+          const int32_t* dst, const uint64_t* dpl, cudaStream_t st) override {
+    if (Sk) {
+      CU(cudaMemcpyAsync(st_idoff + s0 + k, set_idoff(m, b)->p, (Sk + 1) * 8, cudaMemcpyDeviceToHost, st));
+      if (want_status) CU(cudaMemcpyAsync(st_status + s0, dst, Sk * 4, cudaMemcpyDeviceToHost, st));
+      if (want_plen) CU(cudaMemcpyAsync(st_plen + s0, dpl, Sk * 8, cudaMemcpyDeviceToHost, st));
+    } else {
+      st_idoff[s0 + k] = 0;
+    }
+    if (base + tot > ids_cap) overflow = true;
+    if (!overflow && tot) CU(cudaMemcpyAsync(ids + base, set_ids(m, b)->p, tot * 4, cudaMemcpyDeviceToHost, st));
+    bases[k] = base;
+    return TGX_OK;
+  }
+};
+
+// Input stage of tgx_encode_corpus: the H2D copy of a raw chunk (cut after a NUL byte) and its split on the device.
+// The split's counts are read back through the control stream.  They are queued behind the previous chunk's kernels,
+// so the host's wait for them in samples() comes right after its wait for that chunk and overlaps its encode.
+struct CorpusInput : ChunkInput {
+  const uint8_t* data;
+  std::vector<uint64_t> cut;  // first byte of every chunk
+  uint64_t next_s0 = 0;       // samples in the chunks split so far
+  int64_t bad_sample = -1;    // lowest sample that is not UTF-8 (relative to the buffer), once samples() refused it
+  double split_ms = 0;        // device time of the split kernels, all chunks
+  CorpusInput(tgx_model* m, const uint8_t* data_, uint64_t n) : data(data_) {
+    K = std::max<uint64_t>(1, std::min<uint64_t>(16, (n + m->chunk_bytes - 1) / m->chunk_bytes));
+    cut.assign(K + 1, n);
+    cut[0] = 0;
+    for (uint64_t k = 1; k < K; k++) {  // after the first NUL at or beyond the target: a long sample enlarges its chunk
+      const uint64_t from = std::max<uint64_t>(n / K * k, cut[k - 1]);
+      const void* z = from < n ? memchr(data + from, 0, n - from) : nullptr;
+      cut[k] = z ? (uint64_t)(static_cast<const uint8_t*>(z) - data) + 1 : n;
+    }
+    for (uint64_t k = 0; k < K; k++) max_b = std::max(max_b, cut[k + 1] - cut[k]);
+  }
+  int h2d(tgx_model* m, uint64_t k, int b, cudaStream_t st) override {
+    const uint64_t nb = cut[k + 1] - cut[k];
+    CU(m->raw[b].reserve(max_b + 16));
+    if (nb) CU(cudaMemcpyAsync(m->raw[b].p, data + cut[k], nb, cudaMemcpyHostToDevice, st));
+    return TGX_OK;
+  }
+  KeptStarts* tile_counts(tgx_model* m, int b) { return reinterpret_cast<KeptStarts*>(m->split[b].as<unsigned char>() + 32); }
+  int after_h2d(tgx_model* m, uint64_t k, int b) override {
+    cudaStream_t st = m->w().stream;
+    if (K > 1) CU(cudaStreamWaitEvent(st, m->ev_h2d[b], 0));
+    const uint64_t N = cut[k + 1] - cut[k], n_tiles = (N + CRLF_TILE - 1) / CRLF_TILE;
+    // m->split[b]: bad_pos, words[3], tile counts (n_tiles + 1), their exclusive scan (n_tiles + 1)
+    CU(m->split[b].reserve(32 + (n_tiles + 1) * 2 * sizeof(KeptStarts)));
+    unsigned long long* bad_pos = m->split[b].as<unsigned long long>();
+    unsigned long long* words = bad_pos + 1;
+    KeptStarts* cnt = tile_counts(m, b);
+    KeptStarts* prefix = cnt + n_tiles + 1;
+    CU(cudaEventRecord(m->ev_split[b][0], st));
+    CU(dev_fill(bad_pos, 0xFF, 8, st));
+    CU(dev_fill(cnt + n_tiles, 0, sizeof(KeptStarts), st));
+    const uint8_t* raw = m->raw[b].as<uint8_t>();
+    if (n_tiles) corpus_count<<<(uint32_t)n_tiles, CRLF_BLOCK, 0, st>>>(raw, N, cnt, bad_pos);
+    size_t tmp = 0;
+    CU(cub::DeviceScan::ExclusiveScan(nullptr, tmp, cnt, prefix, AddKeptStarts(), KeptStarts{0, 0}, (int)(n_tiles + 1),
+                                      st));
+    CU(m->w().cubtmp.reserve(tmp));
+    CU(cub::DeviceScan::ExclusiveScan(m->w().cubtmp.p, tmp, cnt, prefix, AddKeptStarts(), KeptStarts{0, 0},
+                                      (int)(n_tiles + 1), st));
+    corpus_words<<<1, 32, 0, st>>>(raw, prefix, n_tiles, bad_pos, words);
+    CU(cudaGetLastError());
+    CU(cudaEventRecord(m->ev_split[b][1], st));
+    CU(cudaEventRecord(m->w().ev_ctl, st));
+    CU(cudaStreamWaitEvent(m->w().stream_ctl, m->w().ev_ctl, 0));
+    CU(cudaMemcpyAsync(m->w().h_words + 4, words, 24, cudaMemcpyDeviceToHost, m->w().stream_ctl));
+    return TGX_OK;
+  }
+  int samples(tgx_model* m, uint64_t k, int b, uint64_t* s0, uint64_t* S, uint64_t* n) override {
+    CU(cudaStreamSynchronize(m->w().stream_ctl));
+    const uint64_t Sk = m->w().h_words[4], kept = m->w().h_words[5], bad = m->w().h_words[6];
+    float ms = 0;
+    if (cudaEventElapsedTime(&ms, m->ev_split[b][0], m->ev_split[b][1]) == cudaSuccess) split_ms += ms;
+    if (bad != ~0ull) {
+      bad_sample = (int64_t)(next_s0 + bad);
+      return fail(TGX_ERR_NOT_UTF8, "sample " + std::to_string(bad_sample) + " is not valid UTF-8");
+    }
+    const uint64_t N = cut[k + 1] - cut[k], n_tiles = (N + CRLF_TILE - 1) / CRLF_TILE;
+    if (N >= (1ull << 32)) {  // (the kernels index the positions of a sample with 32 bits)
+      for (uint64_t p = cut[k]; p < cut[k + 1];) {
+        const void* z = memchr(data + p, 0, cut[k + 1] - p);
+        const uint64_t e = z ? (uint64_t)(static_cast<const uint8_t*>(z) - data) : cut[k + 1];
+        if (e - p >= (1ull << 32)) return fail(TGX_ERR_UNSUPPORTED, "a sample of 4 GiB or more is not supported");
+        p = e + 1;
+      }
+    }
+    CU(set_off(m, b)->reserve((Sk + 1) * 8));
+    cudaStream_t st = m->w().stream;
+    CU(cudaEventRecord(m->ev_split[b][2], st));
+    if (n_tiles)
+      corpus_scatter<<<(uint32_t)n_tiles, CRLF_BLOCK, 0, st>>>(m->raw[b].as<uint8_t>(), N, tile_counts(m, b) + n_tiles + 1,
+                                                               n_tiles, set_text(m, b)->as<uint8_t>(),
+                                                               set_off(m, b)->as<uint64_t>());
+    CU(cudaGetLastError());
+    CU(cudaEventRecord(m->ev_split[b][3], st));
+    *s0 = next_s0;
+    *S = Sk;
+    *n = kept;
+    next_s0 += Sk;
+    return TGX_OK;
+  }
+  void add_scatter_ms(tgx_model* m, int b) {  // (chunk's kernels have finished)
+    float ms = 0;
+    if (cudaEventElapsedTime(&ms, m->ev_split[b][2], m->ev_split[b][3]) == cudaSuccess) split_ms += ms;
+  }
+};
+
+// Output stage of tgx_encode_corpus: the ids narrowed and separated by corpus_finalize (or the u32 ids as they are)
+// and the id offsets straight into the caller's buffers; the offsets are rebased when every chunk is done.
+struct CorpusOutput : ChunkOutput {
+  CorpusInput* in = nullptr;
+  int64_t sep = -1;
+  uint32_t id_bytes = 4;
+  unsigned char* ids = nullptr;
+  uint64_t ids_cap = 0, off_cap = 0;
+  uint64_t* id_off = nullptr;
+  std::vector<uint64_t> bases, s0s;
+  bool ids_overflow = false, off_overflow = false;
+  int64_t bad = -1;  // lowest sample without a path (relative to the buffer) and its length after processing
+  uint64_t bad_len = 0;
+  bool finalize() const { return sep >= 0 || id_bytes == 2; }
+  int after_encode(tgx_model* m, uint64_t, int b, uint64_t Sk) override {
+    if (!finalize()) return TGX_OK;
+    CU(m->fin[b].reserve((in->max_b + 4 + Sk) * id_bytes));
+    cudaStream_t st = m->w().stream;
+    const uint32_t grid = (uint32_t)m->num_sms * 8;
+    const uint32_t* d_ids = set_ids(m, b)->as<uint32_t>();
+    const uint64_t* d_idoff = set_idoff(m, b)->as<uint64_t>();
+    if (id_bytes == 2)
+      corpus_finalize<uint16_t><<<grid, 256, 0, st>>>(d_ids, d_idoff, Sk, sep, m->fin[b].as<uint16_t>());
+    else
+      corpus_finalize<uint32_t><<<grid, 256, 0, st>>>(d_ids, d_idoff, Sk, sep, m->fin[b].as<uint32_t>());
+    m->w().stats.launches += 1;
+    CU(cudaGetLastError());
+    return TGX_OK;
+  }
+  int d2h(tgx_model* m, uint64_t k, int b, uint64_t s0, uint64_t Sk, uint64_t tot, uint64_t base, int64_t chunk_bad,
+          const int32_t*, const uint64_t* dpl, cudaStream_t st) override {
+    if (Sk) in->add_scatter_ms(m, b);  // (the encode that followed the scatter has finished)
+    bases[k] = base;
+    s0s[k] = s0;
+    if (bad < 0 && chunk_bad >= 0) {  // (error path: the length is read at once)
+      CU(cudaMemcpyAsync(&bad_len, dpl + chunk_bad, 8, cudaMemcpyDeviceToHost, st));
+      CU(cudaStreamSynchronize(st));
+      bad = (int64_t)s0 + chunk_bad;
+    }
+    if (s0 + Sk + 1 > off_cap) off_overflow = true;
+    if (!off_overflow && Sk) CU(cudaMemcpyAsync(id_off + s0, set_idoff(m, b)->p, Sk * 8, cudaMemcpyDeviceToHost, st));
+    const uint64_t n_out = tot + (sep >= 0 ? Sk : 0), at = base + (sep >= 0 ? s0 : 0);
+    if (at + n_out > ids_cap) ids_overflow = true;
+    if (!ids_overflow && n_out)
+      CU(cudaMemcpyAsync(ids + at * id_bytes, finalize() ? m->fin[b].p : set_ids(m, b)->p, n_out * id_bytes,
+                         cudaMemcpyDeviceToHost, st));
+    return TGX_OK;
+  }
+};
+
+}  // namespace
+
+int tgx_encode_batch(tgx_model* m, const uint8_t* text, const uint64_t* off, uint64_t S, uint32_t flags,
+                     uint32_t* ids, uint64_t ids_cap, uint64_t* id_off, int32_t* status, uint64_t* proc_len,
+                     int64_t* first_bad_out) {
+  int rc = check_model(m);
+  if (rc) return rc;
+  if (!off || !id_off || off[0] != 0) return fail(TGX_ERR_INVALID, "offsets must start at 0");
+  for (uint64_t i = 0; i < S; i++) {  // (the reference has no limit on a sample; the kernels index positions with 32 bits)
+    if (off[i + 1] < off[i]) return fail(TGX_ERR_INVALID, "offsets must not decrease");
+    if (off[i + 1] - off[i] >= (1ull << 32)) return fail(TGX_ERR_UNSUPPORTED, "a sample of 4 GiB or more is not supported");
+  }
+  std::lock_guard<std::recursive_mutex> g(m->mu);
+  struct WiGuard {  // whatever path leaves this function, the next call starts on workspace 0
+    tgx_model* m;
+    ~WiGuard() { m->wi = 0; }
+  } wi_guard{m};
+  if (first_bad_out) *first_bad_out = -1;
+  if (S == 0) {
+    id_off[0] = 0;
+    return TGX_OK;
+  }
+  PackedInput in(m, text, off, S);
+  const uint64_t K = in.K;
+  // rebased offsets travel through pinned staging (one slice per chunk, alive until the end)
+  if (m->h_off_cap < S + K + 1) {
+    if (m->h_off) cudaFreeHost(m->h_off);
+    m->h_off = nullptr;
+    m->h_off_cap = 0;
+    CU(cudaHostAlloc(reinterpret_cast<void**>(&m->h_off), (S + K + 1) * 8, cudaHostAllocDefault));
+    m->h_off_cap = S + K + 1;
+  }
+  const uint64_t so_idoff = 0, so_status = (S + K + 1) * 8, so_plen = so_status + ((S * 4 + 15) & ~15ull);
+  const uint64_t out_bytes = so_plen + S * 8 + 16;
+  if (m->h_out_cap < out_bytes) {
+    if (m->h_out) cudaFreeHost(m->h_out);
+    m->h_out = nullptr;
+    m->h_out_cap = 0;
+    CU(cudaHostAlloc(reinterpret_cast<void**>(&m->h_out), out_bytes, cudaHostAllocDefault));
+    m->h_out_cap = out_bytes;
+  }
+  PackedOutput out;
+  out.ids = ids;
+  out.ids_cap = ids_cap;
+  out.want_status = status != nullptr;
+  out.want_plen = proc_len != nullptr;
+  out.st_idoff = reinterpret_cast<uint64_t*>(m->h_out + so_idoff);
+  out.st_status = reinterpret_cast<int32_t*>(m->h_out + so_status);
+  out.st_plen = reinterpret_cast<uint64_t*>(m->h_out + so_plen);
+  out.bases.assign(K, 0);
+  int64_t bad_all = -1;
+  uint64_t base = 0;
+  rc = encode_chunks(m, flags, 0, in, out, &bad_all, &base);
+  if (rc) return rc;
   // chunk-relative id offsets -> global; small outputs leave the pinned staging
   for (uint64_t k = 0; k < K; k++) {
-    const uint64_t add = bases[k];
-    const uint64_t* src = st_idoff + cut[k] + k;
-    for (uint64_t s = cut[k]; s < cut[k + 1]; s++) id_off[s] = src[s - cut[k]] + add;
+    const uint64_t add = out.bases[k];
+    const uint64_t* src = out.st_idoff + in.cut[k] + k;
+    for (uint64_t s = in.cut[k]; s < in.cut[k + 1]; s++) id_off[s] = src[s - in.cut[k]] + add;
   }
   id_off[S] = base;
-  if (status) std::memcpy(status, st_status, S * 4);
-  if (proc_len) std::memcpy(proc_len, st_plen, S * 8);
+  if (status) std::memcpy(status, out.st_status, S * 4);
+  if (proc_len) std::memcpy(proc_len, out.st_plen, S * 8);
   if (first_bad_out) *first_bad_out = bad_all;
-  if (overflow) return fail(TGX_ERR_CAPACITY, "ids capacity too small: need " + std::to_string(base));
-  if (final_rc == TGX_ERR_NO_PATH) return fail(final_rc, keep_err);
+  if (out.overflow) return fail(TGX_ERR_CAPACITY, "ids capacity too small: need " + std::to_string(base));
+  if (bad_all >= 0) return fail(TGX_ERR_NO_PATH, "no path for sample " + std::to_string(bad_all));
+  return TGX_OK;
+}
+
+int tgx_encode_corpus(tgx_model* m, const uint8_t* data, uint64_t n, uint32_t flags, uint64_t sample_base,
+                      int64_t sep_id, uint32_t id_bytes, void* ids, uint64_t ids_cap, uint64_t* id_off,
+                      uint64_t off_cap, uint64_t* n_samples, uint64_t* n_ids, int64_t* first_bad, uint64_t* bad_pos) {
+  int rc = check_model(m);
+  if (rc) return rc;
+  if ((!data && n) || !n_samples || !n_ids || (!ids && ids_cap) || (!id_off && off_cap))
+    return fail(TGX_ERR_INVALID, "null argument");
+  if (id_bytes != 2 && id_bytes != 4) return fail(TGX_ERR_INVALID, "id_bytes must be 2 or 4");
+  if (sep_id < -1 || sep_id >= (int64_t)1 << 32) return fail(TGX_ERR_INVALID, "sep_id must be -1 or a u32 id");
+  if (id_bytes == 2 && (m->V > 65536 || sep_id >= 65536))
+    return fail(TGX_ERR_UNSUPPORTED, "16-bit ids need a vocabulary (and separator) below 65536");
+  std::lock_guard<std::recursive_mutex> g(m->mu);
+  struct WiGuard {
+    tgx_model* m;
+    ~WiGuard() { m->wi = 0; }
+  } wi_guard{m};
+  *n_samples = *n_ids = 0;
+  if (first_bad) *first_bad = -1;
+  if (bad_pos) *bad_pos = 0;
+  m->last_stats = Stats();
+  if (n == 0) {
+    if (off_cap < 1) return fail(TGX_ERR_CAPACITY, "offsets capacity too small: need 1");
+    id_off[0] = 0;
+    return TGX_OK;
+  }
+  CorpusInput in(m, data, n);
+  CorpusOutput out;
+  out.in = &in;
+  out.sep = sep_id;
+  out.id_bytes = id_bytes;
+  out.ids = static_cast<unsigned char*>(ids);
+  out.ids_cap = ids_cap;
+  out.id_off = id_off;
+  out.off_cap = off_cap;
+  out.bases.assign(in.K, 0);
+  out.s0s.assign(in.K, 0);
+  int64_t bad_all = -1;
+  uint64_t base = 0;
+  rc = encode_chunks(m, flags, sample_base, in, out, &bad_all, &base);
+  m->last_stats.split_ms = in.split_ms;
+  if (rc == TGX_ERR_NOT_UTF8) {  // (lowest invalid sample: the chunks are split in order and stop at the first)
+    if (first_bad) *first_bad = in.bad_sample;
+    if (bad_pos) {  // byte offset of that sample's first byte: walk the non-empty samples of the buffer
+      uint64_t p = 0;
+      for (int64_t s = -1;;) {
+        while (p < n && data[p] == 0) p++;
+        if (++s == in.bad_sample) break;
+        const void* z = memchr(data + p, 0, n - p);
+        p = z ? (uint64_t)(static_cast<const uint8_t*>(z) - data) : n;
+      }
+      *bad_pos = p;
+    }
+    return rc;
+  }
+  if (rc) return rc;
+  const uint64_t S = in.next_s0;
+  const uint64_t total = base + (sep_id >= 0 ? S : 0);
+  *n_samples = S;
+  *n_ids = total;
+  if (out.off_overflow || S + 1 > off_cap)
+    return fail(TGX_ERR_CAPACITY, "offsets capacity too small: need " + std::to_string(S + 1));
+  // chunk-relative id offsets -> global, separators counted
+  for (uint64_t k = 0; k < in.K; k++) {
+    const uint64_t s0 = out.s0s[k], s1 = k + 1 < in.K ? out.s0s[k + 1] : S;
+    for (uint64_t s = s0; s < s1; s++) id_off[s] += out.bases[k] + (sep_id >= 0 ? s : 0);
+  }
+  id_off[S] = total;
+  if (out.ids_overflow) return fail(TGX_ERR_CAPACITY, "ids capacity too small: need " + std::to_string(total));
+  if (bad_all >= 0) {
+    if (first_bad) *first_bad = bad_all;
+    if (bad_pos) *bad_pos = out.bad_len;
+    return fail(TGX_ERR_NO_PATH, "no path for sample " + std::to_string(bad_all));
+  }
   return TGX_OK;
 }
 

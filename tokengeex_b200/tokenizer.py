@@ -134,6 +134,20 @@ def id_rows(ids: np.ndarray, id_off: np.ndarray) -> List[List[int]]:
     return [flat[cut[i]:cut[i + 1]] for i in range(n)]
 
 
+def corpus_layout(ids: np.ndarray, id_off: np.ndarray, sep_id: int, dt: np.dtype) -> Tuple[np.ndarray, np.ndarray]:
+    """u32 ids + offsets → the output of encode_corpus: ids as `dt`, `sep_id` (if >= 0) after every sample."""
+    id_off = np.asarray(id_off, np.uint64)
+    if sep_id < 0:
+        return np.asarray(ids).astype(dt), id_off.copy()
+    S = len(id_off) - 1
+    lens = np.diff(id_off).astype(np.int64)
+    out = np.empty(len(ids) + S, dt)
+    rows = np.repeat(np.arange(S, dtype=np.int64), lens)
+    out[np.arange(len(ids), dtype=np.int64) + rows] = ids
+    out[id_off[1:].astype(np.int64) + np.arange(S, dtype=np.int64)] = sep_id
+    return out, id_off + np.arange(S + 1, dtype=np.uint64)
+
+
 class Tokenizer:
     """tokengeex.Tokenizer (bindings/python/tokengeex.pyi:10-255)."""
 
@@ -444,6 +458,96 @@ class Tokenizer:
 
     def encode_ordinary_batch(self, texts: List[str], dropout: float) -> List[List[int]]:
         return self._encode_many(texts, dropout, ordinary=True)
+
+    # ---- corpus images (tokengeex_b200/corpus.py) -------------------------------------------------------------
+    def corpus_dtype(self, dtype=None) -> np.dtype:
+        """dtype=None: uint16 when every id fits (vocab_size() <= 65536), else uint32."""
+        if dtype is None:
+            return np.dtype(np.uint16 if self.vocab_size() <= 65536 else np.uint32)
+        dt = np.dtype(dtype)
+        if dt not in (np.dtype(np.uint16), np.dtype(np.uint32)):
+            raise TokenGeeXError(f"unsupported id dtype {dt}: uint16 or uint32")
+        return dt
+
+    def separator_id(self, separator: Optional[str]) -> int:
+        """-1 for None, else the id of the token (usually a special token such as "<eos>")."""
+        if separator is None:
+            return -1
+        i = self.token_to_id(separator.encode("utf-8"))
+        if i is None:
+            raise TokenGeeXError(f"unknown separator token {separator!r}")
+        return i
+
+    def corpus_on_device(self) -> bool:
+        """The device splits the corpus when the processors are [] or exactly [crlf] (crlf twice is not crlf once:
+        "\r\r\n"); any other list takes the host path of encode_corpus."""
+        return [p.kind for p in self._processors] in ([], ["crlf"])
+
+    def encode_corpus(self, data, dropout: float = 0.0, separator: Optional[str] = None, dtype=None,
+                      source: str = "<corpus>"):
+        """Ordinary encoding (special tokens in the text are not split out) of every non-empty sample of a
+        NUL-separated corpus image (bytes-like or uint8 array), as `load_sources` + `Model::encode` would do.
+        → (ids, offsets u64[S+1]): sample i (and its separator) is ids[offsets[i]:offsets[i+1]].  Invalid UTF-8
+        raises ValueError with load_sources' text (`source` names the file in it)."""
+        arr = data if isinstance(data, np.ndarray) else np.frombuffer(data, np.uint8)
+        seed = self.dropout_seed if self.dropout_seed is not None else secrets.randbits(64)
+        return self._encode_corpus(np.ascontiguousarray(arr, np.uint8).reshape(-1), dropout, self.separator_id(separator),
+                                   self.corpus_dtype(dtype), 0, seed, source)
+
+    def _encode_corpus(self, arr: np.ndarray, dropout: float, sep_id: int, dt: np.dtype, sample_base: int, seed: int,
+                       source: str, ids_out=None, off_out=None):
+        if dt == np.uint16 and (len(self._tokens) > 65536 or sep_id >= 65536):
+            raise TokenGeeXError("uint16 ids need a vocabulary (and separator) below 65536")
+        if not self.corpus_on_device():
+            return self._encode_corpus_host(arr, dropout, sep_id, dt, seed, source)
+        model = self._dev(dropout)
+        drawn = 0.0 < dropout < 1.0
+        try:
+            with self._dropout_lock:
+                if drawn:
+                    model.set_dropout(dropout, seed)
+                try:
+                    ids, off, rc, bad, pos = model.encode_corpus(arr, crlf=bool(self._processors),
+                                                                 sample_base=sample_base, sep_id=sep_id, dtype=dt,
+                                                                 ids_out=ids_out, off_out=off_out)
+                finally:
+                    if drawn:
+                        model.set_dropout(0.0, 0)
+        except N.TgxError as e:
+            raise TokenGeeXError(e.msg)
+        if rc == N.TGX_ERR_NOT_UTF8:
+            z = np.flatnonzero(arr[pos:] == 0)
+            end = pos + int(z[0]) if z.size else arr.size
+            try:
+                arr[pos:end].tobytes().decode("utf-8")
+            except UnicodeDecodeError as e:
+                raise ValueError(f"Sample in {source!r} is not valid UTF-8: {e}") from None
+            raise TokenGeeXError(f"sample {bad} reported as invalid UTF-8 decodes on the host")
+        if rc == N.TGX_ERR_NO_PATH:
+            raise TokenGeeXError(f"no path to position {pos}/{pos}")  # Display of Error::NoPath, src/lib.rs:243-245
+        return ids, off
+
+    def _encode_corpus_host(self, arr: np.ndarray, dropout: float, sep_id: int, dt: np.dtype, seed: int, source: str):
+        """load_sources' split, check and processors on the host, then Model.encode_batch and the same layout."""
+        samples = []
+        for piece in arr.tobytes().split(b"\x00"):
+            if not piece:
+                continue
+            try:
+                s = piece.decode("utf-8")
+            except UnicodeDecodeError as e:
+                raise ValueError(f"Sample in {source!r} is not valid UTF-8: {e}") from None
+            for p in self._processors:
+                s = p.preprocess(s)
+            if s:
+                samples.append(s.encode("utf-8"))
+        saved = self.dropout_seed
+        self.dropout_seed = seed
+        try:
+            ids, id_off = self._encode_pieces(samples, False, dropout)
+        finally:
+            self.dropout_seed = saved
+        return corpus_layout(ids, id_off, sep_id, dt)
 
     # ---- decode (src/tokenizer.rs:126-187, src/model.rs:146-160) ------------------------------------------
     def _decode_base(self, ids: Sequence[int]) -> str:
