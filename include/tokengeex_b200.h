@@ -152,9 +152,12 @@ int tgx_expected_counts_dev(tgx_model* m, const uint8_t* d_text, const uint64_t*
  * point with integer atomics, so a count is the EXACT sum of its contributions (each truncated to 2^-128) —
  * bit-identical from run to run, for every chunking of the corpus and, after an integer (int64 SUM) all-reduce of the
  * limbs, for every number of GPUs — where the reference's f64 sum depends on rayon's completion order
- * (src/prune.rs:104-112).  Counts below ~1e-29 are below the resolution (the M-step's only threshold is 0.5).
- * tgx_counts_from_limbs_dev turns (summed) limbs into the f64 vector the M-step reads: expected[id] = value (overwritten).
- * tgx_expected_counts{,_dev} are this followed by that conversion. */
+ * (src/prune.rs:104-112).  Counts below ~1e-29 are below the resolution (the M-step's only threshold is 0.5).  A single
+ * contribution must be below 2^64, the range of the integer word; only a lattice with positions nothing begins at
+ * (beta = log 1 there, src/lattice.rs:275-287: vocabularies without every byte) can exceed it.
+ * tgx_counts_from_limbs_dev turns (summed) limbs into the f64 vector the M-step reads: expected[id] = the exact sum
+ * rounded to the nearest f64 (ties to even), overwritten.  tgx_expected_counts{,_dev} are this followed by that
+ * conversion, so their f64 counts are the same correctly rounded values. */
 int tgx_expected_counts_fixed_dev(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint64_t S,
                                   uint64_t n_bytes, uint64_t snippet_len, int64_t* d_limbs, int64_t* bad_sample,
                                   double* bad_z);

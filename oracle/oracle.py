@@ -70,6 +70,12 @@ def lib() -> C.CDLL:
         L.orc_run_e_step_dropout.restype = C.c_int
         L.orc_run_e_step_dropout.argtypes = [C.c_void_p, u8p, u64p, C.c_uint64, C.c_int, C.c_uint64, C.c_double,
                                              C.c_int, C.c_uint64, C.c_uint64, f64p, i64p, f64p]
+        L.orc_run_e_step_fixed.restype = C.c_int
+        L.orc_run_e_step_fixed.argtypes = [C.c_void_p, u8p, u64p, C.c_uint64, C.c_int, C.c_uint64, C.c_double,
+                                           C.c_int, C.c_uint64, C.c_uint64, u64p, i64p, f64p]
+        L.orc_marginal_contributions.restype = C.c_double
+        L.orc_marginal_contributions.argtypes = [C.c_void_p, u8p, C.c_uint64, u32p, f64p, C.c_uint64, u64p,
+                                                 C.c_double, C.c_uint64, C.c_uint64]
         L.orc_digamma.restype = C.c_double
         L.orc_digamma.argtypes = [C.c_double]
         L.orc_log_sum_exp.restype = C.c_double
@@ -255,6 +261,35 @@ class OracleModel:
                                       max_sample_length, dropout, int(keyed), seed & 0xFFFFFFFFFFFFFFFF, byte_base,
                                       _p(ex, f64p), C.byref(bad), C.byref(badz))
         return ex, rc, int(bad.value), float(badz.value)
+
+    def run_e_step_fixed(self, blob: np.ndarray, off: np.ndarray, dropout: float = 0.0, seed: int = 0,
+                         keyed: bool = True, byte_base: int = 0, threads: int = 1, max_sample_length: int = 81920):
+        """run_e_step (dropout 0) or run_e_step_dropout with exact sums: → (counts, rc, bad_sample), counts[id] = the
+        Python int sum(floor(c * 2^128)) over token id's contributions c."""
+        L = lib()
+        fx = np.zeros((max(self.V, 1), 3), np.uint64)
+        bad = C.c_int64(-1)
+        badz = C.c_double(0.0)
+        rc = L.orc_run_e_step_fixed(self._h, _p(blob, u8p), _p(off, u64p), len(off) - 1, threads, max_sample_length,
+                                    dropout, int(keyed), seed & 0xFFFFFFFFFFFFFFFF, byte_base, _p(fx, u64p),
+                                    C.byref(bad), C.byref(badz))
+        counts = [int(w0) | (int(w1) << 64) | (int(w2) << 128) for w0, w1, w2 in fx[:self.V].tolist()]
+        return counts, rc, int(bad.value)
+
+    def marginal_contributions(self, text: bytes, dropout: float = 0.0, seed: int = 0, byte_base: int = 0):
+        """(z, [(id, contribution), ...]) of one lattice, in the order populate_marginal adds them.  dropout > 0: the
+        keyed draw of run_e_step_fixed, `text` starting at byte `byte_base` of the call's text."""
+        L = lib()
+        a = _bytes_arr(text)
+        n = C.c_uint64(0)
+        args = (dropout, seed & 0xFFFFFFFFFFFFFFFF, byte_base)
+        L.orc_marginal_contributions(self._h, _p(a, u8p), len(text), None, None, 0, C.byref(n), *args)
+        k = int(n.value)
+        ids = np.zeros(max(k, 1), np.uint32)
+        vals = np.zeros(max(k, 1), np.float64)
+        z = L.orc_marginal_contributions(self._h, _p(a, u8p), len(text), _p(ids, u32p), _p(vals, f64p), k,
+                                         C.byref(n), *args)
+        return float(z), list(zip(ids[:k].tolist(), vals[:k].tolist()))
 
     def run_m_step(self, expected: np.ndarray) -> "OracleModel":
         L = lib()

@@ -368,9 +368,50 @@ static inline double log_sum_exp(double x, double y, bool init_mode) {
   return vmax + std::log(std::exp(vmin - vmax) + 1.0);
 }
 
+// Exact fixed-point sums of the contributions (tests only): fixed[3 * id + 0 / 1 / 2] = bits 65..128 / bits 1..64 /
+// integer part of sum(floor(c * 2^128)) mod 2^192, a 192-bit integer kept as three u64 words (low to high).  The floor
+// is derived from c's significand and exponent, independently of the product's decomposition (acc_add).  The modulus
+// only matters for a contribution of 2^64 or more, which the product's accumulators cannot hold either; only a lattice
+// with positions nothing begins at (beta = log 1 there, src/lattice.rs:275-287) can produce one.
+static inline void fixed_merge(uint64_t* w, const uint64_t* x) {  // w += x (mod 2^192)
+  uint64_t carry = 0;
+  for (int k = 0; k < 3; k++) {
+    const unsigned __int128 t = (unsigned __int128)w[k] + x[k] + carry;
+    w[k] = (uint64_t)t;
+    carry = (uint64_t)(t >> 64);
+  }
+}
+static inline void fixed_add(uint64_t* w, double c) {
+  if (!(c > 0.0) || !std::isfinite(c)) return;  // exp() >= 0; a NaN only comes from a bad z (reported as such)
+  int e = 0;
+  const double f = std::frexp(c, &e);  // c = f * 2^e, f in [0.5, 1)
+  const uint64_t m = (uint64_t)std::ldexp(f, 53);  // exact: c = m * 2^(e - 53), m < 2^53
+  const int s = e - 53 + 128;  // c * 2^128 = m * 2^s
+  uint64_t add[3] = {0, 0, 0};
+  if (s < 0) {
+    if (s > -64) add[0] = m >> -s;  // the floor: the bits shifted out are dropped
+  } else {
+    const int wi = s / 64, b = s % 64;
+    if (wi < 3) add[wi] = m << b;
+    if (b && wi + 1 < 3) add[wi + 1] = m >> (64 - b);
+  }
+  fixed_merge(w, add);
+}
+
+// Optional outputs of the marginal functions beside expected[]: the exact fixed-point sums and / or the list of
+// (id, contribution) in the order they are added.
+struct MarginalSinks {
+  uint64_t* fixed = nullptr;                             // [V][3]
+  std::vector<std::pair<uint32_t, double>>* contribs = nullptr;
+  void add(uint32_t id, double c) const {
+    if (fixed) fixed_add(fixed + 3 * (size_t)id, c);
+    if (contribs) contribs->emplace_back(id, c);
+  }
+};
+
 // src/lattice.rs:245-312  Lattice::populate_marginal — literal restatement,
 // including the O(|begin|*|end|) double loops.
-static double populate_marginal(const Lattice& lat, double* expected) {
+static double populate_marginal(const Lattice& lat, double* expected, const MarginalSinks* sinks = nullptr) {
   size_t len = lat.len;
   size_t num_nodes = lat.nodes.size();
   std::vector<double> alpha(num_nodes, 0.0), beta(num_nodes, 0.0);
@@ -400,6 +441,7 @@ static double populate_marginal(const Lattice& lat, double* expected) {
       double total = a + score + b - z;
       double update = std::exp(total);
       expected[id] += update;
+      if (sinks) sinks->add(id, update);
     }
   }
   return z;
@@ -412,7 +454,7 @@ static double populate_marginal(const Lattice& lat, double* expected) {
 // is what the CPU baseline times and what the CUDA kernels restate.
 static double marginal_per_position(const Model& m, const uint8_t* s, size_t n, double* expected,
                                     std::vector<double>& A, std::vector<double>& B,
-                                    std::vector<uint8_t>& seen) {
+                                    std::vector<uint8_t>& seen, const MarginalSinks* sinks = nullptr) {
   A.assign(n + 1, 0.0);
   B.assign(n + 1, 0.0);
   seen.assign(n + 1, 0);
@@ -450,7 +492,9 @@ static double marginal_per_position(const Model& m, const uint8_t* s, size_t n, 
     common_prefix_search(m.trie, s + pos, n - pos, [&](uint32_t id, uint32_t len) {
       double sc = m.vocab[id].score;
       double total = a + sc + B[pos + len] - z;
-      expected[id] += std::exp(total);
+      const double update = std::exp(total);
+      expected[id] += update;
+      if (sinks) sinks->add(id, update);
     });
   }
   return z;
@@ -603,17 +647,24 @@ static void parallel_chunks(size_t n_items, size_t chunk, int threads, F&& f) {
 static int run_e_step(const Model& m, const uint8_t* blob, const uint64_t* off, size_t S,
                       int threads, int literal, size_t max_sample_length, double* expected_out,
                       int64_t* bad_sample, double* bad_z, double dropout = 0.0, const KeyedDraw* keyed = nullptr,
-                      uint64_t byte_base = 0) {
+                      uint64_t byte_base = 0, uint64_t* fixed_out = nullptr) {
   size_t V = m.vocab_size();
   size_t chunk = par_chunk_size(S, (size_t)std::max(1, threads), 8);  // :66
   size_t n_chunks = S ? (S + chunk - 1) / chunk : 0;
   std::vector<std::vector<double>> partial(n_chunks);
+  std::vector<std::vector<uint64_t>> partial_fixed(fixed_out ? n_chunks : 0);  // exact sums (fixed_out != null)
   std::atomic<int64_t> bad{-1};
   std::mutex bad_mu;
   double badz = 0.0;
   parallel_chunks(S, chunk, threads, [&](size_t c, size_t lo, size_t hi, int) {
     std::vector<double>& ef = partial[c];
     ef.assign(V, 0.0);  // :78
+    MarginalSinks sinks;
+    if (fixed_out) {
+      partial_fixed[c].assign(3 * V, 0);
+      sinks.fixed = partial_fixed[c].data();
+    }
+    const MarginalSinks* sk = fixed_out ? &sinks : nullptr;
     Lattice lat;
     std::vector<double> A, B;
     std::vector<uint8_t> seen;
@@ -627,9 +678,9 @@ static int run_e_step(const Model& m, const uint8_t* blob, const uint64_t* off, 
         if (literal || dropout > 0.0) {
           lat.from(p + o, sn);
           populate_nodes(m, lat, dropout, &rng, keyed, byte_base + off[s] + o);  // :87
-          z = populate_marginal(lat, ef.data());
+          z = populate_marginal(lat, ef.data(), sk);
         } else {
-          z = marginal_per_position(m, p + o, sn, ef.data(), A, B, seen);
+          z = marginal_per_position(m, p + o, sn, ef.data(), A, B, seen, sk);
         }
         if (!std::isnormal(z)) {  // :90-96 panic
           std::lock_guard<std::mutex> g(bad_mu);
@@ -641,6 +692,11 @@ static int run_e_step(const Model& m, const uint8_t* blob, const uint64_t* off, 
   for (size_t i = 0; i < V; i++) expected_out[i] = 0.0;
   for (size_t c = 0; c < n_chunks; c++)  // :104-112
     for (size_t i = 0; i < V; i++) expected_out[i] += partial[c][i];
+  if (fixed_out) {  // integer additions: the merge order does not matter
+    std::fill(fixed_out, fixed_out + 3 * V, 0);
+    for (size_t c = 0; c < n_chunks; c++)
+      for (size_t i = 0; i < V; i++) fixed_merge(fixed_out + 3 * i, partial_fixed[c].data() + 3 * i);
+  }
   *bad_sample = bad.load();
   *bad_z = badz;
   return bad.load() >= 0 ? 1 : 0;
@@ -1028,6 +1084,41 @@ int orc_run_e_step_dropout(orc_model* h, const uint8_t* blob, const uint64_t* of
   KeyedDraw kd(seed, ~0ull);
   return run_e_step(*h->m, blob, off, S, threads, 1, max_sample_length, expected, bad_sample, bad_z, dropout,
                     keyed ? &kd : nullptr, byte_base);
+}
+
+// run_e_step (dropout 0: the plain E-step; else as orc_run_e_step_dropout) with the exact sums beside the f64 ones:
+// fixed[3 * id + 0 / 1 / 2] = bits 65..128 / bits 1..64 / integer part of sum(floor(c * 2^128)) over token id's
+// contributions c.  The integer sums do not depend on the thread count or the order of the additions.
+int orc_run_e_step_fixed(orc_model* h, const uint8_t* blob, const uint64_t* off, uint64_t S, int threads,
+                         uint64_t max_sample_length, double dropout, int keyed, uint64_t seed, uint64_t byte_base,
+                         uint64_t* fixed, int64_t* bad_sample, double* bad_z) {
+  KeyedDraw kd(seed, ~0ull);
+  std::vector<double> ex(h->m->vocab_size());
+  return run_e_step(*h->m, blob, off, S, threads, dropout > 0.0 ? 1 : 0, max_sample_length, ex.data(), bad_sample,
+                    bad_z, dropout, keyed ? &kd : nullptr, byte_base, fixed);
+}
+
+// The contributions (id, exp(a + score + b - z)) of one lattice (populate_nodes + populate_marginal) in the order the
+// reference adds them.  dropout > 0: the keyed draw of orc_run_e_step_fixed, with the lattice's first byte at position
+// byte_base.  Writes at most cap of them; *count = their number.  Returns z.
+double orc_marginal_contributions(orc_model* h, const uint8_t* s, uint64_t n, uint32_t* ids_out, double* vals_out,
+                                  uint64_t cap, uint64_t* count, double dropout, uint64_t seed, uint64_t byte_base) {
+  Lattice lat;
+  uint64_t rng = 0;
+  KeyedDraw kd(seed, ~0ull);
+  lat.from(s, n);
+  populate_nodes(*h->m, lat, dropout, &rng, &kd, byte_base);
+  std::vector<double> ex(h->m->vocab_size(), 0.0);
+  std::vector<std::pair<uint32_t, double>> cs;
+  MarginalSinks sinks;
+  sinks.contribs = &cs;
+  const double z = populate_marginal(lat, ex.data(), &sinks);
+  for (size_t i = 0; i < cs.size() && i < cap; i++) {
+    ids_out[i] = cs[i].first;
+    vals_out[i] = cs[i].second;
+  }
+  *count = cs.size();
+  return z;
 }
 
 double orc_digamma(double x) { return digamma(x); }

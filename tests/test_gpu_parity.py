@@ -10,7 +10,7 @@ import numpy as np
 import pytest
 
 from oracle import oracle as O
-from tests.util import counts_rel_err, rand_samples, rand_vocab, split_ids, synth_setup
+from tests.util import counts_rel_err, estep_cfg, rand_samples, rand_vocab, split_ids, synth_setup
 
 pytestmark = pytest.mark.gpu
 
@@ -356,18 +356,6 @@ def test_token_frequencies_exact(N):
 
 
 # ----------------------------------------------------------------------------- E-step
-def estep_cfg(m, g):
-    """g = lanes per snippet of the lane-group kernels (lane-per-snippet kernels off); g = 0: every snippet below
-    the long threshold runs one lane each (fb_*_lane_kernel), the rest a warp each."""
-    if g in (0, -2, -3):  # 0: split form, lane kernels that walk the trie (the default); -2: the lane kernels over the
-        m.set_option(17, 1 << 30)  # match stream; -3: no beta array (fused backward + counts on the lane-group kernels)
-        m.set_option(2, 4)
-        m.set_option(19, {0: 1, -2: 2, -3: 0}[g])
-    else:
-        m.set_option(17, 0)
-        m.set_option(2, g)
-
-
 LATTICE_VOCAB = [(b"<", -3.0), (b" value", -6.0), (b">", -3.0), (b"DC value", -8.0), (b"<DC", -4.0),
                  (b"<DC value>", -12.0)]
 

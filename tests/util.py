@@ -35,6 +35,34 @@ def synth_setup(kind: int, seed: int, nbytes: int, vocab_size: int, max_len: int
     return blob, off, toks, sc, kp
 
 
+def estep_cfg(m, g):
+    """E-step kernel set of a device Model.  g = lanes per snippet of the lane-group kernels (lane-per-snippet kernels
+    off); g = 0: every snippet below the long threshold runs one lane each (fb_*_lane_kernel), the rest a warp each."""
+    if g in (0, -2, -3):  # 0: split form, lane kernels that walk the trie (the default); -2: the lane kernels over the
+        m.set_option(17, 1 << 30)  # match stream; -3: no beta array (fused backward + counts on the lane-group kernels)
+        m.set_option(2, 4)
+        m.set_option(19, {0: 1, -2: 2, -3: 0}[g])
+    else:
+        m.set_option(17, 0)
+        m.set_option(2, g)
+
+
+def fixed_point_samples(om, samples, snip, limit=2.0 ** 64):
+    """The samples whose every snippet has a path (z normal, so the E-step reports no error) and whose contributions
+    are all below `limit`.  The device's 192-bit accumulators hold contributions below 2^64; only a lattice with
+    positions nothing begins at (incomplete vocabularies: beta = log 1 there) can have larger ones."""
+    import math
+    out = []
+    for s in samples:
+        ok = True
+        for o in range(0, len(s), snip):
+            z, cs = om.marginal_contributions(s[o:o + snip])
+            ok = ok and math.isfinite(z) and z != 0.0 and all(c < limit for _, c in cs)
+        if ok:
+            out.append(s)
+    return out
+
+
 def split_ids(ids: np.ndarray, id_off: np.ndarray):
     return [ids[int(id_off[i]):int(id_off[i + 1])].tolist() for i in range(len(id_off) - 1)]
 

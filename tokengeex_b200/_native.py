@@ -320,7 +320,7 @@ class Model:
 
     def expected_counts_fixed_dev(self, d_text: int, d_off: int, S: int, n_bytes: int, d_limbs: int,
                                   snippet_len: int = SNIPPET_LEN):
-        """E-step with exact integer counts: d_limbs int64[3 V] += limbs (see include/tokengeex_b200.h).  → (rc, bad_sample, bad_z)"""
+        """E-step with exact integer counts: d_limbs int64[5 V] += limbs (see include/tokengeex_b200.h).  → (rc, bad_sample, bad_z)"""
         bad = C.c_int64(-1)
         badz = C.c_double(0.0)
         rc = lib().tgx_expected_counts_fixed_dev(self._h, d_text, d_off, S, n_bytes, snippet_len, d_limbs, C.byref(bad),

@@ -2462,7 +2462,7 @@ int tgx_pair_frequencies(tgx_model* m, const uint8_t* text, const uint64_t* off,
 // ---------------------------------------------------------------------------- E-step
 namespace {
 
-// The E-step over device-resident text.  Results: d_expected[V] += counts (f64) and / or d_limbs[3V] += counts as exact
+// The E-step over device-resident text.  Results: d_expected[V] += counts (f64) and / or d_limbs[5V] += counts as exact
 // integer limbs (tgx_expected_counts_fixed_dev); either may be null.
 int expected_counts_impl(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint64_t S, uint64_t n_bytes,
                          uint64_t snippet_len, double* d_expected, long long* d_limbs, int64_t* bad_sample,

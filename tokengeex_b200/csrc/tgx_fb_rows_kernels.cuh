@@ -297,10 +297,26 @@ __global__ void fold_hot_acc_kernel(const unsigned long long* __restrict__ hot_a
 // words of the 128-bit fraction, low to high, and the integer part) — int64 limbs that an integer all-reduce over any
 // number of ranks sums exactly (tgx_expected_counts_fixed_dev).
 constexpr int COUNT_LIMBS = 5;
+// X = ip * 2^128 + f1 * 2^64 + f0  ->  the f64 nearest to X * 2^-128 (ties to even).  X is normalised so that its top
+// 64 bits T start with a one; a sticky bit ORed into T's bit 0 stands for the bits below T (bit 0 is far below T's
+// rounding position, bit 10), so the one rounding of the u64 -> f64 conversion is the rounding of X itself.  The
+// scaling by a power of two is exact: every nonzero X * 2^-128 is at least 2^-128, a normal double.
 __device__ __host__ __forceinline__ double fixed_to_double(unsigned long long f0, unsigned long long f1,
                                                            unsigned long long ip) {
-  const double k = 1.0 / 18446744073709551616.0;  // 2^-64
-  return (double)ip + ((double)f1 + (double)f0 * k) * k;
+  int scale = 128;  // value = (hi * 2^128 + mid * 2^64 + lo) * 2^-scale
+  unsigned long long hi = ip, mid = f1, lo = f0;
+  if (!hi) { hi = mid; mid = lo; lo = 0; scale += 64; }
+  if (!hi) { hi = mid; mid = 0; scale += 64; }
+  if (!hi) return 0.0;
+#if defined(__CUDA_ARCH__)
+  const int s = __clzll((long long)hi);
+#else
+  const int s = __builtin_clzll(hi);
+#endif
+  const unsigned long long t = (hi << s) | (s ? mid >> (64 - s) : 0ull);
+  const unsigned long long sticky = ((mid << s) | lo) ? 1ull : 0ull;
+  // value ~ T * 2^(128 - s - scale); the power of two is built from its exponent field (it is at least 2^-191)
+  return (double)(t | sticky) * TGX_AS_F64((unsigned long long)(1023 + 128 - s - scale) << 52);
 }
 __global__ void export_acc_kernel(const unsigned long long* __restrict__ acc, uint32_t V, double* __restrict__ expected,
                                   long long* __restrict__ limbs) {
