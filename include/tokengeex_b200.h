@@ -278,8 +278,11 @@ int tgx_model_set_option(tgx_model* m, int key, int64_t value);
  * The setting belongs to the model handle and applies to the calls that follow it: threads that encode through one
  * handle with different dropout values serialise set + call themselves (tokengeex_b200/tokenizer.py holds a lock).
  * With dropout > 0 the forward pass runs on the pair kernel with the draw in its producers
- * (viterbi_pair_drop_kernel; lane-group viterbi_kernel<G, true> for tokens > 16 bytes) and the E-step on the lane kernels
- * over the match stream (fbr_split_kernel<true> / fbr_contrib_kernel<true>; lane-group kernels for tokens > 16 bytes). */
+ * (viterbi_pair_drop_kernel; lane-group viterbi_kernel<G, true> for tokens > 16 bytes).  The E-step draws in the kernels
+ * option 19 selects: by default (1) the lane kernels that walk the trie (fb_split_lane_kernel<true> /
+ * fb_contrib_kernel<true>), with 2 the lane kernels over the match stream (fbr_split_kernel<true> /
+ * fbr_contrib_kernel<true>), with 0 the lane-group kernels; snippets past the lane threshold (option 17) and tokens
+ * > 16 bytes always run on the lane-group kernels. */
 int tgx_model_set_dropout(tgx_model* m, double dropout, uint64_t seed);
 
 #ifdef __cplusplus

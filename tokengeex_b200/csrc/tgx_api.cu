@@ -830,8 +830,8 @@ int order_after_caller(tgx_model* m) {
   return TGX_OK;
 }
 
-// Token hash of the emit kernel (max_token_len <= 16 only); a vocabulary it cannot serve simply leaves hash.mask == 0
-// and emit walks the trie.  On failure nothing the model already holds has been touched.
+// Token hash of the emit kernel (max_token_len <= 16 only); in a rebuild, a vocabulary it cannot serve leaves
+// hash.mask == 0 and emit walks the trie.  On failure nothing the model already holds has been touched.
 // `built`: a token hash of this vocabulary that the caller has built already (beside the trie, on a thread of its own),
 // with the builder's message in `built_err`; null = build it here.
 int upload_aux_tables(tgx_model* m, const tgx::DoubleArray& da, const uint8_t* token_bytes, const uint64_t* token_offsets,
@@ -846,7 +846,11 @@ int upload_aux_tables(tgx_model* m, const tgx::DoubleArray& da, const uint8_t* t
     hash_ok = built_err->empty();
     if (hash_ok) h = std::move(*built);
   } else if (hash_ok) {
-    hash_ok = tgx::build_token_hash(token_bytes, token_offsets, V, &h).empty();
+    // (model creation: every vocabulary of 1..16-byte tokens gets its hash unless two distinct tokens share their key
+    //  under every seed, i.e. the key function is broken — reported, not hidden behind the trie walk.  A rebuild builds
+    //  the hash beside the trie and must leave the model unchanged on failure, so it keeps the trie walk instead.)
+    const std::string herr = tgx::build_token_hash(token_bytes, token_offsets, V, &h);
+    if (!herr.empty()) return fail(TGX_ERR_UNSUPPORTED, herr);
   }
   if (hash_ok) CU(m->d_hash.reserve(h.slots.size() * sizeof(tgx::Slot)));
   m->hash.mask = 0;
