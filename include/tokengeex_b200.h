@@ -247,7 +247,6 @@ double tgx_model_last_stat(const tgx_model* m, int what);
  *        full warp (also: warp-cooperative backtrack);
  *    6 / 13 / 14 = pair-CTA kernel: groups per CTA (0 = as many as fit), trie
  *        levels staged in shared memory (0..2), shape (0 = by batch size, 1 = 5 groups, 2 = 6 groups);
- *   11 = chunked host entry point queues the next chunk's kernels before the current chunk has finished (default 0);
  *   16 = emit looks token ids up in the token hash (1, default when max_token_len <= 16) or re-walks the trie (0);
  *    2 / 5 / 17 / 18 / 19 / 20 / 21 / 30 / 31 = E-step: lanes per snippet of the lane-group kernels; byte threshold from
  *        which a snippet gets a full warp (0 = automatic); byte threshold below which a snippet runs on ONE lane (< 0 =

@@ -289,12 +289,11 @@ def test_chunked_host_entry_point(N):
     blob, off, toks, sc, kp = synth_setup(2, 31, 1_200_000, 6000, 16)
     gm, om = both(N, toks, sc)
     wids, wid_off, wstatus, wplen, wbad = om.encode_batch(blob, off, crlf=True, threads=8)
-    for chunk, overlap in ((4096, 1), (100_000, 1), (100_000, 0), (300_000, 1), (1 << 30, 1)):
+    for chunk in (4096, 100_000, 300_000, 1 << 30):
         gm.set_option(7, chunk)
-        gm.set_option(11, overlap)  # queue chunk k+1's kernels before chunk k has finished (two workspaces)
         for rep in range(2):
             ids, id_off, status, plen, rc, bad = gm.encode_batch(blob, off, crlf=True)
-            assert rc == 0 and np.array_equal(ids, wids) and np.array_equal(id_off, wid_off), (chunk, overlap, rep)
+            assert rc == 0 and np.array_equal(ids, wids) and np.array_equal(id_off, wid_off), (chunk, rep)
         assert np.array_equal(plen, wplen) and not status.any()
     # a vocabulary without some bytes: NoPath samples in several chunks; the LOWEST index is reported
     toks2 = [t for t in toks if t not in (b"e", b"{")]

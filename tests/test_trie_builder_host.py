@@ -79,6 +79,9 @@ def test_rebuild_keeps_the_layout_for_a_subset_and_builds_afresh_otherwise():
     for q in (b"zzzzab", toks[0] + b"a", toks[5]):
         assert hm.common_prefix_search(q) == om.common_prefix_search(q)
     hm.set_option(45, 0)
+    with pytest.raises(N.TgxError) as ei:  # 11 is not an option key: refused like any unknown key
+        hm.set_option(11, 0)
+    assert ei.value.code == N.TGX_ERR_INVALID
     hm.rebuild(t3[:-3], s3[:-3])
     om = O.OracleModel(t3[:-3], s3[:-3])
     for q in (toks[0] + b"a", toks[7], b"zzzz"):

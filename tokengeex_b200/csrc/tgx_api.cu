@@ -40,10 +40,16 @@ int fail(int code, const std::string& msg) {
       return fail(TGX_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(_e));               \
   } while (0)
 
-// Growable device buffer (never shrinks; reused across calls).
+// Growable device buffer (never shrinks; reused across calls; freed with its owner).
 struct DevBuf {
   void* p = nullptr;
   size_t cap = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() {
+    if (p) cudaFree(p);
+  }
   cudaError_t reserve(size_t bytes) {
     if (bytes <= cap) return cudaSuccess;
     if (p) cudaFree(p);
@@ -56,11 +62,6 @@ struct DevBuf {
   }
   template <class T>
   T* as() const { return reinterpret_cast<T*>(p); }
-  void release() {
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
-  }
 };
 
 struct Stats {
@@ -70,9 +71,8 @@ struct Stats {
 
 }  // namespace
 
-// Scratch of one batch in flight: its compute stream, the stream its control words are read through, events and
-// every intermediate buffer.  The model owns two, so that the chunked host entry point can have the kernels of
-// chunk k+1 queued behind chunk k (the tail of a chunk is a handful of long samples on a few SMs).
+// Scratch of the batch in flight: its compute stream, the stream its control words are read through, events and
+// every intermediate buffer.
 struct Workspace {
   cudaStream_t stream = nullptr;
   // The compute stream never issues a D2H copy itself: measured on B200 (profiles/r01_ubench_overlap.txt),
@@ -108,16 +108,13 @@ struct tgx_model {
   DevBuf d_trie8, d_rows, d_rowids, d_pair2;
   bool have_rows = false;
   uint32_t rows16 = 0;  // 16-byte units in the row table
-  Workspace ws[2];
-  int wi = 0;  // workspace the next launches go to
-  Workspace& w() { return ws[wi]; }
-  const Workspace& w() const { return ws[wi]; }
+  Workspace ws;
   Stats last_stats;  // of the last finished call (tgx_model_last_stat)
   cudaStream_t stream2 = nullptr;  // long units run beside the short ones (E-step)
   cudaStream_t stream3 = nullptr;  // lane-per-snippet kernels (E-step)
   cudaStream_t stream4 = nullptr;  // beta chains of the warp-per-snippet kernels in split form
   cudaStream_t stream5 = nullptr, stream6 = nullptr;  // second / third group of lane snippets (E-step)
-  cudaEvent_t ev_grp[4] = {}, ev_join5 = nullptr, ev_join6 = nullptr;
+  cudaEvent_t ev_join5 = nullptr, ev_join6 = nullptr;
   int estep_cut1 = 150, estep_cut2 = 1000;  // per mille of the lane snippets (longest first) where the groups end
   cudaEvent_t ev_join3 = nullptr, ev_join4 = nullptr;
   cudaStream_t stream_h2d = nullptr, stream_d2h = nullptr;  // copy engines of the chunked host entry points
@@ -174,13 +171,7 @@ struct tgx_model {
   int64_t rows_hot_bytes = 96 << 10;  // leading bytes of the row table viterbi_rows_kernel stages in shared memory
   int num_sms = 148;
   int groups = 0;       // consumer/producer groups per CTA of the pair kernel; 0 = as many as fit
-  uint32_t pair_grid_cap = 0;  // CTAs the next pair-kernel launch may use (0 = one per SM); set and cleared by algo 3
   int smem_optin = 232448;
-  // Chunked host entry point: queue chunk k+1's kernels (second workspace) before chunk k has finished.  Off by
-  // default: measured on B200 (tools/e2e_trace.py, 1 GB) it LOSES, 75.4 vs 67.6 ms with two chunks — the next
-  // chunk's persistent forward CTAs take every SM the moment the current forward kernel drains, and the current
-  // chunk's backtrack / emit kernels then wait for registers until those CTAs exit.
-  int overlap_chunks = 0;
   int hot_levels = 2;  // leading trie levels the pair kernel may stage in shared memory (0..2)
   int emit_hash = 1;   // emit: token ids through the token hash (1 probe per token) instead of re-walking the trie
   int pair_shape = 0;  // 0 = by batch size, 1 = latency shape (5 groups), 2 = throughput shape (6 groups)
@@ -188,7 +179,6 @@ struct tgx_model {
   // 0.0 = off (every BASELINE configuration); in (0, 1) the keyed draw of tgx_kernels.cuh::drop_draw.
   double dropout = 0.0;
   uint64_t drop_seed = 0;
-  uint64_t drop_unit_base = 0;  // first sample of the chunk being queued (chunked host entry point)
   uint64_t drop_byte_base = 0;  // E-step: offset of this call's text in the whole (sharded) corpus, option 22
   uint64_t wide_bytes = 600ull << 20;
   // buffers of the host entry points (two sets for the chunk pipeline) and of the E-step / frequency pass
@@ -676,10 +666,6 @@ namespace {
 
 using namespace tgxk;
 
-struct Timer {
-  cudaEvent_t a, b;
-};
-
 cudaError_t dev_fill(void* p, int byte, size_t n, cudaStream_t st) {
   if (!n) return cudaSuccess;
   const uint32_t blocks = (uint32_t)std::min<uint64_t>(std::max<uint64_t>(1, (n + 4095) / 4096), 148 * 8);
@@ -695,13 +681,16 @@ cudaError_t launch_viterbi(tgx_model* m, ViterbiParams p) {
   if (e != cudaSuccess) return e;
   uint32_t per_block = WPB * (32 / G);
   uint32_t blocks = (p.u.count + per_block - 1) / per_block;
-  viterbi_kernel<G, DROP><<<blocks, WPB * 32, smem, m->w().stream>>>(p);
-  m->w().stats.launches += 1;
+  viterbi_kernel<G, DROP><<<blocks, WPB * 32, smem, m->ws.stream>>>(p);
+  m->ws.stats.launches += 1;
   return cudaGetLastError();
 }
 
+// The pair-CTA kernel on `st`: at most `grid_cap` CTAs (0 = one per SM) of at most `group_cap` groups each (0 = as
+// many as fit).  The caller has cleared p.counter.
 template <int R, int HOT, int MAXT, bool DROP = false>
-cudaError_t launch_viterbi_pair(tgx_model* m, PairParams p, DropInfo di = DropInfo()) {
+cudaError_t launch_viterbi_pair(tgx_model* m, PairParams p, DropInfo di, cudaStream_t st, uint32_t grid_cap,
+                                int group_cap) {
   auto kernel = [] {
     if constexpr (DROP) return viterbi_pair_drop_kernel<R, HOT, MAXT>;
     else return viterbi_pair_kernel<R, HOT, MAXT>;
@@ -710,7 +699,7 @@ cudaError_t launch_viterbi_pair(tgx_model* m, PairParams p, DropInfo di = DropIn
   const size_t budget = (size_t)m->smem_optin;
   uint32_t groups = (uint32_t)std::min<size_t>({(budget - (size_t)p.hot_slots * 16) / pair_group_bytes(R),
                                                 (size_t)(MAXT / (32 * WG)), (size_t)15});
-  if (m->groups > 0) groups = std::min<uint32_t>(groups, (uint32_t)m->groups);
+  if (group_cap > 0) groups = std::min<uint32_t>(groups, (uint32_t)group_cap);
   groups = std::max<uint32_t>(1, std::min<uint32_t>(groups, (p.u.count + 1) / 2));
   p.groups = groups;
   const size_t smem = pair_smem_bytes(R, groups, p.hot_slots);
@@ -720,17 +709,11 @@ cudaError_t launch_viterbi_pair(tgx_model* m, PairParams p, DropInfo di = DropIn
   e = cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
                            (int)std::min<size_t>(100, (smem + 1024) * 100 / (228 * 1024) + 1));
   if (e != cudaSuccess) return e;
-  const uint32_t grid =
-      (uint32_t)std::min<uint64_t>(((uint64_t)p.u.count + 2 * groups - 1) / (2 * groups),
-                                   (uint64_t)(m->pair_grid_cap ? m->pair_grid_cap : (uint32_t)m->num_sms));
-  if (!m->pair_grid_cap) {  // (algo 3 clears the counter before it forks: nothing may sit in front of this kernel on
-                            //  its stream, or the spare team CTAs take the SMs that were left free for it)
-    e = dev_fill(p.counter, 0, 4, m->w().stream);
-    if (e != cudaSuccess) return e;
-  }
-  if constexpr (DROP) kernel<<<grid, groups * WG * 32, smem, m->w().stream>>>(p, di);
-  else kernel<<<grid, groups * WG * 32, smem, m->w().stream>>>(p);
-  m->w().stats.launches += 1;
+  const uint32_t grid = (uint32_t)std::min<uint64_t>(((uint64_t)p.u.count + 2 * groups - 1) / (2 * groups),
+                                                     (uint64_t)(grid_cap ? grid_cap : (uint32_t)m->num_sms));
+  if constexpr (DROP) kernel<<<grid, groups * WG * 32, smem, st>>>(p, di);
+  else kernel<<<grid, groups * WG * 32, smem, st>>>(p);
+  m->ws.stats.launches += 1;
   return cudaGetLastError();
 }
 
@@ -740,28 +723,32 @@ cudaError_t launch_viterbi_pair(tgx_model* m, PairParams p, DropInfo di = DropIn
 // A batch is bound by its longest sample unless it is large, so the throughput shape is used from
 // `wide_bytes` input bytes on (the chunks of the host entry point stay below it).
 template <int R>
-cudaError_t launch_viterbi_pair_r(tgx_model* m, PairParams p, uint64_t n_bytes, DropInfo di = DropInfo()) {
+cudaError_t launch_viterbi_pair_r(tgx_model* m, PairParams p, uint64_t n_bytes, DropInfo di, cudaStream_t st,
+                                  uint32_t grid_cap, int group_cap) {
   const size_t cap = (size_t)m->smem_optin / 4;
   if (di.dropout > 0.0) {  // one shape with the keyed draw in the producers: 5 groups, 72 registers
     if ((size_t)m->da.hot[1] * 16 <= cap) {
       p.hot_slots = m->da.hot[1];
-      return launch_viterbi_pair<2, 1, 800, true>(m, p, di);
+      return launch_viterbi_pair<2, 1, 800, true>(m, p, di, st, grid_cap, group_cap);
     }
     p.hot_slots = 0;
-    return launch_viterbi_pair<2, 0, 800, true>(m, p, di);
+    return launch_viterbi_pair<2, 0, 800, true>(m, p, di, st, grid_cap, group_cap);
   }
   const bool wide = m->pair_shape == 2 || (m->pair_shape == 0 && n_bytes >= m->wide_bytes);
   const int levels = std::min(m->hot_levels, wide ? 1 : 2);
   if (levels >= 2 && (size_t)m->da.hot[2] * 16 <= cap) {
     p.hot_slots = m->da.hot[2];
-    return wide ? launch_viterbi_pair<R, 2, 960>(m, p) : launch_viterbi_pair<R, 2, 800>(m, p);
+    return wide ? launch_viterbi_pair<R, 2, 960>(m, p, di, st, grid_cap, group_cap)
+                : launch_viterbi_pair<R, 2, 800>(m, p, di, st, grid_cap, group_cap);
   }
   if (levels >= 1 && (size_t)m->da.hot[1] * 16 <= cap) {
     p.hot_slots = m->da.hot[1];
-    return wide ? launch_viterbi_pair<R, 1, 960>(m, p) : launch_viterbi_pair<R, 1, 800>(m, p);
+    return wide ? launch_viterbi_pair<R, 1, 960>(m, p, di, st, grid_cap, group_cap)
+                : launch_viterbi_pair<R, 1, 800>(m, p, di, st, grid_cap, group_cap);
   }
   p.hot_slots = 0;
-  return wide ? launch_viterbi_pair<R, 0, 960>(m, p) : launch_viterbi_pair<R, 0, 800>(m, p);
+  return wide ? launch_viterbi_pair<R, 0, 960>(m, p, di, st, grid_cap, group_cap)
+              : launch_viterbi_pair<R, 0, 800>(m, p, di, st, grid_cap, group_cap);
 }
 
 cudaError_t launch_viterbi_g(tgx_model* m, int G, const ViterbiParams& p) {
@@ -792,7 +779,7 @@ cudaError_t launch_fb(tgx_model* m, FbParams p, bool backward, cudaStream_t st) 
     if (e != cudaSuccess) return e;
     fb_backward_kernel<G, false, DROP><<<blocks, WPB * 32, smem, st>>>(p);
   }
-  m->w().stats.launches += 1;
+  m->ws.stats.launches += 1;
   return cudaGetLastError();
 }
 
@@ -826,7 +813,7 @@ int check_model(tgx_model* m) {
 // callers on other streams synchronise them first.  Results are complete when the call returns.
 int order_after_caller(tgx_model* m) {
   CU(cudaEventRecord(m->ev_caller, cudaStreamLegacy));
-  CU(cudaStreamWaitEvent(m->w().stream, m->ev_caller, 0));
+  CU(cudaStreamWaitEvent(m->ws.stream, m->ev_caller, 0));
   return TGX_OK;
 }
 
@@ -834,12 +821,10 @@ int order_after_caller(tgx_model* m) {
 // hash.mask == 0 and emit walks the trie.  On failure nothing the model already holds has been touched.
 // `built`: a token hash of this vocabulary that the caller has built already (beside the trie, on a thread of its own),
 // with the builder's message in `built_err`; null = build it here.
-int upload_aux_tables(tgx_model* m, const tgx::DoubleArray& da, const uint8_t* token_bytes, const uint64_t* token_offsets,
-                      uint64_t V, uint32_t max_token_len, tgx::TokenHash* built = nullptr,
-                      const std::string* built_err = nullptr) {
-  (void)da;
+int upload_aux_tables(tgx_model* m, const uint8_t* token_bytes, const uint64_t* token_offsets, uint64_t V,
+                      uint32_t max_token_len, tgx::TokenHash* built = nullptr, const std::string* built_err = nullptr) {
   if (m->device < 0) return TGX_OK;
-  cudaStream_t st = m->w().stream;
+  cudaStream_t st = m->ws.stream;
   tgx::TokenHash h;
   bool hash_ok = V != 0 && max_token_len >= 1 && max_token_len <= 16;
   if (hash_ok && built) {
@@ -870,7 +855,7 @@ int ensure_match_tables(tgx_model* m) {
   if (m->have_rows || m->device < 0) return TGX_OK;
   if (!tgx::build_match_tables(&m->da).empty()) return TGX_OK;
   const tgx::DoubleArray& da = m->da;
-  cudaStream_t st = m->w().stream;
+  cudaStream_t st = m->ws.stream;
   CU(m->d_trie8.reserve(da.slots8.size() * 8));
   CU(m->d_rows.reserve(da.rows.size() * 8 + 256));
   CU(m->d_rowids.reserve(da.row_ids.size() * 4 + 256));
@@ -885,71 +870,71 @@ int ensure_match_tables(tgx_model* m) {
   return TGX_OK;
 }
 
-// crlf on device: (d_text,d_off) -> (m->w().text2, m->w().off2).  N = total bytes.
+// crlf on device: (d_text,d_off) -> (m->ws.text2, m->ws.off2).  N = total bytes.
 int run_crlf(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint64_t S, uint64_t N) {
-  cudaStream_t st = m->w().stream;
+  cudaStream_t st = m->ws.stream;
   uint64_t n_tiles = (N + CRLF_TILE - 1) / CRLF_TILE;
-  CU(m->w().text2.reserve(N + 16));
-  CU(m->w().off2.reserve((S + 1) * 8));
-  CU(m->w().bitmap.reserve((N / 32 + 4) * 4));
-  CU(m->w().blk.reserve((n_tiles + 1) * 8 * 2));
-  CU(dev_fill(m->w().bitmap.p, 0, (N / 32 + 4) * 4, st));
+  CU(m->ws.text2.reserve(N + 16));
+  CU(m->ws.off2.reserve((S + 1) * 8));
+  CU(m->ws.bitmap.reserve((N / 32 + 4) * 4));
+  CU(m->ws.blk.reserve((n_tiles + 1) * 8 * 2));
+  CU(dev_fill(m->ws.bitmap.p, 0, (N / 32 + 4) * 4, st));
   if (S > 1) {
-    crlf_mark_starts<<<nblk(S, 256), 256, 0, st>>>(d_off, S, m->w().bitmap.as<uint32_t>());
-    m->w().stats.launches += 1;
+    crlf_mark_starts<<<nblk(S, 256), 256, 0, st>>>(d_off, S, m->ws.bitmap.as<uint32_t>());
+    m->ws.stats.launches += 1;
   }
-  unsigned long long* removed = m->w().blk.as<unsigned long long>();
+  unsigned long long* removed = m->ws.blk.as<unsigned long long>();
   unsigned long long* prefix = removed + n_tiles + 1;
   CU(dev_fill(removed, 0, (n_tiles + 1) * 8, st));
   if (n_tiles) {
-    crlf_count<<<(uint32_t)n_tiles, CRLF_BLOCK, 0, st>>>(d_text, N, m->w().bitmap.as<uint32_t>(), removed);
-    m->w().stats.launches += 1;
+    crlf_count<<<(uint32_t)n_tiles, CRLF_BLOCK, 0, st>>>(d_text, N, m->ws.bitmap.as<uint32_t>(), removed);
+    m->ws.stats.launches += 1;
   }
   size_t tmp = 0;
   CU(cub::DeviceScan::ExclusiveSum(nullptr, tmp, removed, prefix, (int)(n_tiles + 1), st));
-  CU(m->w().cubtmp.reserve(tmp));
-  CU(cub::DeviceScan::ExclusiveSum(m->w().cubtmp.p, tmp, removed, prefix, (int)(n_tiles + 1), st));
-  m->w().stats.launches += 2;
+  CU(m->ws.cubtmp.reserve(tmp));
+  CU(cub::DeviceScan::ExclusiveSum(m->ws.cubtmp.p, tmp, removed, prefix, (int)(n_tiles + 1), st));
+  m->ws.stats.launches += 2;
   if (n_tiles) {
-    crlf_scatter<<<(uint32_t)n_tiles, CRLF_BLOCK, 0, st>>>(d_text, N, d_off, S, m->w().bitmap.as<uint32_t>(), prefix,
-                                                          n_tiles, m->w().text2.as<uint8_t>(), m->w().off2.as<uint64_t>());
-    m->w().stats.launches += 1;
+    crlf_scatter<<<(uint32_t)n_tiles, CRLF_BLOCK, 0, st>>>(d_text, N, d_off, S, m->ws.bitmap.as<uint32_t>(), prefix,
+                                                          n_tiles, m->ws.text2.as<uint8_t>(), m->ws.off2.as<uint64_t>());
+    m->ws.stats.launches += 1;
   } else {
-    CU(dev_fill(m->w().off2.p, 0, (S + 1) * 8, st));  // no bytes at all: every sample is empty
+    CU(dev_fill(m->ws.off2.p, 0, (S + 1) * 8, st));  // no bytes at all: every sample is empty
   }
   CU(cudaGetLastError());
   return TGX_OK;
 }
 
-// sort unit indices by length, descending: keys in m->w().ulen, values in m->w().vals_in -> m->w().vals_out
+// sort unit indices by length, descending: keys in m->ws.ulen, values in m->ws.vals_in -> m->ws.vals_out
 int sort_units(tgx_model* m, uint32_t U) {
-  CU(m->w().keys_out.reserve((size_t)U * 4 + 4));
-  CU(m->w().vals_out.reserve((size_t)U * 4 + 4));
+  CU(m->ws.keys_out.reserve((size_t)U * 4 + 4));
+  CU(m->ws.vals_out.reserve((size_t)U * 4 + 4));
   size_t tmp = 0;
-  CU(cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp, m->w().ulen.as<uint32_t>(), m->w().keys_out.as<uint32_t>(),
-                                               m->w().vals_in.as<uint32_t>(), m->w().vals_out.as<uint32_t>(), (int)U, 0, 32,
-                                               m->w().stream));
-  CU(m->w().cubtmp.reserve(tmp));
-  CU(cub::DeviceRadixSort::SortPairsDescending(m->w().cubtmp.p, tmp, m->w().ulen.as<uint32_t>(), m->w().keys_out.as<uint32_t>(),
-                                               m->w().vals_in.as<uint32_t>(), m->w().vals_out.as<uint32_t>(), (int)U, 0, 32,
-                                               m->w().stream));
-  m->w().stats.launches += 4;
+  CU(cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp, m->ws.ulen.as<uint32_t>(), m->ws.keys_out.as<uint32_t>(),
+                                               m->ws.vals_in.as<uint32_t>(), m->ws.vals_out.as<uint32_t>(), (int)U, 0, 32,
+                                               m->ws.stream));
+  CU(m->ws.cubtmp.reserve(tmp));
+  CU(cub::DeviceRadixSort::SortPairsDescending(m->ws.cubtmp.p, tmp, m->ws.ulen.as<uint32_t>(), m->ws.keys_out.as<uint32_t>(),
+                                               m->ws.vals_in.as<uint32_t>(), m->ws.vals_out.as<uint32_t>(), (int)U, 0, 32,
+                                               m->ws.stream));
+  m->ws.stats.launches += 4;
   return TGX_OK;
 }
 
 int read_words(tgx_model* m, const void* d0, const void* d1, unsigned long long* o0, unsigned long long* o1);
 
-// match_kernel over the whole blob: m->w().rec[p] = record of start position p (tgx_match_kernels.cuh)
+// match_kernel over the whole blob: m->ws.rec[p] = record of start position p (tgx_match_kernels.cuh)
 int run_match(tgx_model* m, const uint8_t* d_text, uint64_t N, const uint8_t* d_skip = nullptr) {
-  cudaStream_t st = m->w().stream;
-  CU(m->w().rec.reserve((N + 64) * 4));
+  cudaStream_t st = m->ws.stream;
+  CU(m->ws.rec.reserve((N + 64) * 4));
   MatchParams mp;
   mp.text = d_text;
   mp.blob_end = d_text + N;
   mp.N = N;
   mp.trie8 = m->d_trie8.as<uint2>();
   mp.root_base = m->da.root_base;
-  mp.rec = m->w().rec.as<uint32_t>();
+  mp.rec = m->ws.rec.as<uint32_t>();
   mp.skip = d_skip;
   mp.pair2 = m->d_pair2.as<uint2>();
   mp.slice = 0;
@@ -981,51 +966,51 @@ int run_match(tgx_model* m, const uint8_t* d_text, uint64_t N, const uint8_t* d_
     mp.slice = rounds * per_cta;
     match2_kernel<<<(uint32_t)((N + mp.slice - 1) / mp.slice), threads, smem2, st>>>(mp);
     CU(cudaGetLastError());
-    m->w().stats.launches += 1;
+    m->ws.stats.launches += 1;
     return TGX_OK;
   }
   CU(launch(match_kernel<4>, 4));
-  m->w().stats.launches += 1;
+  m->ws.stats.launches += 1;
   return TGX_OK;
 }
 
 // Viterbi over all samples: forward dp (back lengths) + backtrack (token-end marks).  On return
-// m->w().mark holds the length of the token ending at every marked byte, m->w().ntok token counts,
-// m->w().status per-sample status.
+// m->ws.mark holds the length of the token ending at every marked byte, m->ws.ntok token counts,
+// m->ws.status per-sample status.  `unit_base`: index of sample 0 in the whole input (it keys the dropout draw).
 int run_viterbi(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint64_t S, uint64_t N,
-                uint64_t* d_proc_len, bool with_dropout = false) {
-  cudaStream_t st = m->w().stream;
+                uint64_t* d_proc_len, bool with_dropout = false, uint64_t unit_base = 0) {
+  cudaStream_t st = m->ws.stream;
   if (S >= (1ull << 32)) return fail(TGX_ERR_INVALID, "too many samples in one call (< 2^32)");
   uint32_t U = (uint32_t)S;
   const uint64_t n_tiles = (N + EM_TILE - 1) / EM_TILE;
-  CU(m->w().ustart.reserve((size_t)U * 8 + 8));
-  CU(m->w().ulen.reserve((size_t)U * 4 + 4));
-  CU(m->w().vals_in.reserve((size_t)U * 4 + 4));
-  CU(m->w().bp.reserve(N + 64));
-  CU(m->w().mark.reserve(n_tiles * EM_TILE + 64));
-  CU(m->w().ntok.reserve(((size_t)U + 1) * 8));
-  CU(m->w().status.reserve((size_t)U * 4 + 4));
-  CU(m->w().small.reserve(256));
-  units_from_samples<<<nblk(U, 256), 256, 0, st>>>(d_off, S, m->w().ustart.as<uint64_t>(), m->w().ulen.as<uint32_t>(),
-                                                  m->w().vals_in.as<uint32_t>(), d_proc_len);
-  m->w().stats.launches += 1;
+  CU(m->ws.ustart.reserve((size_t)U * 8 + 8));
+  CU(m->ws.ulen.reserve((size_t)U * 4 + 4));
+  CU(m->ws.vals_in.reserve((size_t)U * 4 + 4));
+  CU(m->ws.bp.reserve(N + 64));
+  CU(m->ws.mark.reserve(n_tiles * EM_TILE + 64));
+  CU(m->ws.ntok.reserve(((size_t)U + 1) * 8));
+  CU(m->ws.status.reserve((size_t)U * 4 + 4));
+  CU(m->ws.small.reserve(256));
+  units_from_samples<<<nblk(U, 256), 256, 0, st>>>(d_off, S, m->ws.ustart.as<uint64_t>(), m->ws.ulen.as<uint32_t>(),
+                                                  m->ws.vals_in.as<uint32_t>(), d_proc_len);
+  m->ws.stats.launches += 1;
   int rc = sort_units(m, U);
   if (rc) return rc;
-  uint32_t* counts = m->w().small.as<uint32_t>();
+  uint32_t* counts = m->ws.small.as<uint32_t>();
   uint32_t thr = (uint32_t)std::min<int64_t>(m->long_threshold, 0x7FFFFFFF);
   const uint32_t thr2 = (uint32_t)std::min<int64_t>(m->team_long_threshold, 0x7FFFFFFF);
-  split_sorted<<<1, 32, 0, st>>>(m->w().keys_out.as<uint32_t>(), U, thr, thr2, counts);
-  m->w().stats.launches += 1;
-  CU(dev_fill(m->w().ntok.p, 0, ((size_t)U + 1) * 8, st));
-  CU(dev_fill(m->w().status.p, 0, (size_t)U * 4 + 4, st));
-  CU(dev_fill(m->w().mark.p, 0, n_tiles * EM_TILE, st));
+  split_sorted<<<1, 32, 0, st>>>(m->ws.keys_out.as<uint32_t>(), U, thr, thr2, counts);
+  m->ws.stats.launches += 1;
+  CU(dev_fill(m->ws.ntok.p, 0, ((size_t)U + 1) * 8, st));
+  CU(dev_fill(m->ws.status.p, 0, (size_t)U * 4 + 4, st));
+  CU(dev_fill(m->ws.mark.p, 0, n_tiles * EM_TILE, st));
   // (no host synchronisation here: every kernel below reads its unit range from `counts`)
 
   UnitParams u;
   u.text = d_text;
-  u.unit_start = m->w().ustart.as<uint64_t>();
-  u.unit_len = m->w().ulen.as<uint32_t>();
-  u.order = m->w().vals_out.as<uint32_t>();
+  u.unit_start = m->ws.ustart.as<uint64_t>();
+  u.unit_len = m->ws.ulen.as<uint32_t>();
+  u.order = m->ws.vals_out.as<uint32_t>();
   u.trie = m->d_trie;
   u.root_base = m->da.root_base;
   u.rows = std::max<uint32_t>(1, m->da.max_token_len);
@@ -1045,8 +1030,8 @@ int run_viterbi(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint
     if (rc) return rc;
   }
   const int algo = dropout > 0.0 ? (algo_req == 1 ? 1 : 2) : ((algo_req == 0 || algo_req == 3) && !m->have_rows ? 2 : algo_req);
-  m->w().algo_used = algo;
-  m->w().side_used = false;
+  m->ws.algo_used = algo;
+  m->ws.side_used = false;
   uint32_t n_long = 0;  // algo 3: samples of at least team_long_threshold bytes (the one host wait in the middle of a call)
   if (algo == 3 && u.rows <= 16 && N && U) {
     unsigned long long w01 = 0, w23 = 0;
@@ -1054,24 +1039,24 @@ int run_viterbi(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint
     if (rc) return rc;
     n_long = std::min<uint32_t>((uint32_t)w23, (uint32_t)(w01 >> 32));  // min(counts[2], counts[1])
   }
-  CU(cudaEventRecord(m->w().ev[8], st));
+  CU(cudaEventRecord(m->ws.ev[8], st));
   if ((algo == 0 || algo == 3) && u.rows <= 16 && N) {
     const uint8_t* d_skip = nullptr;
     if (algo == 3 && n_long && m->match_compact && m->match_skip) {
       // nobody reads the records inside the samples the pair-CTA kernel takes: match2_kernel writes row 0 there
       const size_t nb = (size_t)((N + 127) >> 7);
-      CU(m->w().skip.reserve(nb + 64));
-      CU(dev_fill(m->w().skip.p, 0, nb, st));
+      CU(m->ws.skip.reserve(nb + 64));
+      CU(dev_fill(m->ws.skip.p, 0, nb, st));
       mark_skip_kernel<<<nblk((uint64_t)n_long * 32, 256), 256, 0, st>>>(u.unit_start, u.unit_len, u.order, n_long,
-                                                                        m->w().skip.as<uint8_t>());
-      m->w().stats.launches += 1;
-      d_skip = m->w().skip.as<uint8_t>();
+                                                                        m->ws.skip.as<uint8_t>());
+      m->ws.stats.launches += 1;
+      d_skip = m->ws.skip.as<uint8_t>();
     }
     rc = run_match(m, d_text, N, d_skip);
     if (rc) return rc;
   }
-  CU(cudaEventRecord(m->w().ev[9], st));
-  CU(cudaEventRecord(m->w().ev[0], st));  // [0]..[1]: the consumer of the match stream / the forward kernel
+  CU(cudaEventRecord(m->ws.ev[9], st));
+  CU(cudaEventRecord(m->ws.ev[0], st));  // [0]..[1]: the consumer of the match stream / the forward kernel
   if (algo == 3 && u.rows <= 16) {
     if (N && U) {
       // The samples of at least team_long_threshold bytes run on the pair-CTA kernel (16 lanes per sample: the shortest
@@ -1085,45 +1070,38 @@ int run_viterbi(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint
       // 262144 bytes), and the shorter long ones fit behind each other inside that time on fewer SMs.
       const uint32_t per_cta = (uint32_t)std::max(1, m->side_load);
       const uint32_t P = n_long ? std::min<uint32_t>((n_long + per_cta - 1) / per_cta, (uint32_t)m->num_sms * 2u / 3u) : 0u;
-      unsigned int* ctr = m->w().small.as<unsigned int>() + 8;
+      unsigned int* ctr = m->ws.small.as<unsigned int>() + 8;
+      // both work counters are cleared before the fork: nothing may sit in front of the pair kernel on its stream, or
+      // the spare team CTAs take the SMs that were left free for it
       CU(dev_fill(ctr, 0, 8, st));
-      CU(cudaEventRecord(m->w().ev_side_fork, st));
+      CU(cudaEventRecord(m->ws.ev_side_fork, st));
       if (P) {
-        CU(cudaStreamWaitEvent(m->w().stream_side, m->w().ev_side_fork, 0));
+        CU(cudaStreamWaitEvent(m->ws.stream_side, m->ws.ev_side_fork, 0));
         PairParams pp;
         pp.u = u;
         pp.u.part = 3;
         pp.u.count = n_long;
         pp.blob_end = d_text + N;
-        pp.bp = m->w().bp.as<uint8_t>();
+        pp.bp = m->ws.bp.as<uint8_t>();
         pp.counter = ctr;
         pp.dbg = 0;
-        m->w().side_used = true;
-        CU(cudaEventRecord(m->w().ev[10], m->w().stream_side));
-        {
-          cudaStream_t keep = m->w().stream;
-          m->w().stream = m->w().stream_side;
-          m->pair_grid_cap = P;
-          const int keep_groups = m->groups;
-          if (m->side_groups > 0) m->groups = m->groups > 0 ? std::min(m->groups, m->side_groups) : m->side_groups;
-          cudaError_t e = launch_viterbi_pair_r<2>(m, pp, 0);
-          m->groups = keep_groups;
-          m->pair_grid_cap = 0;
-          m->w().stream = keep;
-          CU(e);
-        }
-        CU(cudaEventRecord(m->w().ev[11], m->w().stream_side));
-        CU(cudaEventRecord(m->w().ev_side_join, m->w().stream_side));
-        CU(cudaStreamWaitEvent(m->w().stream_low, m->w().ev_side_fork, 0));
+        m->ws.side_used = true;
+        CU(cudaEventRecord(m->ws.ev[10], m->ws.stream_side));
+        int side_groups = m->groups;
+        if (m->side_groups > 0) side_groups = m->groups > 0 ? std::min(m->groups, m->side_groups) : m->side_groups;
+        CU(launch_viterbi_pair_r<2>(m, pp, 0, DropInfo(), m->ws.stream_side, P, side_groups));
+        CU(cudaEventRecord(m->ws.ev[11], m->ws.stream_side));
+        CU(cudaEventRecord(m->ws.ev_side_join, m->ws.stream_side));
+        CU(cudaStreamWaitEvent(m->ws.stream_low, m->ws.ev_side_fork, 0));
       }
       TeamParams tm;
       tm.u = u;
       tm.u.part = 4;
       tm.u.count = U - std::min(U, n_long);
-      tm.rec = m->w().rec.as<uint32_t>();
+      tm.rec = m->ws.rec.as<uint32_t>();
       tm.rows = m->d_rows.as<double>();
-      tm.bp = m->w().bp.as<uint8_t>();
-      tm.counter = m->w().small.as<unsigned int>() + 9;
+      tm.bp = m->ws.bp.as<uint8_t>();
+      tm.counter = m->ws.small.as<unsigned int>() + 9;
       const size_t budget = (size_t)std::min<int64_t>(m->team_hot_bytes, (int64_t)m->smem_optin - 1024);
       tm.hot16 = (uint32_t)std::max<size_t>(std::min<size_t>(m->rows16, budget / 16), std::min<size_t>(m->rows16, 9));  // (row 0 is always staged)
       const size_t smem = (size_t)tm.hot16 * 16;
@@ -1134,16 +1112,16 @@ int run_viterbi(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint
         const uint32_t ctas = ((n_short + per_warp - 1) / per_warp + warps - 1) / warps;
         const uint32_t g1 = std::max<uint32_t>(1, std::min<uint32_t>(ctas, (uint32_t)m->num_sms - P));
         viterbi_team_kernel<warps><<<g1, warps * 32, smem, st>>>(tm);
-        m->w().stats.launches += 1;
+        m->ws.stats.launches += 1;
         if (P && ctas > g1) {
-          viterbi_team_kernel<warps><<<std::min<uint32_t>(ctas - g1, P), warps * 32, smem, m->w().stream_low>>>(tm);
-          m->w().stats.launches += 1;
+          viterbi_team_kernel<warps><<<std::min<uint32_t>(ctas - g1, P), warps * 32, smem, m->ws.stream_low>>>(tm);
+          m->ws.stats.launches += 1;
         }
         CU(cudaGetLastError());
       }
       if (P) {
-        CU(cudaEventRecord(m->w().ev_low_join, m->w().stream_low));
-        CU(cudaStreamWaitEvent(st, m->w().ev_low_join, 0));
+        CU(cudaEventRecord(m->ws.ev_low_join, m->ws.stream_low));
+        CU(cudaStreamWaitEvent(st, m->ws.ev_low_join, 0));
       }
     }
   } else if (algo == 0 && u.rows <= 16) {
@@ -1151,19 +1129,19 @@ int run_viterbi(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint
       RowsParams rp;
       rp.u = u;
       rp.u.part = 0;
-      rp.rec = m->w().rec.as<uint32_t>();
+      rp.rec = m->ws.rec.as<uint32_t>();
       rp.rows = m->d_rows.as<double>();
       const size_t budget = (size_t)std::min<int64_t>(m->rows_hot_bytes, (int64_t)m->smem_optin - 1024);
       rp.hot16 = (uint32_t)std::min<size_t>(m->rows16, budget / 16);
-      rp.bp = m->w().bp.as<uint8_t>();
-      rp.counter = m->w().small.as<unsigned int>() + 8;
+      rp.bp = m->ws.bp.as<uint8_t>();
+      rp.counter = m->ws.small.as<unsigned int>() + 8;
       const size_t smem = (size_t)rp.hot16 * 16;
       CU(cudaFuncSetAttribute(viterbi_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       CU(dev_fill(rp.counter, 0, 4, st));
       const uint32_t warps = (uint32_t)std::max(1, std::min(16, m->rows_warps));
       const uint32_t grid = (uint32_t)std::min<uint64_t>(((uint64_t)U + 2 * warps - 1) / (2 * warps), (uint64_t)m->num_sms);
       viterbi_rows_kernel<<<grid, warps * 32, smem, st>>>(rp);
-      m->w().stats.launches += 1;
+      m->ws.stats.launches += 1;
       CU(cudaGetLastError());
     }
   } else if (algo == 2 && u.rows <= 16) {
@@ -1171,33 +1149,33 @@ int run_viterbi(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint
     p.u = u;
     p.u.part = 0;
     p.blob_end = d_text + N;
-    p.bp = m->w().bp.as<uint8_t>();
-    p.counter = m->w().small.as<unsigned int>() + 8;
+    p.bp = m->ws.bp.as<uint8_t>();
+    p.counter = m->ws.small.as<unsigned int>() + 8;
     p.dbg = 0;
     DropInfo di;
     di.dropout = dropout;
     di.seed = m->drop_seed;
-    di.unit_base = m->drop_unit_base;
-    if (!p.u.count) {
-    } else {
-      CU(launch_viterbi_pair_r<2>(m, p, N, di));
+    di.unit_base = unit_base;
+    if (p.u.count) {
+      CU(dev_fill(p.counter, 0, 4, st));
+      CU(launch_viterbi_pair_r<2>(m, p, N, di, st, 0, m->groups));
     }
   } else {
     ViterbiParams p;
     p.u = u;
-    p.bp = m->w().bp.as<uint8_t>();
+    p.bp = m->ws.bp.as<uint8_t>();
     p.dropout = dropout;
     p.drop_seed = m->drop_seed;
-    p.unit_base = m->drop_unit_base;
+    p.unit_base = unit_base;
     p.u.part = 1;
     CU(launch_viterbi_g(m, 32, p));
     p.u.part = 2;
     CU(launch_viterbi_g(m, m->g_short, p));
   }
-  CU(cudaEventRecord(m->w().ev[1], st));
-  if (m->w().side_used) CU(cudaStreamWaitEvent(st, m->w().ev_side_join, 0));
-  CU(cudaEventRecord(m->w().ev[12], st));
-  CU(cudaEventRecord(m->w().ev[2], st));
+  CU(cudaEventRecord(m->ws.ev[1], st));
+  if (m->ws.side_used) CU(cudaStreamWaitEvent(st, m->ws.ev_side_join, 0));
+  CU(cudaEventRecord(m->ws.ev[12], st));
+  CU(cudaEventRecord(m->ws.ev[2], st));
   if (U) {
     BacktrackParams b;
     b.unit_start = u.unit_start;
@@ -1206,40 +1184,40 @@ int run_viterbi(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint
     b.counts = counts;
     b.first = 0;
     b.count = U;
-    b.bp = m->w().bp.as<uint8_t>();
-    b.mark = m->w().mark.as<uint8_t>();
-    b.n_tokens = m->w().ntok.as<unsigned long long>();
-    b.status = m->w().status.as<int32_t>();
+    b.bp = m->ws.bp.as<uint8_t>();
+    b.mark = m->ws.mark.as<uint8_t>();
+    b.n_tokens = m->ws.ntok.as<unsigned long long>();
+    b.status = m->ws.status.as<int32_t>();
     // long samples (sorted first): one warp each; short ones: one thread each
     b.part = 1;
     backtrack_warp_kernel<<<nblk(U, BW_WARPS), BW_WARPS * 32, 0, st>>>(b);
     b.part = 2;
     backtrack_thread_kernel<<<nblk(U, BT_THREADS), BT_THREADS, 0, st>>>(b);
-    m->w().stats.launches += 2;
+    m->ws.stats.launches += 2;
     CU(cudaGetLastError());
   }
-  CU(cudaEventRecord(m->w().ev[3], st));
+  CU(cudaEventRecord(m->ws.ev[3], st));
   return TGX_OK;
 }
 
 // Token ids (and/or frequencies) from the marks: count per tile, scan, emit.
 int run_emit(tgx_model* m, const uint8_t* d_text, uint64_t N, uint32_t* d_ids, uint64_t ids_cap,
              unsigned long long* d_freq) {
-  cudaStream_t st = m->w().stream;
+  cudaStream_t st = m->ws.stream;
   const uint64_t n_tiles = (N + EM_TILE - 1) / EM_TILE;
-  CU(cudaEventRecord(m->w().ev[4], st));
+  CU(cudaEventRecord(m->ws.ev[4], st));
   if (n_tiles) {
-    CU(m->w().tilecnt.reserve((n_tiles + 1) * 16));
-    unsigned long long* cnt = m->w().tilecnt.as<unsigned long long>();
+    CU(m->ws.tilecnt.reserve((n_tiles + 1) * 16));
+    unsigned long long* cnt = m->ws.tilecnt.as<unsigned long long>();
     unsigned long long* prefix = cnt + n_tiles + 1;
     const uint32_t grid = (uint32_t)std::min<uint64_t>(n_tiles, (uint64_t)m->num_sms * 8);
-    mark_count_kernel<<<grid, EM_BLOCK, 0, st>>>(m->w().mark.as<uint4>(), n_tiles, cnt);
+    mark_count_kernel<<<grid, EM_BLOCK, 0, st>>>(m->ws.mark.as<uint4>(), n_tiles, cnt);
     size_t tmp = 0;
     CU(cub::DeviceScan::ExclusiveSum(nullptr, tmp, cnt, prefix, (int)n_tiles, st));
-    CU(m->w().cubtmp.reserve(tmp));
-    CU(cub::DeviceScan::ExclusiveSum(m->w().cubtmp.p, tmp, cnt, prefix, (int)n_tiles, st));
+    CU(m->ws.cubtmp.reserve(tmp));
+    CU(cub::DeviceScan::ExclusiveSum(m->ws.cubtmp.p, tmp, cnt, prefix, (int)n_tiles, st));
     EmitParams e;
-    e.mark = m->w().mark.as<uint4>();
+    e.mark = m->ws.mark.as<uint4>();
     e.text = d_text;
     e.text_bytes = N;
     e.n_tiles = n_tiles;
@@ -1255,32 +1233,32 @@ int run_emit(tgx_model* m, const uint8_t* d_text, uint64_t N, uint32_t* d_ids, u
     e.hash_mask = use_hash ? m->hash.mask : 0;
     e.hash_seed = m->hash.seed;
     emit_kernel<<<grid, EM_BLOCK, d_freq ? EM_HOT * 4 : 0, st>>>(e);
-    m->w().stats.launches += 4;
+    m->ws.stats.launches += 4;
     CU(cudaGetLastError());
   }
-  CU(cudaEventRecord(m->w().ev[5], st));
+  CU(cudaEventRecord(m->ws.ev[5], st));
   return TGX_OK;
 }
 
 // Reads up to two device words once everything queued on the compute stream has finished, through
 // the control stream (see tgx_model::stream_ctl); returns with both streams idle.
 int read_words(tgx_model* m, const void* d0, const void* d1, unsigned long long* o0, unsigned long long* o1) {
-  CU(cudaEventRecord(m->w().ev_ctl, m->w().stream));
-  CU(cudaStreamWaitEvent(m->w().stream_ctl, m->w().ev_ctl, 0));
-  if (d0) CU(cudaMemcpyAsync(m->w().h_words, d0, 8, cudaMemcpyDeviceToHost, m->w().stream_ctl));
-  if (d1) CU(cudaMemcpyAsync(m->w().h_words + 1, d1, 8, cudaMemcpyDeviceToHost, m->w().stream_ctl));
-  CU(cudaStreamSynchronize(m->w().stream_ctl));
-  if (d0 && o0) *o0 = m->w().h_words[0];
-  if (d1 && o1) *o1 = m->w().h_words[1];
+  CU(cudaEventRecord(m->ws.ev_ctl, m->ws.stream));
+  CU(cudaStreamWaitEvent(m->ws.stream_ctl, m->ws.ev_ctl, 0));
+  if (d0) CU(cudaMemcpyAsync(m->ws.h_words, d0, 8, cudaMemcpyDeviceToHost, m->ws.stream_ctl));
+  if (d1) CU(cudaMemcpyAsync(m->ws.h_words + 1, d1, 8, cudaMemcpyDeviceToHost, m->ws.stream_ctl));
+  CU(cudaStreamSynchronize(m->ws.stream_ctl));
+  if (d0 && o0) *o0 = m->ws.h_words[0];
+  if (d1 && o1) *o1 = m->ws.h_words[1];
   return TGX_OK;
 }
 
 int first_bad(tgx_model* m, uint32_t U, int64_t* out_idx, const void* extra = nullptr, unsigned long long* extra_out = nullptr) {
-  unsigned long long* d = m->w().small.as<unsigned long long>() + 2;
-  CU(dev_fill(d, 0xFF, 8, m->w().stream));
+  unsigned long long* d = m->ws.small.as<unsigned long long>() + 2;
+  CU(dev_fill(d, 0xFF, 8, m->ws.stream));
   if (U) {
-    first_bad_unit<<<nblk(U, 256), 256, 0, m->w().stream>>>(m->w().status.as<int32_t>(), U, d);
-    m->w().stats.launches += 1;
+    first_bad_unit<<<nblk(U, 256), 256, 0, m->ws.stream>>>(m->ws.status.as<int32_t>(), U, d);
+    m->ws.stats.launches += 1;
   }
   unsigned long long h = ~0ull;
   int rc = read_words(m, d, extra, &h, extra_out);
@@ -1291,19 +1269,19 @@ int first_bad(tgx_model* m, uint32_t U, int64_t* out_idx, const void* extra = nu
 
 void finish_stats(tgx_model* m, int which) {
   float ms = 0;
-  if (cudaEventElapsedTime(&ms, m->w().ev[0], m->w().ev[1]) == cudaSuccess) {
-    if (which == 1) m->w().stats.viterbi_ms = ms;
-    if (which == 2) m->w().stats.fwd_ms = ms;
+  if (cudaEventElapsedTime(&ms, m->ws.ev[0], m->ws.ev[1]) == cudaSuccess) {
+    if (which == 1) m->ws.stats.viterbi_ms = ms;
+    if (which == 2) m->ws.stats.fwd_ms = ms;
   }
-  if (which == 2 && cudaEventElapsedTime(&ms, m->w().ev[2], m->w().ev[3]) == cudaSuccess) m->w().stats.bwd_ms = ms;
-  if (which == 1 && cudaEventElapsedTime(&ms, m->w().ev[2], m->w().ev[3]) == cudaSuccess) m->w().stats.back_ms = ms;
-  if (which == 1 && cudaEventElapsedTime(&ms, m->w().ev[4], m->w().ev[5]) == cudaSuccess) m->w().stats.emit_ms = ms;
-  if (which == 1 && cudaEventElapsedTime(&ms, m->w().ev[8], m->w().ev[9]) == cudaSuccess) m->w().stats.match_ms = ms;
-  if (which == 1 && cudaEventElapsedTime(&ms, m->w().ev[8], m->w().ev[12]) == cudaSuccess) m->w().stats.forward_ms = ms;
-  if (which == 1) m->w().stats.algo = m->w().algo_used;
-  if (which == 1 && m->w().side_used && cudaEventElapsedTime(&ms, m->w().ev[10], m->w().ev[11]) == cudaSuccess) m->w().stats.side_ms = ms;
-  if (cudaEventElapsedTime(&ms, m->w().ev[6], m->w().ev[7]) == cudaSuccess) m->w().stats.total_ms = ms;
-  m->last_stats = m->w().stats;
+  if (which == 2 && cudaEventElapsedTime(&ms, m->ws.ev[2], m->ws.ev[3]) == cudaSuccess) m->ws.stats.bwd_ms = ms;
+  if (which == 1 && cudaEventElapsedTime(&ms, m->ws.ev[2], m->ws.ev[3]) == cudaSuccess) m->ws.stats.back_ms = ms;
+  if (which == 1 && cudaEventElapsedTime(&ms, m->ws.ev[4], m->ws.ev[5]) == cudaSuccess) m->ws.stats.emit_ms = ms;
+  if (which == 1 && cudaEventElapsedTime(&ms, m->ws.ev[8], m->ws.ev[9]) == cudaSuccess) m->ws.stats.match_ms = ms;
+  if (which == 1 && cudaEventElapsedTime(&ms, m->ws.ev[8], m->ws.ev[12]) == cudaSuccess) m->ws.stats.forward_ms = ms;
+  if (which == 1) m->ws.stats.algo = m->ws.algo_used;
+  if (which == 1 && m->ws.side_used && cudaEventElapsedTime(&ms, m->ws.ev[10], m->ws.ev[11]) == cudaSuccess) m->ws.stats.side_ms = ms;
+  if (cudaEventElapsedTime(&ms, m->ws.ev[6], m->ws.ev[7]) == cudaSuccess) m->ws.stats.total_ms = ms;
+  m->last_stats = m->ws.stats;
 }
 
 }  // namespace
@@ -1336,29 +1314,27 @@ int tgx_model_create(const uint8_t* token_bytes, const uint64_t* token_offsets, 
     CU(cudaMemcpyToSymbol(tgxk::c_log_hdr, TGX_LOG_HDR, sizeof(TGX_LOG_HDR)));
     CU(cudaMemcpyToSymbol(tgxk::c_exp_tab, TGX_EXP_TAB, sizeof(TGX_EXP_TAB)));
     CU(cudaMemcpyToSymbol(tgxk::c_log_tab, TGX_LOG_TAB, sizeof(TGX_LOG_TAB)));
-    for (auto& w : m->ws) {
-      CU(cudaStreamCreateWithFlags(&w.stream, cudaStreamNonBlocking));
-      CU(cudaStreamCreateWithFlags(&w.stream_ctl, cudaStreamNonBlocking));
-      CU(cudaEventCreateWithFlags(&w.ev_ctl, cudaEventDisableTiming));
-      {  // forked when match_kernel has finished: pair CTAs first, then the teams, then the spare team CTAs
-        int lo = 0, hi = 0;
-        CU(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-        CU(cudaStreamCreateWithPriority(&w.stream_side, cudaStreamNonBlocking, hi));
-        CU(cudaStreamCreateWithPriority(&w.stream_low, cudaStreamNonBlocking, lo));
-      }
-      CU(cudaEventCreateWithFlags(&w.ev_low_join, cudaEventDisableTiming));
-      CU(cudaEventCreateWithFlags(&w.ev_side_fork, cudaEventDisableTiming));
-      CU(cudaEventCreateWithFlags(&w.ev_side_join, cudaEventDisableTiming));
-      CU(cudaHostAlloc(reinterpret_cast<void**>(&w.h_words), 64, cudaHostAllocDefault));
-      for (auto& e : w.ev) CU(cudaEventCreate(&e));
+    Workspace& w = m->ws;
+    CU(cudaStreamCreateWithFlags(&w.stream, cudaStreamNonBlocking));
+    CU(cudaStreamCreateWithFlags(&w.stream_ctl, cudaStreamNonBlocking));
+    CU(cudaEventCreateWithFlags(&w.ev_ctl, cudaEventDisableTiming));
+    {  // forked when match_kernel has finished: pair CTAs first, then the teams, then the spare team CTAs
+      int lo = 0, hi = 0;
+      CU(cudaDeviceGetStreamPriorityRange(&lo, &hi));
+      CU(cudaStreamCreateWithPriority(&w.stream_side, cudaStreamNonBlocking, hi));
+      CU(cudaStreamCreateWithPriority(&w.stream_low, cudaStreamNonBlocking, lo));
     }
+    CU(cudaEventCreateWithFlags(&w.ev_low_join, cudaEventDisableTiming));
+    CU(cudaEventCreateWithFlags(&w.ev_side_fork, cudaEventDisableTiming));
+    CU(cudaEventCreateWithFlags(&w.ev_side_join, cudaEventDisableTiming));
+    CU(cudaHostAlloc(reinterpret_cast<void**>(&w.h_words), 64, cudaHostAllocDefault));
+    for (auto& e : w.ev) CU(cudaEventCreate(&e));
     CU(cudaStreamCreateWithFlags(&m->stream2, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&m->stream3, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&m->stream4, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&m->stream5, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&m->stream6, cudaStreamNonBlocking));
     CU(cudaEventCreateWithFlags(&m->ev_join6, cudaEventDisableTiming));
-    for (auto& e : m->ev_grp) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     CU(cudaEventCreateWithFlags(&m->ev_join5, cudaEventDisableTiming));
     CU(cudaEventCreateWithFlags(&m->ev_join3, cudaEventDisableTiming));
     CU(cudaEventCreateWithFlags(&m->ev_join4, cudaEventDisableTiming));
@@ -1375,9 +1351,9 @@ int tgx_model_create(const uint8_t* token_bytes, const uint64_t* token_offsets, 
     size_t bytes = m->da.slots.size() * sizeof(tgx::Slot);
     CU(cudaMalloc(&m->d_trie, bytes));
     m->trie_cap = m->da.slots.size();
-    CU(cudaMemcpyAsync(m->d_trie, m->da.slots.data(), bytes, cudaMemcpyHostToDevice, m->w().stream));
-    CU(cudaStreamSynchronize(m->w().stream));
-    int rc = upload_aux_tables(m.get(), m->da, token_bytes, token_offsets, vocab_size, m->da.max_token_len);
+    CU(cudaMemcpyAsync(m->d_trie, m->da.slots.data(), bytes, cudaMemcpyHostToDevice, m->ws.stream));
+    CU(cudaStreamSynchronize(m->ws.stream));
+    int rc = upload_aux_tables(m.get(), token_bytes, token_offsets, vocab_size, m->da.max_token_len);
     if (rc) return rc;
   }
   *out = m.release();
@@ -1418,7 +1394,7 @@ int tgx_model_rebuild(tgx_model* m, const uint8_t* token_bytes, const uint64_t* 
   const tgx::DoubleArray& da = m->da;
   if (m->device >= 0) {
     CU(cudaSetDevice(m->device));
-    CU(cudaStreamSynchronize(m->w().stream));
+    CU(cudaStreamSynchronize(m->ws.stream));
     if (da.slots.size() > m->trie_cap) {
       uint4* p = nullptr;
       CU(cudaMalloc(&p, da.slots.size() * sizeof(tgx::Slot)));
@@ -1426,10 +1402,10 @@ int tgx_model_rebuild(tgx_model* m, const uint8_t* token_bytes, const uint64_t* 
       m->d_trie = p;
       m->trie_cap = da.slots.size();
     }
-    CU(cudaMemcpyAsync(m->d_trie, da.slots.data(), da.slots.size() * sizeof(tgx::Slot), cudaMemcpyHostToDevice, m->w().stream));
-    CU(cudaStreamSynchronize(m->w().stream));
+    CU(cudaMemcpyAsync(m->d_trie, da.slots.data(), da.slots.size() * sizeof(tgx::Slot), cudaMemcpyHostToDevice, m->ws.stream));
+    CU(cudaStreamSynchronize(m->ws.stream));
     if (hash_thread.joinable()) hash_thread.join();
-    int rc = upload_aux_tables(m, da, token_bytes, token_offsets, vocab_size, da.max_token_len, &hash, &hash_err);
+    int rc = upload_aux_tables(m, token_bytes, token_offsets, vocab_size, da.max_token_len, &hash, &hash_err);
     if (rc) return rc;
   }
   return TGX_OK;
@@ -1439,42 +1415,26 @@ void tgx_model_destroy(tgx_model* m) {
   if (!m) return;
   if (m->device >= 0) {
     cudaSetDevice(m->device);
-    cudaDeviceSynchronize();
-    m->Bbeta.release();
-    m->accfix.release();
-    DevBuf* bufs[] = {&m->text, &m->off, &m->idoff, &m->A, &m->expected, &m->freq, &m->ids, &m->scount, &m->hot,
-                      &m->text_b, &m->off_b, &m->ids_b, &m->idoff_b, &m->scount_b};
-    for (auto* b : bufs) b->release();
-    for (auto& w : m->ws) {
-      DevBuf* wb[] = {&w.text2, &w.off2, &w.bitmap, &w.blk, &w.ustart, &w.ulen, &w.keys_out, &w.vals_in, &w.vals_out,
-                      &w.cubtmp, &w.bp, &w.mark, &w.tilecnt, &w.ntok, &w.status, &w.small, &w.rec};
-      for (auto* b : wb) b->release();
-      for (auto& e : w.ev)
-        if (e) cudaEventDestroy(e);
-      if (w.stream) cudaStreamDestroy(w.stream);
-      if (w.stream_ctl) cudaStreamDestroy(w.stream_ctl);
-      if (w.ev_ctl) cudaEventDestroy(w.ev_ctl);
-      if (w.stream_side) cudaStreamDestroy(w.stream_side);
-      if (w.stream_low) cudaStreamDestroy(w.stream_low);
-      if (w.ev_low_join) cudaEventDestroy(w.ev_low_join);
-      if (w.ev_side_fork) cudaEventDestroy(w.ev_side_fork);
-      if (w.ev_side_join) cudaEventDestroy(w.ev_side_join);
-      if (w.h_words) cudaFreeHost(w.h_words);
-    }
+    cudaDeviceSynchronize();  // (the DevBuf members free their memory when `m` is deleted below)
+    const Workspace& w = m->ws;
+    for (auto& e : w.ev)
+      if (e) cudaEventDestroy(e);
+    if (w.stream) cudaStreamDestroy(w.stream);
+    if (w.stream_ctl) cudaStreamDestroy(w.stream_ctl);
+    if (w.ev_ctl) cudaEventDestroy(w.ev_ctl);
+    if (w.stream_side) cudaStreamDestroy(w.stream_side);
+    if (w.stream_low) cudaStreamDestroy(w.stream_low);
+    if (w.ev_low_join) cudaEventDestroy(w.ev_low_join);
+    if (w.ev_side_fork) cudaEventDestroy(w.ev_side_fork);
+    if (w.ev_side_join) cudaEventDestroy(w.ev_side_join);
+    if (w.h_words) cudaFreeHost(w.h_words);
     if (m->d_trie) cudaFree(m->d_trie);
-    m->d_hash.release();
-    m->d_trie8.release();
-    m->d_rows.release();
-    m->d_pair2.release();
-    m->d_rowids.release();
     if (m->stream2) cudaStreamDestroy(m->stream2);
     if (m->stream3) cudaStreamDestroy(m->stream3);
     if (m->stream4) cudaStreamDestroy(m->stream4);
     if (m->stream5) cudaStreamDestroy(m->stream5);
     if (m->stream6) cudaStreamDestroy(m->stream6);
     if (m->ev_join6) cudaEventDestroy(m->ev_join6);
-    for (auto& e : m->ev_grp)
-      if (e) cudaEventDestroy(e);
     if (m->ev_join5) cudaEventDestroy(m->ev_join5);
     if (m->ev_join3) cudaEventDestroy(m->ev_join3);
     if (m->ev_join4) cudaEventDestroy(m->ev_join4);
@@ -1485,9 +1445,6 @@ void tgx_model_destroy(tgx_model* m) {
       if (m->ev_d2h[i]) cudaEventDestroy(m->ev_d2h[i]);
       for (auto& e : m->ev_split[i])
         if (e) cudaEventDestroy(e);
-      m->raw[i].release();
-      m->split[i].release();
-      m->fin[i].release();
     }
     if (m->h_off) cudaFreeHost(m->h_off);
     if (m->h_out) cudaFreeHost(m->h_out);
@@ -1548,7 +1505,6 @@ int tgx_model_set_option(tgx_model* m, int key, int64_t value) {
     case 20: if (value < 1 || value > 4096) return fail(TGX_ERR_INVALID, "replicas must be 1..4096"); m->hot_r = (int)value; break;
     case 21: if (value < 0 || value > (1 << 20)) return fail(TGX_ERR_INVALID, "hot ids must be 0..2^20"); m->hot_k = (int)value; break;
     case 18: if (value < 0 || value > 16) return fail(TGX_ERR_INVALID, "blocks per SM must be 0..16"); m->lane_blocks_per_sm = (int)value; break;
-    case 11: m->overlap_chunks = value ? 1 : 0; break;
     case 14: if (value < 0 || value > 2) return fail(TGX_ERR_INVALID, "pair shape must be 0..2"); m->pair_shape = (int)value; break;
     case 13: if (value < 0 || value > 2) return fail(TGX_ERR_INVALID, "hot levels must be 0..2"); m->hot_levels = (int)value; break;
     case 7: if (value < 4096) return fail(TGX_ERR_INVALID, "chunk bytes must be >= 4096"); m->chunk_bytes = (uint64_t)value; break;
@@ -1650,78 +1606,79 @@ int tgx_crlf_batch(tgx_model* m, const uint8_t* text, const uint64_t* off, uint6
   if (rc) return rc;
   if (!off || !out_off || off[0] != 0) return fail(TGX_ERR_INVALID, "offsets must start at 0");
   std::lock_guard<std::recursive_mutex> g(m->mu);
-  m->w().stats = Stats();
+  m->ws.stats = Stats();
   uint64_t N = off[S];
   CU(m->text.reserve(N + 16));
   CU(m->off.reserve((S + 1) * 8));
-  CU(cudaMemcpyAsync(m->text.p, text, N, cudaMemcpyHostToDevice, m->w().stream));
-  CU(cudaMemcpyAsync(m->off.p, off, (S + 1) * 8, cudaMemcpyHostToDevice, m->w().stream));
+  CU(cudaMemcpyAsync(m->text.p, text, N, cudaMemcpyHostToDevice, m->ws.stream));
+  CU(cudaMemcpyAsync(m->off.p, off, (S + 1) * 8, cudaMemcpyHostToDevice, m->ws.stream));
   rc = run_crlf(m, m->text.as<uint8_t>(), m->off.as<uint64_t>(), S, N);
   if (rc) return rc;
-  CU(cudaMemcpyAsync(out_off, m->w().off2.p, (S + 1) * 8, cudaMemcpyDeviceToHost, m->w().stream));
-  CU(cudaStreamSynchronize(m->w().stream));
-  CU(cudaMemcpyAsync(out_text, m->w().text2.p, out_off[S], cudaMemcpyDeviceToHost, m->w().stream));
-  CU(cudaStreamSynchronize(m->w().stream));
+  CU(cudaMemcpyAsync(out_off, m->ws.off2.p, (S + 1) * 8, cudaMemcpyDeviceToHost, m->ws.stream));
+  CU(cudaStreamSynchronize(m->ws.stream));
+  CU(cudaMemcpyAsync(out_text, m->ws.text2.p, out_off[S], cudaMemcpyDeviceToHost, m->ws.stream));
+  CU(cudaStreamSynchronize(m->ws.stream));
   return TGX_OK;
 }
 
 // ---------------------------------------------------------------------------- encode
 namespace {
 
-// Queues every kernel of one encode batch on the current workspace; nothing here waits for the device.
+// Queues every kernel of one encode batch on the workspace; nothing here waits for the device.  `unit_base`: see
+// run_viterbi.
 int encode_enqueue(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint64_t S, uint64_t n_bytes,
                    uint32_t flags, uint32_t* d_ids, uint64_t ids_cap, uint64_t* d_id_off, int32_t* d_status,
-                   uint64_t* d_proc_len, bool with_dropout = false) {
-  m->w().stats = Stats();
-  cudaStream_t st = m->w().stream;
-  CU(cudaEventRecord(m->w().ev[6], st));
+                   uint64_t* d_proc_len, bool with_dropout = false, uint64_t unit_base = 0) {
+  m->ws.stats = Stats();
+  cudaStream_t st = m->ws.stream;
+  CU(cudaEventRecord(m->ws.ev[6], st));
   const uint8_t* text = d_text;
   const uint64_t* off = d_off;
   int rc;
   if (flags & TGX_FLAG_CRLF) {
     rc = run_crlf(m, d_text, d_off, S, n_bytes);
     if (rc) return rc;
-    text = m->w().text2.as<uint8_t>();
-    off = m->w().off2.as<uint64_t>();
+    text = m->ws.text2.as<uint8_t>();
+    off = m->ws.off2.as<uint64_t>();
   }
-  rc = run_viterbi(m, text, off, S, n_bytes, d_proc_len, with_dropout);
+  rc = run_viterbi(m, text, off, S, n_bytes, d_proc_len, with_dropout, unit_base);
   if (rc) return rc;
   // id offsets = exclusive scan of token counts (S+1 entries; ntok[S] was zeroed)
   size_t tmp = 0;
-  CU(cub::DeviceScan::ExclusiveSum(nullptr, tmp, m->w().ntok.as<unsigned long long>(),
+  CU(cub::DeviceScan::ExclusiveSum(nullptr, tmp, m->ws.ntok.as<unsigned long long>(),
                                    reinterpret_cast<unsigned long long*>(d_id_off), (int)(S + 1), st));
-  CU(m->w().cubtmp.reserve(tmp));
-  CU(cub::DeviceScan::ExclusiveSum(m->w().cubtmp.p, tmp, m->w().ntok.as<unsigned long long>(),
+  CU(m->ws.cubtmp.reserve(tmp));
+  CU(cub::DeviceScan::ExclusiveSum(m->ws.cubtmp.p, tmp, m->ws.ntok.as<unsigned long long>(),
                                    reinterpret_cast<unsigned long long*>(d_id_off), (int)(S + 1), st));
-  m->w().stats.launches += 2;
+  m->ws.stats.launches += 2;
   rc = run_emit(m, text, n_bytes, d_ids, ids_cap, nullptr);
   if (rc) return rc;
   if (d_status) {  // (a kernel, not a D2D memcpy: keep the compute stream off the copy engines)
-    copy_u32<<<nblk(S, 256), 256, 0, st>>>(reinterpret_cast<const uint32_t*>(m->w().status.p),
+    copy_u32<<<nblk(S, 256), 256, 0, st>>>(reinterpret_cast<const uint32_t*>(m->ws.status.p),
                                            reinterpret_cast<uint32_t*>(d_status), S);
-    m->w().stats.launches += 1;
+    m->ws.stats.launches += 1;
   }
   // control words: lowest failing sample and the total id count, read through the control stream
-  unsigned long long* d = m->w().small.as<unsigned long long>() + 2;
+  unsigned long long* d = m->ws.small.as<unsigned long long>() + 2;
   CU(dev_fill(d, 0xFF, 8, st));
-  first_bad_unit<<<nblk(S, 256), 256, 0, st>>>(m->w().status.as<int32_t>(), (uint32_t)S, d);
-  m->w().stats.launches += 1;
-  CU(cudaEventRecord(m->w().ev[7], st));
-  CU(cudaEventRecord(m->w().ev_ctl, st));
-  CU(cudaStreamWaitEvent(m->w().stream_ctl, m->w().ev_ctl, 0));
-  CU(cudaMemcpyAsync(m->w().h_words, d, 8, cudaMemcpyDeviceToHost, m->w().stream_ctl));
-  CU(cudaMemcpyAsync(m->w().h_words + 1, d_id_off + S, 8, cudaMemcpyDeviceToHost, m->w().stream_ctl));
+  first_bad_unit<<<nblk(S, 256), 256, 0, st>>>(m->ws.status.as<int32_t>(), (uint32_t)S, d);
+  m->ws.stats.launches += 1;
+  CU(cudaEventRecord(m->ws.ev[7], st));
+  CU(cudaEventRecord(m->ws.ev_ctl, st));
+  CU(cudaStreamWaitEvent(m->ws.stream_ctl, m->ws.ev_ctl, 0));
+  CU(cudaMemcpyAsync(m->ws.h_words, d, 8, cudaMemcpyDeviceToHost, m->ws.stream_ctl));
+  CU(cudaMemcpyAsync(m->ws.h_words + 1, d_id_off + S, 8, cudaMemcpyDeviceToHost, m->ws.stream_ctl));
   return TGX_OK;
 }
 
-// Waits for the batch queued on the current workspace; total id count and lowest failing sample (-1 = none).
+// Waits for the batch queued on the workspace; total id count and lowest failing sample (-1 = none).
 int encode_finish(tgx_model* m, uint64_t* total_ids, int64_t* bad) {
-  CU(cudaStreamSynchronize(m->w().stream_ctl));
-  CU(cudaStreamSynchronize(m->w().stream));
+  CU(cudaStreamSynchronize(m->ws.stream_ctl));
+  CU(cudaStreamSynchronize(m->ws.stream));
   finish_stats(m, 1);
-  const unsigned long long h = m->w().h_words[0];
+  const unsigned long long h = m->ws.h_words[0];
   *bad = (h == ~0ull) ? -1 : (int64_t)h;
-  *total_ids = m->w().h_words[1];
+  *total_ids = m->ws.h_words[1];
   return TGX_OK;
 }
 
@@ -1739,11 +1696,10 @@ int tgx_encode_batch_dev(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
   if (total_ids) *total_ids = 0;
   if (S >= (1ull << 32)) return fail(TGX_ERR_INVALID, "too many samples in one call (< 2^32)");
   if (S == 0) {
-    CU(dev_fill(d_id_off, 0, 8, m->w().stream));
-    CU(cudaStreamSynchronize(m->w().stream));
+    CU(dev_fill(d_id_off, 0, 8, m->ws.stream));
+    CU(cudaStreamSynchronize(m->ws.stream));
     return TGX_OK;
   }
-  m->drop_unit_base = 0;
   rc = encode_enqueue(m, d_text, d_off, S, n_bytes, flags, d_ids, ids_cap, d_id_off, d_status, d_proc_len, true);
   if (rc) return rc;
   uint64_t tot = 0;
@@ -1771,8 +1727,8 @@ struct ChunkInput {
   virtual ~ChunkInput() = default;
   // Queues the H2D copy of chunk k on `st` (the copy-in stream when K > 1); returns without waiting.
   virtual int h2d(tgx_model* m, uint64_t k, int b, cudaStream_t st) = 0;
-  // Queued on the compute stream of chunk k's workspace right after the copy was queued (so behind the previous
-  // chunk's kernels); returns without waiting.
+  // Queued on the compute stream right after the copy was queued (so behind the previous chunk's kernels); returns
+  // without waiting.
   virtual int after_h2d(tgx_model*, uint64_t, int) { return TGX_OK; }
   // Chunk k's first sample, sample count and text bytes once its blob + offsets are (queued to be) in set b.  May wait.
   virtual int samples(tgx_model* m, uint64_t k, int b, uint64_t* s0, uint64_t* S, uint64_t* n) = 0;
@@ -1816,20 +1772,15 @@ int encode_chunks(tgx_model* m, uint32_t flags, uint64_t unit_base, ChunkInput& 
     return TGX_OK;
   };
   std::vector<cudaEvent_t> tev;  // trace: [base, per chunk: h2d0,h2d1,c0,c1,d2h0,d2h1]
-  const bool overlap = K > 1 && m->overlap_chunks;
   auto h2d = [&](uint64_t k) -> int {
     const int b = (int)(k & 1);
-    cudaStream_t st = K > 1 ? m->stream_h2d : m->w().stream;
+    cudaStream_t st = K > 1 ? m->stream_h2d : m->ws.stream;
     if (!tev.empty()) cudaEventRecord(tev[1 + 6 * k + 0], st);
     int r = in.h2d(m, k, b, st);
     if (r) return r;
     if (!tev.empty()) cudaEventRecord(tev[1 + 6 * k + 1], st);
     if (K > 1) CU(cudaEventRecord(m->ev_h2d[b], st));
-    const int wi = m->wi;
-    m->wi = overlap ? b : 0;
-    r = in.after_h2d(m, k, b);
-    m->wi = wi;
-    return r;
+    return in.after_h2d(m, k, b);
   };
   const bool trace = getenv("TGX_TRACE") != nullptr;
   auto now_ms = [] {
@@ -1841,19 +1792,19 @@ int encode_chunks(tgx_model* m, uint32_t flags, uint64_t unit_base, ChunkInput& 
   if (trace) {
     tev.resize(1 + 6 * K);
     for (auto& e : tev) cudaEventCreate(&e);
-    cudaEventRecord(tev[0], m->w().stream);
+    cudaEventRecord(tev[0], m->ws.stream);
   }
-  // Pipeline over chunks k = 0..K-1 with two buffer sets and two workspaces (set / workspace k & 1):
-  //   H2D(k+1) on the copy-in stream, kernels(k+1) QUEUED on the other workspace before the host waits for
-  //   chunk k, D2H(k) on the copy-out stream.  Queuing the next chunk early lets its kernels take over the SMs
-  //   that chunk k's forward kernel frees while its last long samples finish on a few SMs.
+  // Pipeline over chunks k = 0..K-1 with two buffer sets (set k & 1) and one workspace: H2D(k+1) on the copy-in
+  // stream, then the host waits for chunk k's kernels, queues D2H(k) on the copy-out stream and then chunk k+1's
+  // kernels.  (Queuing chunk k+1's kernels before chunk k has finished, on a second workspace, was measured on B200
+  // and lost: 75.4 against 67.6 ms for 1 GB in two chunks — the next chunk's persistent forward CTAs take every SM
+  // the moment the current forward kernel drains, and chunk k's backtrack / emit kernels wait for them to exit.)
   std::vector<uint64_t> s0s(K, 0), Sks(K, 0), nbs(K, 0);
   auto enqueue = [&](uint64_t k) -> int {
     const int b = (int)(k & 1);
-    m->wi = overlap ? b : 0;
     if (K > 1) {
-      CU(cudaStreamWaitEvent(m->w().stream, m->ev_h2d[b], 0));
-      if (k >= 2) CU(cudaStreamWaitEvent(m->w().stream, m->ev_d2h[b], 0));  // the set's previous results left the device
+      CU(cudaStreamWaitEvent(m->ws.stream, m->ev_h2d[b], 0));
+      if (k >= 2) CU(cudaStreamWaitEvent(m->ws.stream, m->ev_d2h[b], 0));  // the set's previous results left the device
     }
     uint64_t s0 = 0, Sk = 0, nb = 0;
     int r = in.samples(m, k, b, &s0, &Sk, &nb);
@@ -1866,15 +1817,16 @@ int encode_chunks(tgx_model* m, uint32_t flags, uint64_t unit_base, ChunkInput& 
     if (r) return r;
     int32_t* dst = set_sc(m, b)->as<int32_t>();
     uint64_t* dpl = reinterpret_cast<uint64_t*>(set_sc(m, b)->as<unsigned char>() + ((Sk * 4 + 15) & ~15ull));
-    if (!tev.empty()) cudaEventRecord(tev[1 + 6 * k + 2], m->w().stream);
+    if (!tev.empty()) cudaEventRecord(tev[1 + 6 * k + 2], m->ws.stream);
     if (Sk == 0) return TGX_OK;
-    m->drop_unit_base = unit_base + s0;  // the draw is keyed by the sample's index in the whole input, not in its chunk
+    // unit_base + s0: the draw is keyed by the sample's index in the whole input, not in its chunk
     r = encode_enqueue(m, set_text(m, b)->as<uint8_t>(), set_off(m, b)->as<uint64_t>(), Sk, nb, flags,
-                       set_ids(m, b)->as<uint32_t>(), nb + 4, set_idoff(m, b)->as<uint64_t>(), dst, dpl, true);
+                       set_ids(m, b)->as<uint32_t>(), nb + 4, set_idoff(m, b)->as<uint64_t>(), dst, dpl, true,
+                       unit_base + s0);
     if (r) return r;
     r = out.after_encode(m, k, b, Sk);
     if (r) return r;
-    if (!tev.empty()) cudaEventRecord(tev[1 + 6 * k + 3], m->w().stream);
+    if (!tev.empty()) cudaEventRecord(tev[1 + 6 * k + 3], m->ws.stream);
     return TGX_OK;
   };
   // (a failure below leaves copies in flight: callers' buffers are written until the streams drain)
@@ -1883,7 +1835,7 @@ int encode_chunks(tgx_model* m, uint32_t flags, uint64_t unit_base, ChunkInput& 
       cudaStreamSynchronize(m->stream_h2d);
       cudaStreamSynchronize(m->stream_d2h);
     }
-    for (auto& w : m->ws) cudaStreamSynchronize(w.stream);
+    cudaStreamSynchronize(m->ws.stream);
     for (auto& e : tev) cudaEventDestroy(e);
     return rc;
   };
@@ -1898,17 +1850,12 @@ int encode_chunks(tgx_model* m, uint32_t flags, uint64_t unit_base, ChunkInput& 
     if (k + 1 < K) {
       rc = h2d(k + 1);
       if (rc) return drain(rc);
-      if (overlap) {
-        rc = enqueue(k + 1);
-        if (rc) return drain(rc);
-      }
     }
     const uint64_t s0 = s0s[k], Sk = Sks[k];
     int32_t* dst = set_sc(m, b)->as<int32_t>();
     uint64_t* dpl = reinterpret_cast<uint64_t*>(set_sc(m, b)->as<unsigned char>() + ((Sk * 4 + 15) & ~15ull));
     uint64_t tot = 0;
     int64_t bad = -1;
-    m->wi = overlap ? b : 0;
     if (Sk) {
       rc = encode_finish(m, &tot, &bad);
       if (rc) return drain(rc);
@@ -1918,20 +1865,19 @@ int encode_chunks(tgx_model* m, uint32_t flags, uint64_t unit_base, ChunkInput& 
               (unsigned long long)K, now_ms() - t_begin, m->last_stats.total_ms);
     if (tot > nbs[k] + 4) return drain(fail(TGX_ERR_CUDA, "internal: more ids than bytes"));
     if (bad >= 0 && bad_all < 0) bad_all = (int64_t)(s0 + bad);
-    cudaStream_t st = K > 1 ? m->stream_d2h : m->w().stream;  // the chunk's kernels have finished
+    cudaStream_t st = K > 1 ? m->stream_d2h : m->ws.stream;  // the chunk's kernels have finished
     if (!tev.empty()) cudaEventRecord(tev[1 + 6 * k + 4], st);
     rc = out.d2h(m, k, b, s0, Sk, tot, base, bad, dst, dpl, st);
     if (rc) return drain(rc);
     if (K > 1) CU(cudaEventRecord(m->ev_d2h[b], st));
     if (!tev.empty()) cudaEventRecord(tev[1 + 6 * k + 5], st);
     base += tot;
-    if (!overlap && k + 1 < K) {
+    if (k + 1 < K) {
       rc = enqueue(k + 1);
       if (rc) return drain(rc);
     }
   }
-  CU(cudaStreamSynchronize(K > 1 ? m->stream_d2h : m->w().stream));
-  m->wi = 0;
+  CU(cudaStreamSynchronize(K > 1 ? m->stream_d2h : m->ws.stream));
   if (trace) {
     fprintf(stderr, "[tgx] all copies done at %.2f ms\n", now_ms() - t_begin);
     cudaDeviceSynchronize();
@@ -2039,7 +1985,7 @@ struct CorpusInput : ChunkInput {
   }
   KeptStarts* tile_counts(tgx_model* m, int b) { return reinterpret_cast<KeptStarts*>(m->split[b].as<unsigned char>() + 32); }
   int after_h2d(tgx_model* m, uint64_t k, int b) override {
-    cudaStream_t st = m->w().stream;
+    cudaStream_t st = m->ws.stream;
     if (K > 1) CU(cudaStreamWaitEvent(st, m->ev_h2d[b], 0));
     const uint64_t N = cut[k + 1] - cut[k], n_tiles = (N + CRLF_TILE - 1) / CRLF_TILE;
     // m->split[b]: bad_pos, words[3], tile counts (n_tiles + 1), their exclusive scan (n_tiles + 1)
@@ -2056,20 +2002,20 @@ struct CorpusInput : ChunkInput {
     size_t tmp = 0;
     CU(cub::DeviceScan::ExclusiveScan(nullptr, tmp, cnt, prefix, AddKeptStarts(), KeptStarts{0, 0}, (int)(n_tiles + 1),
                                       st));
-    CU(m->w().cubtmp.reserve(tmp));
-    CU(cub::DeviceScan::ExclusiveScan(m->w().cubtmp.p, tmp, cnt, prefix, AddKeptStarts(), KeptStarts{0, 0},
+    CU(m->ws.cubtmp.reserve(tmp));
+    CU(cub::DeviceScan::ExclusiveScan(m->ws.cubtmp.p, tmp, cnt, prefix, AddKeptStarts(), KeptStarts{0, 0},
                                       (int)(n_tiles + 1), st));
     corpus_words<<<1, 32, 0, st>>>(raw, prefix, n_tiles, bad_pos, words);
     CU(cudaGetLastError());
     CU(cudaEventRecord(m->ev_split[b][1], st));
-    CU(cudaEventRecord(m->w().ev_ctl, st));
-    CU(cudaStreamWaitEvent(m->w().stream_ctl, m->w().ev_ctl, 0));
-    CU(cudaMemcpyAsync(m->w().h_words + 4, words, 24, cudaMemcpyDeviceToHost, m->w().stream_ctl));
+    CU(cudaEventRecord(m->ws.ev_ctl, st));
+    CU(cudaStreamWaitEvent(m->ws.stream_ctl, m->ws.ev_ctl, 0));
+    CU(cudaMemcpyAsync(m->ws.h_words + 4, words, 24, cudaMemcpyDeviceToHost, m->ws.stream_ctl));
     return TGX_OK;
   }
   int samples(tgx_model* m, uint64_t k, int b, uint64_t* s0, uint64_t* S, uint64_t* n) override {
-    CU(cudaStreamSynchronize(m->w().stream_ctl));
-    const uint64_t Sk = m->w().h_words[4], kept = m->w().h_words[5], bad = m->w().h_words[6];
+    CU(cudaStreamSynchronize(m->ws.stream_ctl));
+    const uint64_t Sk = m->ws.h_words[4], kept = m->ws.h_words[5], bad = m->ws.h_words[6];
     float ms = 0;
     if (cudaEventElapsedTime(&ms, m->ev_split[b][0], m->ev_split[b][1]) == cudaSuccess) split_ms += ms;
     if (bad != ~0ull) {
@@ -2086,7 +2032,7 @@ struct CorpusInput : ChunkInput {
       }
     }
     CU(set_off(m, b)->reserve((Sk + 1) * 8));
-    cudaStream_t st = m->w().stream;
+    cudaStream_t st = m->ws.stream;
     CU(cudaEventRecord(m->ev_split[b][2], st));
     if (n_tiles)
       corpus_scatter<<<(uint32_t)n_tiles, CRLF_BLOCK, 0, st>>>(m->raw[b].as<uint8_t>(), N, tile_counts(m, b) + n_tiles + 1,
@@ -2123,7 +2069,7 @@ struct CorpusOutput : ChunkOutput {
   int after_encode(tgx_model* m, uint64_t, int b, uint64_t Sk) override {
     if (!finalize()) return TGX_OK;
     CU(m->fin[b].reserve((in->max_b + 4 + Sk) * id_bytes));
-    cudaStream_t st = m->w().stream;
+    cudaStream_t st = m->ws.stream;
     const uint32_t grid = (uint32_t)m->num_sms * 8;
     const uint32_t* d_ids = set_ids(m, b)->as<uint32_t>();
     const uint64_t* d_idoff = set_idoff(m, b)->as<uint64_t>();
@@ -2131,7 +2077,7 @@ struct CorpusOutput : ChunkOutput {
       corpus_finalize<uint16_t><<<grid, 256, 0, st>>>(d_ids, d_idoff, Sk, sep, m->fin[b].as<uint16_t>());
     else
       corpus_finalize<uint32_t><<<grid, 256, 0, st>>>(d_ids, d_idoff, Sk, sep, m->fin[b].as<uint32_t>());
-    m->w().stats.launches += 1;
+    m->ws.stats.launches += 1;
     CU(cudaGetLastError());
     return TGX_OK;
   }
@@ -2169,10 +2115,6 @@ int tgx_encode_batch(tgx_model* m, const uint8_t* text, const uint64_t* off, uin
     if (off[i + 1] - off[i] >= (1ull << 32)) return fail(TGX_ERR_UNSUPPORTED, "a sample of 4 GiB or more is not supported");
   }
   std::lock_guard<std::recursive_mutex> g(m->mu);
-  struct WiGuard {  // whatever path leaves this function, the next call starts on workspace 0
-    tgx_model* m;
-    ~WiGuard() { m->wi = 0; }
-  } wi_guard{m};
   if (first_bad_out) *first_bad_out = -1;
   if (S == 0) {
     id_off[0] = 0;
@@ -2237,10 +2179,6 @@ int tgx_encode_corpus(tgx_model* m, const uint8_t* data, uint64_t n, uint32_t fl
   if (id_bytes == 2 && (m->V > 65536 || sep_id >= 65536))
     return fail(TGX_ERR_UNSUPPORTED, "16-bit ids need a vocabulary (and separator) below 65536");
   std::lock_guard<std::recursive_mutex> g(m->mu);
-  struct WiGuard {
-    tgx_model* m;
-    ~WiGuard() { m->wi = 0; }
-  } wi_guard{m};
   *n_samples = *n_ids = 0;
   if (first_bad) *first_bad = -1;
   if (bad_pos) *bad_pos = 0;
@@ -2309,18 +2247,18 @@ int tgx_token_frequencies_dev(tgx_model* m, const uint8_t* d_text, const uint64_
   if (rc) return rc;
   if (!d_off || !d_freq) return fail(TGX_ERR_INVALID, "null argument");
   std::lock_guard<std::recursive_mutex> g(m->mu);
-  m->w().stats = Stats();
-  cudaStream_t st = m->w().stream;
+  m->ws.stats = Stats();
+  cudaStream_t st = m->ws.stream;
   if (first_bad_out) *first_bad_out = -1;
   if (S == 0) return TGX_OK;
-  CU(cudaEventRecord(m->w().ev[6], st));
+  CU(cudaEventRecord(m->ws.ev[6], st));
   const uint8_t* text = d_text;
   const uint64_t* off = d_off;
   if (flags & TGX_FLAG_CRLF) {
     rc = run_crlf(m, d_text, d_off, S, n_bytes);
     if (rc) return rc;
-    text = m->w().text2.as<uint8_t>();
-    off = m->w().off2.as<uint64_t>();
+    text = m->ws.text2.as<uint8_t>();
+    off = m->ws.off2.as<uint64_t>();
   }
   rc = run_viterbi(m, text, off, S, n_bytes, nullptr);
   if (rc) return rc;
@@ -2329,13 +2267,13 @@ int tgx_token_frequencies_dev(tgx_model* m, const uint8_t* d_text, const uint64_
   int64_t bad = -1;
   rc = first_bad(m, (uint32_t)S, &bad);
   if (rc) return rc;
-  CU(cudaEventRecord(m->w().ev[7], st));
+  CU(cudaEventRecord(m->ws.ev[7], st));
   CU(cudaStreamSynchronize(st));
   finish_stats(m, 1);
   if (first_bad_out) *first_bad_out = bad;
   if (bad >= 0) {
     uint32_t l = 0;
-    CU(cudaMemcpy(&l, m->w().ulen.as<uint32_t>() + bad, 4, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(&l, m->ws.ulen.as<uint32_t>() + bad, 4, cudaMemcpyDeviceToHost));
     if (bad_len) *bad_len = l;
     return fail(TGX_ERR_NO_PATH, "no path to position " + std::to_string(l) + "/" + std::to_string(l));
   }
@@ -2352,9 +2290,9 @@ int tgx_token_frequencies(tgx_model* m, const uint8_t* text, const uint64_t* off
   CU(m->text.reserve(N + 16));
   CU(m->off.reserve((S + 1) * 8));
   CU(m->freq.reserve(m->V * 8 + 8));
-  CU(cudaMemcpyAsync(m->text.p, text, N, cudaMemcpyHostToDevice, m->w().stream));
-  CU(cudaMemcpyAsync(m->off.p, off, (S + 1) * 8, cudaMemcpyHostToDevice, m->w().stream));
-  CU(dev_fill(m->freq.p, 0, m->V * 8 + 8, m->w().stream));
+  CU(cudaMemcpyAsync(m->text.p, text, N, cudaMemcpyHostToDevice, m->ws.stream));
+  CU(cudaMemcpyAsync(m->off.p, off, (S + 1) * 8, cudaMemcpyHostToDevice, m->ws.stream));
+  CU(dev_fill(m->freq.p, 0, m->V * 8 + 8, m->ws.stream));
   rc = tgx_token_frequencies_dev(m, m->text.as<uint8_t>(), m->off.as<uint64_t>(), S, N, flags, m->freq.as<uint64_t>(),
                                  first_bad_out, bad_len);
   if (rc) return rc;
@@ -2386,7 +2324,7 @@ int tgx_pair_frequencies_dev(tgx_model* m, const uint8_t* d_text, const uint64_t
   if (rc) return rc;
   if (bad >= 0) {  // the reference unwraps the encode error (src/merge.rs:59)
     uint32_t l = 0;
-    CU(cudaMemcpy(&l, m->w().ulen.as<uint32_t>() + bad, 4, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(&l, m->ws.ulen.as<uint32_t>() + bad, 4, cudaMemcpyDeviceToHost));
     if (first_bad_out) *first_bad_out = bad;
     if (bad_len) *bad_len = l;
     return fail(TGX_ERR_NO_PATH, "no path to position " + std::to_string(l) + "/" + std::to_string(l));
@@ -2394,13 +2332,13 @@ int tgx_pair_frequencies_dev(tgx_model* m, const uint8_t* d_text, const uint64_t
   if (T < 2) return TGX_OK;
   if (T >= (1ull << 31)) return fail(TGX_ERR_INVALID, "too many tokens in one call (< 2^31); split the batch");
   // 2. keys -> sort -> run lengths -> sort by count (stable: ties stay key-ascending)
-  cudaStream_t st = m->w().stream;
+  cudaStream_t st = m->ws.stream;
   const unsigned long long V = std::max<uint64_t>(m->V, 1);
   int key_bits = 1;
   while (key_bits < 64 && (V * V) >> key_bits) key_bits++;
-  DevBuf& kb = m->w().bp;      // scratch, free again after the encode: keys | sorted keys
-  DevBuf& ub = m->w().mark;    //                                      unique | counts | counts sorted | unique sorted
-  DevBuf& nb = m->w().small;
+  DevBuf& kb = m->ws.bp;      // scratch, free again after the encode: keys | sorted keys
+  DevBuf& ub = m->ws.mark;    //                                      unique | counts | counts sorted | unique sorted
+  DevBuf& nb = m->ws.small;
   CU(kb.reserve(T * 16 + 64));
   CU(ub.reserve(T * 32 + 64));
   unsigned long long* keys = kb.as<unsigned long long>();
@@ -2415,11 +2353,11 @@ int tgx_pair_frequencies_dev(tgx_model* m, const uint8_t* d_text, const uint64_t
   pair_keys_mark_starts<<<nblk(S, 256), 256, 0, st>>>(m->idoff.as<uint64_t>(), S, V, keys);
   size_t tmp = 0;
   CU(cub::DeviceRadixSort::SortKeys(nullptr, tmp, keys, keys_sorted, (int)T, 0, key_bits, st));
-  CU(m->w().cubtmp.reserve(tmp));
-  CU(cub::DeviceRadixSort::SortKeys(m->w().cubtmp.p, tmp, keys, keys_sorted, (int)T, 0, key_bits, st));
+  CU(m->ws.cubtmp.reserve(tmp));
+  CU(cub::DeviceRadixSort::SortKeys(m->ws.cubtmp.p, tmp, keys, keys_sorted, (int)T, 0, key_bits, st));
   CU(cub::DeviceRunLengthEncode::Encode(nullptr, tmp, keys_sorted, uniq, cnt, d_runs, (int)T, st));
-  CU(m->w().cubtmp.reserve(tmp));
-  CU(cub::DeviceRunLengthEncode::Encode(m->w().cubtmp.p, tmp, keys_sorted, uniq, cnt, d_runs, (int)T, st));
+  CU(m->ws.cubtmp.reserve(tmp));
+  CU(cub::DeviceRunLengthEncode::Encode(m->ws.cubtmp.p, tmp, keys_sorted, uniq, cnt, d_runs, (int)T, st));
   pair_count_runs<<<1, 32, 0, st>>>(uniq, d_runs, V, d_np);
   unsigned long long np = 0;
   rc = read_words(m, d_np, nullptr, &np, nullptr);
@@ -2428,8 +2366,8 @@ int tgx_pair_frequencies_dev(tgx_model* m, const uint8_t* d_text, const uint64_t
   if (np == 0) return TGX_OK;
   if (np > cap) return fail(TGX_ERR_CAPACITY, "pair capacity too small: need " + std::to_string(np));
   CU(cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp, cnt, cnt_sorted, uniq, uniq_sorted, (int)np, 0, 64, st));
-  CU(m->w().cubtmp.reserve(tmp));
-  CU(cub::DeviceRadixSort::SortPairsDescending(m->w().cubtmp.p, tmp, cnt, cnt_sorted, uniq, uniq_sorted, (int)np, 0, 64, st));
+  CU(m->ws.cubtmp.reserve(tmp));
+  CU(cub::DeviceRadixSort::SortPairsDescending(m->ws.cubtmp.p, tmp, cnt, cnt_sorted, uniq, uniq_sorted, (int)np, 0, 64, st));
   pair_unpack<<<nblk(np, 256), 256, 0, st>>>(uniq_sorted, np, V, reinterpret_cast<unsigned long long*>(d_pairs));
   copy_u32<<<nblk(np * 2, 256), 256, 0, st>>>(reinterpret_cast<const uint32_t*>(cnt_sorted),
                                               reinterpret_cast<uint32_t*>(d_counts), np * 2);
@@ -2449,8 +2387,8 @@ int tgx_pair_frequencies(tgx_model* m, const uint8_t* text, const uint64_t* off,
   CU(m->text.reserve(N + 16));
   CU(m->off.reserve((S + 1) * 8));
   CU(m->freq.reserve(cap * 16 + 16));
-  CU(cudaMemcpyAsync(m->text.p, text, N, cudaMemcpyHostToDevice, m->w().stream));
-  CU(cudaMemcpyAsync(m->off.p, off, (S + 1) * 8, cudaMemcpyHostToDevice, m->w().stream));
+  CU(cudaMemcpyAsync(m->text.p, text, N, cudaMemcpyHostToDevice, m->ws.stream));
+  CU(cudaMemcpyAsync(m->off.p, off, (S + 1) * 8, cudaMemcpyHostToDevice, m->ws.stream));
   uint64_t* d_pairs = m->freq.as<uint64_t>();
   uint64_t* d_counts = d_pairs + cap;
   rc = tgx_pair_frequencies_dev(m, m->text.as<uint8_t>(), m->off.as<uint64_t>(), S, N, flags, d_pairs, d_counts, cap, n_pairs,
@@ -2476,57 +2414,57 @@ int expected_counts_impl(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
   if (!d_off || (!d_expected && !d_limbs) || snippet_len == 0) return fail(TGX_ERR_INVALID, "bad argument");
   if (snippet_len >= (1ull << 31)) return fail(TGX_ERR_INVALID, "snippet_len must be < 2^31");
   std::lock_guard<std::recursive_mutex> g(m->mu);
-  m->w().stats = Stats();
-  cudaStream_t st = m->w().stream;
+  m->ws.stats = Stats();
+  cudaStream_t st = m->ws.stream;
   rc = order_after_caller(m);
   if (rc) return rc;
-  CU(cudaEventRecord(m->w().ev[6], st));
+  CU(cudaEventRecord(m->ws.ev[6], st));
   if (bad_sample) *bad_sample = -1;
   if (bad_z) *bad_z = 0.0;
   // 1. snippet table
-  CU(m->w().ntok.reserve((S + 2) * 16));
-  unsigned long long* cnt = m->w().ntok.as<unsigned long long>();
+  CU(m->ws.ntok.reserve((S + 2) * 16));
+  unsigned long long* cnt = m->ws.ntok.as<unsigned long long>();
   unsigned long long* first_unit = cnt + S + 1;
   CU(dev_fill(cnt, 0, (S + 1) * 8, st));
   if (S) {
     snippet_counts<<<nblk(S, 256), 256, 0, st>>>(d_off, S, snippet_len, cnt);
-    m->w().stats.launches += 1;
+    m->ws.stats.launches += 1;
   }
   size_t tmp = 0;
   CU(cub::DeviceScan::ExclusiveSum(nullptr, tmp, cnt, first_unit, (int)(S + 1), st));
-  CU(m->w().cubtmp.reserve(tmp));
-  CU(cub::DeviceScan::ExclusiveSum(m->w().cubtmp.p, tmp, cnt, first_unit, (int)(S + 1), st));
-  m->w().stats.launches += 2;
+  CU(m->ws.cubtmp.reserve(tmp));
+  CU(cub::DeviceScan::ExclusiveSum(m->ws.cubtmp.p, tmp, cnt, first_unit, (int)(S + 1), st));
+  m->ws.stats.launches += 2;
   unsigned long long U64 = 0;
   CU(cudaMemcpyAsync(&U64, first_unit + S, 8, cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
   if (U64 >= (1ull << 32)) return fail(TGX_ERR_INVALID, "too many snippets in one call (< 2^32)");
   uint32_t U = (uint32_t)U64;
   if (U == 0) {
-    CU(cudaEventRecord(m->w().ev[7], st));
+    CU(cudaEventRecord(m->ws.ev[7], st));
     CU(cudaStreamSynchronize(st));
     return TGX_OK;
   }
-  CU(m->w().ustart.reserve((size_t)U * 8 + 8));
-  CU(m->w().ulen.reserve((size_t)U * 4 + 4));
-  CU(m->w().vals_in.reserve((size_t)U * 4 + 4));
-  CU(m->w().status.reserve((size_t)U * 4 + 4));
+  CU(m->ws.ustart.reserve((size_t)U * 8 + 8));
+  CU(m->ws.ulen.reserve((size_t)U * 4 + 4));
+  CU(m->ws.vals_in.reserve((size_t)U * 4 + 4));
+  CU(m->ws.status.reserve((size_t)U * 4 + 4));
   CU(m->idoff.reserve((size_t)U * 4 + 4));  // unit -> sample
   CU(m->A.reserve((n_bytes + U + 2) * 8));
-  CU(m->w().small.reserve(256));
-  units_from_snippets<<<nblk(S, 256), 256, 0, st>>>(d_off, S, snippet_len, first_unit, m->w().ustart.as<uint64_t>(),
-                                                   m->w().ulen.as<uint32_t>(), m->w().vals_in.as<uint32_t>(),
+  CU(m->ws.small.reserve(256));
+  units_from_snippets<<<nblk(S, 256), 256, 0, st>>>(d_off, S, snippet_len, first_unit, m->ws.ustart.as<uint64_t>(),
+                                                   m->ws.ulen.as<uint32_t>(), m->ws.vals_in.as<uint32_t>(),
                                                    m->idoff.as<uint32_t>());
-  m->w().stats.launches += 1;
+  m->ws.stats.launches += 1;
   rc = sort_units(m, U);
   if (rc) return rc;
-  CU(dev_fill(m->w().status.p, 0, (size_t)U * 4 + 4, st));
+  CU(dev_fill(m->ws.status.p, 0, (size_t)U * 4 + 4, st));
 
   FbParams p;
   p.u.text = d_text;
-  p.u.unit_start = m->w().ustart.as<uint64_t>();
-  p.u.unit_len = m->w().ulen.as<uint32_t>();
-  p.u.order = m->w().vals_out.as<uint32_t>();
+  p.u.unit_start = m->ws.ustart.as<uint64_t>();
+  p.u.unit_len = m->ws.ulen.as<uint32_t>();
+  p.u.order = m->ws.vals_out.as<uint32_t>();
   p.u.first = 0;
   p.u.count = U;
   p.u.counts = nullptr;
@@ -2536,7 +2474,7 @@ int expected_counts_impl(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
   p.u.rows = std::max<uint32_t>(1, m->da.max_token_len);
   p.u.W = p.u.rows + 1;
   p.A = m->A.as<double>();
-  p.status = m->w().status.as<int32_t>();
+  p.status = m->ws.status.as<int32_t>();
   p.dropout = m->dropout;
   p.drop_key = drop_unit_key(m->drop_seed, ~0ull);  // (its own stream of draws, apart from the encode samples')
   p.drop_base = m->drop_byte_base;
@@ -2567,25 +2505,25 @@ int expected_counts_impl(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
   if (rows_ok) {
     const size_t need = ((size_t)n_bytes + U + 2) * 8 + (use_rows ? ((size_t)n_bytes + 64) * 4 : 0);
     size_t fr = 0, tot = 0;
-    const size_t have = m->Bbeta.cap + m->w().rec.cap;
+    const size_t have = m->Bbeta.cap + m->ws.rec.cap;
     if (need > have && (cudaMemGetInfo(&fr, &tot) != cudaSuccess || fr + have < need + need / 8 + ((size_t)2 << 30))) rows_ok = false;
     if (rows_ok && m->Bbeta.reserve(((size_t)n_bytes + U + 2) * 8) != cudaSuccess) {
       (void)cudaGetLastError();
       rows_ok = false;
     }
   }
-  CU(cudaEventRecord(m->w().ev[8], st));
+  CU(cudaEventRecord(m->ws.ev[8], st));
   if (use_rows) {
     rc = run_match(m, d_text, n_bytes);
     if (rc) return rc;
   }
-  CU(cudaEventRecord(m->w().ev[9], st));
+  CU(cudaEventRecord(m->ws.ev[9], st));
 
   // Long snippets (latency-critical: one ordered chain each) get a whole warp on a second stream; the short ones run
   // one lane each on a third; whatever is in between (only when option 17 sets a lane threshold) G lanes per snippet.
   uint32_t n_long = 0, n_lane = 0;
   {
-    uint32_t* counts = m->w().small.as<uint32_t>();
+    uint32_t* counts = m->ws.small.as<uint32_t>();
     const bool lanes_ok = rows_ok && m->estep_lane_threshold != 0;
     int64_t thr64 = m->estep_long_threshold;
     if (thr64 <= 0)
@@ -2596,8 +2534,8 @@ int expected_counts_impl(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
     uint32_t thr_lane = 0;
     if (lanes_ok)
       thr_lane = m->estep_lane_threshold < 0 ? thr : (uint32_t)std::min<int64_t>(m->estep_lane_threshold, (int64_t)thr);
-    split_sorted<<<1, 32, 0, st>>>(m->w().keys_out.as<uint32_t>(), U, thr, thr_lane, counts);
-    m->w().stats.launches += 1;
+    split_sorted<<<1, 32, 0, st>>>(m->ws.keys_out.as<uint32_t>(), U, thr, thr_lane, counts);
+    m->ws.stats.launches += 1;
     uint32_t h[3];
     CU(cudaMemcpyAsync(h, counts, 12, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
@@ -2616,7 +2554,7 @@ int expected_counts_impl(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
   pn.f = p;
   pn.f.u.first = U - n_lane;
   pn.f.u.count = n_lane;
-  pn.rec = m->w().rec.as<uint32_t>();
+  pn.rec = m->ws.rec.as<uint32_t>();
   pn.rows = m->d_rows.as<double>();
   pn.row_ids = m->d_rowids.as<uint32_t>();
   pn.B = m->Bbeta.as<double>();
@@ -2626,12 +2564,8 @@ int expected_counts_impl(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
   pw.blob_end = d_text + n_bytes;
   pw.B = pn.B;
   const bool split = rows_ok;  // beta chains stored and run beside the alpha chains, counts by a third kernel
-  const uint32_t lane_blocks = nblk(n_lane, FR_WARPS * 32);
   static_assert(FR_WARPS == FL_WARPS && FRC_WARPS == FC_WARPS, "one launch shape for both sets of lane kernels");
-  // forward / backward device times (tgx_model_last_stat 2, 3) are taken on the stream that carries most snippets
-  cudaStream_t st_ev = (n_lane > ps.u.count) ? m->stream3 : st;
-  (void)st_ev;
-  CU(cudaEventRecord(m->w().ev[0], st));  // (tgx_model_last_stat 2 = all chains and counts kernels, 3 = 0)
+  CU(cudaEventRecord(m->ws.ev[0], st));  // (tgx_model_last_stat 2 = all chains and counts kernels, 3 = 0)
   CU(launch_fb_g(m, 32, pl, false, m->stream2));
   if (split && pl.u.count) {  // the beta chains of the longest snippets run beside their forward chains
     CU(cudaStreamWaitEvent(m->stream4, m->ev_fork, 0));
@@ -2643,7 +2577,7 @@ int expected_counts_impl(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
       CU(cudaFuncSetAttribute(fb_backward_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       fb_backward_kernel<32, true><<<nblk(pl.u.count, WPB), WPB * 32, smem, m->stream4>>>(pl, pn.B);
     }
-    m->w().stats.launches += 1;
+    m->ws.stats.launches += 1;
     CU(cudaEventRecord(m->ev_join4, m->stream4));
   }
   CU(launch_fb_g(m, m->g_estep, ps, false, st));
@@ -2655,8 +2589,21 @@ int expected_counts_impl(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
   constexpr int NGRP = 3;
   const double c1 = m->estep_cut1 / 1000.0, c2 = m->estep_cut2 / 1000.0;
   const double grp_cut[NGRP + 1] = {0.0, std::min(c1, c2), c2, 1.0};
+  // the lane kernels that walk the trie take `w`, the ones over the match stream `n`: alpha and beta chains in one
+  // launch, then the counts from the stored alpha / beta
+  auto lane_split = [use_rows, drop](uint32_t grid, cudaStream_t s, const FbLaneParams& w, const FbRowsParams& n) {
+    if (!use_rows && drop) fb_split_lane_kernel<true><<<grid, FL_WARPS * 32, 0, s>>>(w);
+    else if (!use_rows) fb_split_lane_kernel<false><<<grid, FL_WARPS * 32, 0, s>>>(w);
+    else if (drop) fbr_split_kernel<true><<<grid, FR_WARPS * 32, 0, s>>>(n);
+    else fbr_split_kernel<false><<<grid, FR_WARPS * 32, 0, s>>>(n);
+  };
+  auto lane_counts = [use_rows, drop](uint32_t grid, cudaStream_t s, const FbLaneParams& w, const FbRowsParams& n) {
+    if (!use_rows && drop) fb_contrib_kernel<true><<<grid, FC_WARPS * 32, 0, s>>>(w);
+    else if (!use_rows) fb_contrib_kernel<false><<<grid, FC_WARPS * 32, 0, s>>>(w);
+    else if (drop) fbr_contrib_kernel<true><<<grid, FRC_WARPS * 32, 0, s>>>(n);
+    else fbr_contrib_kernel<false><<<grid, FRC_WARPS * 32, 0, s>>>(n);
+  };
   if (n_lane) {
-    (void)lane_blocks;
     CU(cudaStreamWaitEvent(m->stream5, m->ev_fork, 0));
     CU(cudaStreamWaitEvent(m->stream6, m->ev_fork, 0));
     for (int gi = 0; gi < NGRP; gi++) {
@@ -2669,15 +2616,9 @@ int expected_counts_impl(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
       FbRowsParams gn = pn;
       gn.f.u = gw.f.u;
       const uint32_t blocks = nblk(g1 - g0, FR_WARPS * 32);
-      if (!use_rows && drop) fb_split_lane_kernel<true><<<2 * blocks, FL_WARPS * 32, 0, gs>>>(gw);
-      else if (!use_rows) fb_split_lane_kernel<false><<<2 * blocks, FL_WARPS * 32, 0, gs>>>(gw);
-      else if (drop) fbr_split_kernel<true><<<2 * blocks, FR_WARPS * 32, 0, gs>>>(gn);
-      else fbr_split_kernel<false><<<2 * blocks, FR_WARPS * 32, 0, gs>>>(gn);
-      if (!use_rows && drop) fb_contrib_kernel<true><<<contrib_grid(g1 - g0), FC_WARPS * 32, 0, gs>>>(gw);
-      else if (!use_rows) fb_contrib_kernel<false><<<contrib_grid(g1 - g0), FC_WARPS * 32, 0, gs>>>(gw);
-      else if (drop) fbr_contrib_kernel<true><<<contrib_grid(g1 - g0), FRC_WARPS * 32, 0, gs>>>(gn);
-      else fbr_contrib_kernel<false><<<contrib_grid(g1 - g0), FRC_WARPS * 32, 0, gs>>>(gn);
-      m->w().stats.launches += 2;
+      lane_split(2 * blocks, gs, gw, gn);
+      lane_counts(contrib_grid(g1 - g0), gs, gw, gn);
+      m->ws.stats.launches += 2;
     }
   }
 
@@ -2687,11 +2628,8 @@ int expected_counts_impl(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
     pc.f.u = pl.u;
     FbLaneParams pcw = pw;
     pcw.f.u = pl.u;
-    if (!use_rows && drop) fb_contrib_kernel<true><<<contrib_grid(pl.u.count), FC_WARPS * 32, 0, m->stream2>>>(pcw);
-    else if (!use_rows) fb_contrib_kernel<false><<<contrib_grid(pl.u.count), FC_WARPS * 32, 0, m->stream2>>>(pcw);
-    else if (drop) fbr_contrib_kernel<true><<<contrib_grid(pl.u.count), FRC_WARPS * 32, 0, m->stream2>>>(pc);
-    else fbr_contrib_kernel<false><<<contrib_grid(pl.u.count), FRC_WARPS * 32, 0, m->stream2>>>(pc);
-    m->w().stats.launches += 1;
+    lane_counts(contrib_grid(pl.u.count), m->stream2, pcw, pc);
+    m->ws.stats.launches += 1;
   } else {
     CU(launch_fb_g(m, 32, pl, true, m->stream2));
   }
@@ -2705,31 +2643,27 @@ int expected_counts_impl(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
   CU(cudaStreamWaitEvent(st, m->ev_join, 0));
   CU(cudaEventRecord(m->ev_join3, m->stream3));
   CU(cudaStreamWaitEvent(st, m->ev_join3, 0));
-  CU(cudaEventRecord(m->w().ev[1], st));
-  CU(cudaEventRecord(m->w().ev[2], st));
-  CU(cudaEventRecord(m->w().ev[3], st));
-  CU(cudaEventRecord(m->ev_join, m->stream2));
-  CU(cudaStreamWaitEvent(st, m->ev_join, 0));
-  CU(cudaEventRecord(m->ev_join3, m->stream3));
-  CU(cudaStreamWaitEvent(st, m->ev_join3, 0));
+  CU(cudaEventRecord(m->ws.ev[1], st));
+  CU(cudaEventRecord(m->ws.ev[2], st));
+  CU(cudaEventRecord(m->ws.ev[3], st));
   fold_hot_acc_kernel<<<nblk(m->V, 256), 256, 0, st>>>(p.hot_acc, p.hot_k, p.hot_r, p.acc, (uint32_t)m->V);
-  m->w().stats.launches += 1;
+  m->ws.stats.launches += 1;
   export_acc_kernel<<<nblk(m->V, 256), 256, 0, st>>>(p.acc, (uint32_t)m->V, d_expected, d_limbs);
-  m->w().stats.launches += 1;
+  m->ws.stats.launches += 1;
   int64_t bad = -1;
   rc = first_bad(m, U, &bad);
   if (rc) return rc;
-  CU(cudaEventRecord(m->w().ev[7], st));
+  CU(cudaEventRecord(m->ws.ev[7], st));
   CU(cudaStreamSynchronize(st));
   finish_stats(m, 2);
   float mms = 0;
-  if (cudaEventElapsedTime(&mms, m->w().ev[8], m->w().ev[9]) == cudaSuccess) m->last_stats.match_ms = mms;
+  if (cudaEventElapsedTime(&mms, m->ws.ev[8], m->ws.ev[9]) == cudaSuccess) m->last_stats.match_ms = mms;
   if (bad >= 0) {
     uint32_t smp = 0, l = 0;
     uint64_t us = 0;
     CU(cudaMemcpy(&smp, m->idoff.as<uint32_t>() + bad, 4, cudaMemcpyDeviceToHost));
-    CU(cudaMemcpy(&l, m->w().ulen.as<uint32_t>() + bad, 4, cudaMemcpyDeviceToHost));
-    CU(cudaMemcpy(&us, m->w().ustart.as<uint64_t>() + bad, 8, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(&l, m->ws.ulen.as<uint32_t>() + bad, 4, cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(&us, m->ws.ustart.as<uint64_t>() + bad, 8, cudaMemcpyDeviceToHost));
     double z = 0;
     CU(cudaMemcpy(&z, m->A.as<double>() + us + bad + l, 8, cudaMemcpyDeviceToHost));
     if (bad_sample) *bad_sample = smp;
@@ -2766,10 +2700,10 @@ int tgx_counts_from_limbs_dev(tgx_model* m, const int64_t* d_limbs, uint64_t voc
   rc = order_after_caller(m);
   if (rc) return rc;
   if (vocab_size)
-    limbs_to_double_kernel<<<nblk(vocab_size, 256), 256, 0, m->w().stream>>>(reinterpret_cast<const long long*>(d_limbs),
+    limbs_to_double_kernel<<<nblk(vocab_size, 256), 256, 0, m->ws.stream>>>(reinterpret_cast<const long long*>(d_limbs),
                                                                           (uint32_t)vocab_size, d_expected);
   CU(cudaGetLastError());
-  CU(cudaStreamSynchronize(m->w().stream));
+  CU(cudaStreamSynchronize(m->ws.stream));
   return TGX_OK;
 }
 
@@ -2783,9 +2717,9 @@ int tgx_expected_counts(tgx_model* m, const uint8_t* text, const uint64_t* off, 
   CU(m->text.reserve(N + 16));
   CU(m->off.reserve((S + 1) * 8));
   CU(m->expected.reserve(m->V * 8 + 8));
-  CU(cudaMemcpyAsync(m->text.p, text, N, cudaMemcpyHostToDevice, m->w().stream));
-  CU(cudaMemcpyAsync(m->off.p, off, (S + 1) * 8, cudaMemcpyHostToDevice, m->w().stream));
-  CU(dev_fill(m->expected.p, 0, m->V * 8 + 8, m->w().stream));
+  CU(cudaMemcpyAsync(m->text.p, text, N, cudaMemcpyHostToDevice, m->ws.stream));
+  CU(cudaMemcpyAsync(m->off.p, off, (S + 1) * 8, cudaMemcpyHostToDevice, m->ws.stream));
+  CU(dev_fill(m->expected.p, 0, m->V * 8 + 8, m->ws.stream));
   rc = tgx_expected_counts_dev(m, m->text.as<uint8_t>(), m->off.as<uint64_t>(), S, N, snippet_len,
                                m->expected.as<double>(), bad_sample, bad_z);
   if (rc) return rc;

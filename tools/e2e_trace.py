@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Developer probe: wall time of the pipelined host entry point (tgx_encode_batch, pinned host buffers) for several
-chunk sizes, with (option 11 = 1) and without queuing the next chunk's kernels early.  TGX_TRACE=1 prints the device timeline."""
+forward passes and chunk sizes.  TGX_TRACE=1 prints the device timeline."""
 import os
 import sys
 import time
@@ -19,16 +19,15 @@ def main():
     blob, off, _ = bench.workload(synth, 1, 0, 1_000_000_000, out=h_text)
     NB = int(off[-1])
     h_ids = N.pinned_empty(4 * (NB // 2 + 16)).view(np.uint32)
-    # argv: "algo:chunk_MiB:overlap[:key=value,...]" ...   (default: the shipped configuration and its neighbours)
-    cfgs = sys.argv[1:] or ["2:352:0", "2:352:1", "3:352:0", "3:352:1", "3:176:1", "3:128:1"]
+    # argv: "algo:chunk_MiB[:key=value,...]" ...   (default: the shipped configuration and its neighbours)
+    cfgs = sys.argv[1:] or ["2:352", "3:352", "3:176", "3:128"]
     for cfg in cfgs:
         parts = cfg.split(":")
-        algo, ch, ov = int(parts[0]), int(parts[1]) << 20, int(parts[2])
+        algo, ch = int(parts[0]), int(parts[1]) << 20
         m.set_option(3, algo)
         m.set_option(7, ch)
-        m.set_option(11, ov)
-        if len(parts) > 3 and parts[3]:
-            for kv in parts[3].split(","):
+        if len(parts) > 2 and parts[2]:
+            for kv in parts[2].split(","):
                 k, v = kv.split("=")
                 m.set_option(int(k), int(v))
         best = 1e9
@@ -38,7 +37,7 @@ def main():
             dt = time.perf_counter() - t
             if i:
                 best = min(best, dt)
-        print(f"algo {algo} chunk {ch >> 20} MiB overlap={ov} {parts[3] if len(parts) > 3 else ''}: best {best * 1e3:.2f} ms  ({NB / best / 1e9:.2f} GB/s)", flush=True)
+        print(f"algo {algo} chunk {ch >> 20} MiB {parts[2] if len(parts) > 2 else ''}: best {best * 1e3:.2f} ms  ({NB / best / 1e9:.2f} GB/s)", flush=True)
 
 
 if __name__ == "__main__":
