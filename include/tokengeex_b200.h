@@ -98,13 +98,17 @@ int tgx_crlf_batch(tgx_model* m, const uint8_t* text, const uint64_t* off, uint6
  *  proc_len [S]        length after the processors — the `len` of NoPath(len,len) (may be NULL)
  * Returns TGX_OK, or TGX_ERR_NO_PATH when any sample failed (*first_bad = lowest failing
  * index, as `collect::<Result<_>>` surfaces one error; other samples are still encoded),
- * or TGX_ERR_CAPACITY (id_off[S] holds the required capacity). */
+ * or TGX_ERR_CAPACITY (id_off[S] holds the required capacity).  CAPACITY wins over NO_PATH: with both, the call
+ * returns TGX_ERR_CAPACITY and id_off, status, proc_len and *first_bad are still complete.  Nothing is written past
+ * ids_cap.  S == 0, or samples that are all empty, return TGX_OK with every id_off entry 0. */
 int tgx_encode_batch(tgx_model* m, const uint8_t* text, const uint64_t* off, uint64_t S, uint32_t flags,
                      uint32_t* ids, uint64_t ids_cap, uint64_t* id_off, int32_t* status, uint64_t* proc_len,
                      int64_t* first_bad);
 /* Same with device-resident inputs and outputs.  n_bytes = off[S].  *total_ids (host)
- * receives id_off[S].  d_off must be non-decreasing with samples shorter than 2^32 bytes (the host variants check it
- * and return TGX_ERR_INVALID / TGX_ERR_UNSUPPORTED; the device variants do not read the offsets on the host). */
+ * receives id_off[S]; d_ids = NULL with ids_cap = 0 is a sizing call (TGX_ERR_CAPACITY unless there are no ids, with
+ * *total_ids and d_id_off filled).  On TGX_ERR_CAPACITY the first ids_cap ids are written.  d_off must be
+ * non-decreasing with samples shorter than 2^32 bytes (the host variants check it and return TGX_ERR_INVALID /
+ * TGX_ERR_UNSUPPORTED; the device variants do not read the offsets on the host). */
 int tgx_encode_batch_dev(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint64_t S,
                          uint64_t n_bytes, uint32_t flags, uint32_t* d_ids, uint64_t ids_cap,
                          uint64_t* d_id_off, int32_t* d_status, uint64_t* d_proc_len, uint64_t* total_ids,
@@ -127,8 +131,9 @@ int tgx_encode_batch_dev(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
  *  n_samples / n_ids  non-empty samples and ids written (also when TGX_ERR_CAPACITY reports what is needed)
  * Returns TGX_OK; TGX_ERR_NOT_UTF8 (*first_bad = lowest invalid sample, relative to the buffer, *bad_pos = byte offset
  * of its first byte in data; nothing else is defined); TGX_ERR_NO_PATH (*first_bad = lowest failing sample, *bad_pos =
- * its length after processing; the other samples are encoded); TGX_ERR_CAPACITY.  The handle's dropout applies as for
- * tgx_encode_batch. */
+ * its length after processing; the other samples are encoded); TGX_ERR_CAPACITY, which wins over NO_PATH (nothing is
+ * written past ids_cap or off_cap).  A buffer without non-empty samples returns TGX_OK with id_off[0] = 0.  The handle's
+ * dropout applies as for tgx_encode_batch. */
 int tgx_encode_corpus(tgx_model* m, const uint8_t* data, uint64_t n, uint32_t flags, uint64_t sample_base,
                       int64_t sep_id, uint32_t id_bytes, void* ids, uint64_t ids_cap, uint64_t* id_off,
                       uint64_t off_cap, uint64_t* n_samples, uint64_t* n_ids, int64_t* first_bad, uint64_t* bad_pos);
@@ -142,7 +147,8 @@ int tgx_encode_corpus(tgx_model* m, const uint8_t* data, uint64_t n, uint32_t fl
 int tgx_expected_counts(tgx_model* m, const uint8_t* text, const uint64_t* off, uint64_t S,
                         uint64_t snippet_len, double* expected, int64_t* bad_sample, double* bad_z);
 /* Device variant: d_expected[V] is ACCUMULATED into (+=) so a caller can sum shards /
- * chunks in place (and all-reduce the same buffer across GPUs). */
+ * chunks in place (and all-reduce the same buffer across GPUs).  A batch without bytes returns TGX_OK and adds
+ * nothing. */
 int tgx_expected_counts_dev(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint64_t S,
                             uint64_t n_bytes, uint64_t snippet_len, double* d_expected, int64_t* bad_sample,
                             double* bad_z);
@@ -165,7 +171,8 @@ int tgx_counts_from_limbs_dev(tgx_model* m, const int64_t* d_limbs, uint64_t voc
 
 /* Frequency pass of prune_vocab (src/prune.rs:205-246): freq[id] += 1 over
  * Model::encode(sample, 0.0) of WHOLE samples.  freq[V] is overwritten (host variant) /
- * accumulated (device variant).  TGX_ERR_NO_PATH as for encode. */
+ * accumulated (device variant).  TGX_ERR_NO_PATH as for encode (*bad_len = the sample's length after processing;
+ * first_bad and bad_len may be NULL).  A batch without bytes returns TGX_OK and adds nothing. */
 int tgx_token_frequencies(tgx_model* m, const uint8_t* text, const uint64_t* off, uint64_t S, uint32_t flags,
                           uint64_t* freq, int64_t* first_bad, uint64_t* bad_len);
 int tgx_token_frequencies_dev(tgx_model* m, const uint8_t* d_text, const uint64_t* d_off, uint64_t S,
@@ -176,8 +183,10 @@ int tgx_token_frequencies_dev(tgx_model* m, const uint8_t* d_text, const uint64_
  * sample (dropout 0.0) and count the adjacent token-id pairs inside each sample.  pairs[i] = (first id << 32) |
  * second id and counts[i], for i < *n_pairs, ordered by count descending (`pairs.sort_unstable_by(|a, b|
  * b.1.cmp(&a.1))`, :83; equal counts — undefined order in the reference — by (first, second) ascending).
- * TGX_ERR_CAPACITY when there are more than cap distinct pairs (*n_pairs = needed); TGX_ERR_NO_PATH as for encode
- * (the reference unwraps the error, :59).  One call handles fewer than 2^31 tokens. */
+ * TGX_ERR_CAPACITY when there are more than cap distinct pairs (*n_pairs = needed, nothing written); TGX_ERR_NO_PATH as
+ * for encode (the reference unwraps the error, :59), checked before the pairs are counted, so it wins over CAPACITY.
+ * A batch without bytes or with fewer than two tokens returns TGX_OK with *n_pairs = 0.  One call handles fewer than
+ * 2^31 tokens. */
 int tgx_pair_frequencies(tgx_model* m, const uint8_t* text, const uint64_t* off, uint64_t S, uint32_t flags,
                          uint64_t* pairs, uint64_t* counts, uint64_t cap, uint64_t* n_pairs, int64_t* first_bad,
                          uint64_t* bad_len);

@@ -339,6 +339,20 @@ class Model:
         _check(rc, (TGX_OK, TGX_ERR_NO_PATH))
         return rc, int(bad.value), int(blen.value)
 
+    def pair_frequencies_dev(self, d_text: int, d_off: int, S: int, n_bytes: int, crlf: bool, d_pairs: int,
+                             d_counts: int, cap: int):
+        """tgx_pair_frequencies_dev: the n distinct pairs ((first << 32) | second, u64[cap]) and their counts
+        (u64[cap]) into device buffers, count-descending.  → (n, rc, first_bad, bad_len); rc is TGX_OK,
+        TGX_ERR_NO_PATH or TGX_ERR_CAPACITY (n > cap: n = pairs needed, nothing written)."""
+        n = C.c_uint64(0)
+        bad = C.c_int64(-1)
+        blen = C.c_uint64(0)
+        rc = lib().tgx_pair_frequencies_dev(self._h, d_text, d_off, S, n_bytes, TGX_FLAG_CRLF if crlf else 0,
+                                            d_pairs or None, d_counts or None, cap, C.byref(n), C.byref(bad),
+                                            C.byref(blen))
+        _check(rc, (TGX_OK, TGX_ERR_NO_PATH, TGX_ERR_CAPACITY))
+        return int(n.value), rc, int(bad.value), int(blen.value)
+
 
 def pinned_empty(nbytes: int) -> np.ndarray:
     """uint8 numpy array over cudaHostAlloc'd memory.  The allocation lives as long as the ctypes buffer every view of

@@ -1695,6 +1695,8 @@ int tgx_encode_batch_dev(tgx_model* m, const uint8_t* d_text, const uint64_t* d_
   if (first_bad_out) *first_bad_out = -1;
   if (total_ids) *total_ids = 0;
   if (S >= (1ull << 32)) return fail(TGX_ERR_INVALID, "too many samples in one call (< 2^32)");
+  rc = order_after_caller(m);
+  if (rc) return rc;
   if (S == 0) {
     CU(dev_fill(d_id_off, 0, 8, m->ws.stream));
     CU(cudaStreamSynchronize(m->ws.stream));
@@ -2251,6 +2253,8 @@ int tgx_token_frequencies_dev(tgx_model* m, const uint8_t* d_text, const uint64_
   cudaStream_t st = m->ws.stream;
   if (first_bad_out) *first_bad_out = -1;
   if (S == 0) return TGX_OK;
+  rc = order_after_caller(m);
+  if (rc) return rc;
   CU(cudaEventRecord(m->ws.ev[6], st));
   const uint8_t* text = d_text;
   const uint64_t* off = d_off;
@@ -2315,6 +2319,8 @@ int tgx_pair_frequencies_dev(tgx_model* m, const uint8_t* d_text, const uint64_t
   // 1. encode into the model's own id buffers
   CU(m->ids.reserve((n_bytes + 4) * 4));
   CU(m->idoff.reserve((S + 1) * 8));
+  rc = order_after_caller(m);
+  if (rc) return rc;
   rc = encode_enqueue(m, d_text, d_off, S, n_bytes, flags, m->ids.as<uint32_t>(), n_bytes + 4, m->idoff.as<uint64_t>(),
                       nullptr, nullptr);
   if (rc) return rc;
