@@ -70,9 +70,12 @@ int tgx_model_create(const uint8_t* token_bytes, const uint64_t* token_offsets, 
  * place: a new trie for the new vocabulary on the same device; streams and workspaces are kept (a fresh handle
  * would free and re-allocate GBs of scratch per EM sub-iteration).  When the new vocabulary is a subset of the one the
  * trie was built for (what the EM loop hands over) and not much smaller, the trie's layout is kept and only terminals,
- * ids and scores are rewritten (option 45; trie_slots of tgx_model_get_info then stays what it was): the same matches
- * as a fresh build.  On failure the model is unchanged.  Must not run concurrently with compute calls on the same
- * handle from other threads that still expect the old vocabulary. */
+ * ids and scores are rewritten (option 45): the same matches, ids, counts and frequencies as a fresh build.
+ * trie_nodes, trie_slots and max_token_len of tgx_model_get_info then stay those of the array: max_token_len is its
+ * depth, which can exceed the longest token left (such a vocabulary keeps running on the kernels for longer tokens).
+ * The handle's options (tgx_model_set_option) and dropout setting (tgx_model_set_dropout) survive a rebuild.  On
+ * failure the model is unchanged.  Must not run concurrently with compute calls on the same handle from other threads
+ * that still expect the old vocabulary. */
 int tgx_model_rebuild(tgx_model* m, const uint8_t* token_bytes, const uint64_t* token_offsets, const double* scores,
                       uint64_t vocab_size);
 void tgx_model_destroy(tgx_model* m);
